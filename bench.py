@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- signal samples/sec basecalled (sup@v3.3 XNA) on B200, with roofline and CPU baseline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dtype fp16|bf16]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dtype fp16|bf16] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: BASELINE.json configs[1] = sup@v3.3 architecture,
 UB "X" alphabet (n_base 5), batch 512 x 4000-sample chunks: conv stem -> 5 LSTMs -> CRF head -> CRF
@@ -20,6 +20,11 @@ input signal samples consumed per second.
 in oracle/bonito_oracle.py + the C CRF decode) on the host cores, same metric.
 Multi-GPU (torchrun): each rank runs the same batch shape on its own GPU (reads/chunks shard with no
 data-path collective -> weak scaling); NCCL only gathers the timing / counters.
+
+--dump-outputs DIR writes what the last timed step returned on rank 0 (default workload): DIR/seq.npy, the (N, T)
+left-packed letter codes, and DIR/lens.npy, the (N,) decoded lengths, both float32 (exact for these integers).  Signal
+and weights are seeded, so two builds run with the same arguments can be compared output for output (the head gain is
+calibrated from decoded lengths; --head-gain pins it).
 """
 import argparse
 import json
@@ -110,6 +115,14 @@ class ClockSampler(threading.Thread):
         sm.sort()
         return {'sm_mhz': sm[len(sm) // 2] if sm else None, 'sm_max_mhz': mx or None, 'reasons': sorted(reasons),
                 'samples': len(sm)}
+
+
+def dump_outputs(dirname, arrays):
+    """Write each tensor as dirname/<name>.npy in float32."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(dirname, name + '.npy'), t.cpu().numpy().astype(np.float32))
 
 
 def workload_config(N, L):
@@ -423,7 +436,13 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-gpu-comparator', action='store_true')
     ap.add_argument('--no-train-step', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed step as DIR/<name>.npy (see the module docstring)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'ours' or args.workload != 'chunks'):
+        ap.error('--dump-outputs is implemented for --impl ours --workload chunks')
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
     local = int(os.environ.get('LOCAL_RANK', 0))
@@ -466,10 +485,10 @@ def main():
         barrier()
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         barrier()
-        return e0.elapsed_time(e1)
+        return e0.elapsed_time(e1), out
 
     for _ in range(max(args.warmup, 3)):
         step_device()
@@ -477,9 +496,10 @@ def main():
     sampler = ClockSampler(local)
     sampler.start()
     launches0 = h.launches
-    dev_ms = timed_steps(step_device, args.steps)              # the `value` region: no profiling events inside
+    dev_ms, (seq, _, lens) = timed_steps(step_device, args.steps)       # the `value` region: no profiling events inside
     launches = h.launches - launches0
-    _, _, lens = step_device()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'seq': seq, 'lens': lens})     # seq is seq_dev: copied before later steps reuse it
     mean_len = lens.float().mean().item()
     # per-stage device times in a separate, profiled pass of the same steps (CUDA-event spans around every stage)
     h.set_profiling(True)
@@ -516,7 +536,7 @@ def main():
     h2.load_weights(sd)
     for _ in range(3):
         step_device(h2)
-    other_ms = timed_steps(lambda: step_device(h2), args.steps)
+    other_ms, _ = timed_steps(lambda: step_device(h2), args.steps)
     run_e2e(h2, 2)
     barrier()
     t0 = time.perf_counter()

@@ -4,8 +4,7 @@ TEST INFRASTRUCTURE ONLY (see oracle/__init__.py): checker for the CUDA kernel i
 
 Follows ub-bonito/bonito/fast5.py: Read.__init__ :88-100 (DAC -> pA scaling, trim, med/MAD normalisation, short reads by
 the noisiest section), trim :149-172, and bonito/util.py med_mad / norm_by_noisiest_section (the helpers fast5.py
-imports).  Pinned against those very functions, imported from /root/reference, by tests/test_cpu_preprocess.py (when the
-tree is present) and through tests/golden/preprocess.npz.
+imports).  Pinned against those very functions through tests/golden/preprocess.npz (tests/test_cpu_preprocess.py).
 
 Arithmetic: float32 throughout, as numpy >= 2 evaluates the reference's expressions (a float32 scalar times a Python
 float stays float32).  The reference's pinned numpy 1.19.5 promoted `median * 1.4826` and the trim threshold to float64

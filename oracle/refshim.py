@@ -2,8 +2,7 @@
 
 TEST INFRASTRUCTURE ONLY (see oracle/__init__.py).  /root/reference does not exist on the
 GPU box: nothing in the ``-m gpu`` tests, ``smoke()`` or ``bench.py`` calls this module.  It is
-used by ``tests/golden/make_golden.py`` (fixture generation) and by the ``not gpu`` tests that
-pin ``oracle.bonito_oracle`` against the reference's own code when the tree is present.
+used by ``tests/golden/make_golden.py`` only (fixture generation).
 
 How: ``bonito/__init__.py`` imports every CLI (mappy, pysam, remora, ...), so ``bonito`` is
 installed as a bare namespace package whose ``__path__`` points at the reference tree; the
