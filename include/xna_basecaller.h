@@ -201,6 +201,17 @@ int xb_adamw_step(float *const *params, float *const *grads, float *const *exp_a
                   const int64_t *numel, int n_tensors, float lr, float beta1, float beta2, float eps, float weight_decay,
                   float max_norm, int64_t step, float *grad_norm, float *scratch, void *stream);
 
+/* Local alignment counts for validation accuracy (util.accuracy, bonito/util.py:402-424): for each pair p, the best local
+ * alignment of query seq[p] (seq_len[p] bytes of row p, rows seq_stride bytes apart) against reference ref[p] under the
+ * contract written in csrc/align.cu (+5 for identical bytes, -4 otherwise, a gap of length k costs 8 + 4 (k - 1), fixed
+ * tie rules).  counts (n_pairs, 5) int32 on the device receives (score, eq, x, ins, del): matching and mismatching
+ * columns, query bases aligned to a gap and reference bases aligned to a gap; all zero for an empty alignment.
+ * seq / ref are letter codes as xb_crf_decode writes them (left-packed rows); seq_len / ref_len are device arrays.
+ * The lengths are copied to the host and checked (0 <= len <= 32767 and len <= row stride, else XB_ERR_ARG), so the
+ * call synchronises the stream once before it enqueues the kernel.  Needs no handle. */
+int xb_align_counts(const int8_t *seq, int seq_stride, const int32_t *seq_len, const int8_t *ref, int ref_stride,
+                    const int32_t *ref_len, int n_pairs, int32_t *counts, void *stream);
+
 /* util.stitch over left-packed chunks (util.py:169-188; crf/basecall.py:15-24): for each read r,
  * concatenates slices of its chunks' packed rows.  chunk_first[r], chunk_count[r], read_len[r]
  * (samples) describe the reads; rows are (n_chunks_total, T) int8; out is (n_reads, out_stride) int8,

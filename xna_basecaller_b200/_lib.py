@@ -27,6 +27,7 @@ SYMBOLS = (
     'xb_set_profiling', 'xb_stage_times', 'xb_crf_head_fwd_exp', 'xb_crf_decode_exp', 'xb_basecall_chunks',
     'xb_crf_logz_s', 'xb_crf_forward_scores_s', 'xb_crf_backward_scores_s', 'xb_crf_posteriors_max',
     'xb_encoder_fwd_train', 'xb_encoder_bwd', 'xb_adamw_step', 'xb_crf_beam_search',
+    'xb_align_counts',
 )
 STAGES = ('conv12_im2col', 'conv3_gemm', 'lstm_inproj_gemm', 'lstm_recurrence', 'crf_head_gemm', 'crf_alpha',
           'crf_backward', 'crf_viterbi', 'train_bptt', 'train_transpose', 'train_weight_grad_gemm', 'train_input_grad_gemm', 'train_head_conv_bwd')
@@ -67,6 +68,7 @@ def load():
     lib.xb_encoder_bwd.argtypes = [vp, vp, ci, vp, vp, ctypes.POINTER(vp), ci, vp]
     lib.xb_adamw_step.argtypes = [ctypes.POINTER(vp), ctypes.POINTER(vp), ctypes.POINTER(vp), ctypes.POINTER(vp),
                                   ctypes.POINTER(ctypes.c_int64), ci, cf, cf, cf, cf, cf, cf, ctypes.c_int64, vp, vp, vp]
+    lib.xb_align_counts.argtypes = [vp, ci, vp, vp, ci, vp, ci, vp, vp]
     lib.xb_crf_beam_search.argtypes = [vp, vp, ci, ci, ci, cf, vp, vp, vp, vp, vp]
     lib.xb_crf_logz_s.argtypes = [vp, vp, ci, ci, ci, vp, vp]
     lib.xb_crf_forward_scores_s.argtypes = [vp, vp, ci, ci, ci, vp, vp]
@@ -103,6 +105,37 @@ def _ptr(t):
 
 def _stream(device):
     return ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+
+
+def align_counts(seq, seq_len, ref, ref_len):
+    """xb_align_counts: local alignment counts of seq[p, :seq_len[p]] (query) against ref[p, :ref_len[p]] for every row p.
+    seq / ref: (N, *) int8 CUDA tensors with unit column stride (left-packed rows, as the decode writes them); lengths (N,)
+    on the same device.  Returns (N, 5) int32 on the device: (score, eq, x, ins, del).  Synchronises the current stream
+    once (the library checks the lengths on the host)."""
+    if not torch.cuda.is_available():
+        raise RuntimeError('xna_basecaller_b200 needs a CUDA device (sm_100a); there is no CPU fallback')
+    lib = load()
+    dev = seq.device
+    if dev.type != 'cuda' or ref.device != dev:
+        raise ValueError('align_counts takes CUDA tensors on one device')
+    if seq.dtype != torch.int8 or ref.dtype != torch.int8 or seq.dim() != 2 or ref.dim() != 2 or len(seq) != len(ref):
+        raise ValueError('seq and ref must be (N, *) int8 with the same N')
+    if seq.stride(1) != 1:
+        seq = seq.contiguous()
+    if ref.stride(1) != 1:
+        ref = ref.contiguous()
+    n = seq.shape[0]
+    sl = seq_len.to(dev, torch.int32).contiguous()
+    rl = ref_len.to(dev, torch.int32).contiguous()
+    if sl.numel() != n or rl.numel() != n:
+        raise ValueError('one length per row')
+    counts = torch.empty(n, 5, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        rc = lib.xb_align_counts(_ptr(seq), seq.stride(0), _ptr(sl), _ptr(ref), ref.stride(0), _ptr(rl), n, _ptr(counts),
+                                 _stream(dev))
+    if rc != 0:
+        raise RuntimeError('xb_align_counts failed (%d): %s' % (rc, lib.xb_last_error(None).decode()))
+    return counts
 
 
 class Handle:

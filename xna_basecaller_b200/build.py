@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libxna_b200.so')
-SOURCES = ["xb_api.cu", "crf_decode.cu", "crf_decode_lin.cu", 'conv_stem.cu', 'gemm_tc.cu', 'conv3_gemm.cu', 'lstm_persistent.cu', 'inproj_gemm.cu', 'misc_kernels.cu', 'preprocess.cu', 'train_bwd.cu', 'lstm_bptt.cu', 'wgrad_gemm.cu', 'optim.cu', 'beam_search.cu']
+SOURCES = ["xb_api.cu", "crf_decode.cu", "crf_decode_lin.cu", 'conv_stem.cu', 'gemm_tc.cu', 'conv3_gemm.cu', 'lstm_persistent.cu', 'inproj_gemm.cu', 'misc_kernels.cu', 'preprocess.cu', 'train_bwd.cu', 'lstm_bptt.cu', 'wgrad_gemm.cu', 'optim.cu', 'beam_search.cu', 'align.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC', '-cudart', 'static']
 

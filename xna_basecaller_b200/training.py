@@ -5,12 +5,18 @@ clip at 2.0 -> AdamW step.  Here the forward / loss / backward run through libxn
 xb_ctc_crf_loss_fwd / _bwd, xb_encoder_bwd behind torch.autograd.Function nodes) and the clip + AdamW update is one fused
 multi-tensor call (xb_adamw_step).  Gradients are transported as bf16 with fp32 accumulation, so there is no GradScaler
 (`use_amp` is accepted for signature compatibility and ignored).  Data loading / augmentation stay with the caller.
+
+validate_one_step / validate_one_epoch (training.py:159-181) score the validation chunks on the device: forward, loss,
+one CRF decode, and the local alignment of every decode against its reference (xb_align_counts) -- only the strings,
+the loss and 20 bytes of alignment counts per chunk come back to the host.
 """
 import ctypes
 
+import numpy as np
 import torch
 
 from . import _lib
+from .util import _accuracy
 from .schedule import linear_warmup_cosine_decay
 
 
@@ -66,8 +72,9 @@ class AdamW(torch.optim.Optimizer):
 
 
 class Trainer:
-    """Trainer.train_one_step / init_optimizer / get_lr_scheduler of the reference; the epoch loops, checkpoints and
-    validation accuracy stay in the reference's own training.py, which can drive this object unchanged."""
+    """Trainer.train_one_step / validate_one_step / validate_one_epoch / init_optimizer / get_lr_scheduler of the
+    reference; the epoch loop and checkpoints stay in the reference's own training.py, which can drive this object
+    unchanged."""
 
     def __init__(self, model, device, train_loader=None, valid_loader=None, criterion=None, use_amp=True,
                  lr_scheduler_fn=None, restore_optim=False, save_optim_every=10, grad_accum_split=1):
@@ -102,3 +109,36 @@ class Trainer:
             losses = {k: (v.item() if losses is None else v.item() + losses[k]) for k, v in losses_.items()}
         grad_norm = self.optimizer.step(max_norm=2.0).item()
         return losses, grad_norm
+
+    def validate_one_step(self, batch):
+        """(seqs, refs, accs, losses) of one validation batch: the decoded strings, the references (decode_ref of the
+        targets), accuracy(ref, seq, min_coverage=0.5) per chunk (0 for an empty decode) and the loss."""
+        data, targets, lengths = batch[:3]
+        self.model.eval()
+        with torch.no_grad():
+            targets, lengths = targets.to(self.device), lengths.to(self.device)
+            scores = self.model(data.to(self.device)).to(torch.float32)
+            losses = self.criterion(scores, targets, lengths)
+            losses = {k: v.item() for k, v in losses.items()} if isinstance(losses, dict) else losses.item()
+            seq, _, seq_len = self.model.seqdist.decode_packed(scores)
+            # reference rows on the device: the non-zero labels moved to the front in order, then letters gathered
+            packed = targets.gather(1, torch.sort((targets == 0).to(torch.int8), dim=1, stable=True).indices)
+            letters = torch.tensor(list(''.join(self.model.alphabet).encode()), dtype=torch.uint8, device=scores.device)
+            ref = letters[packed].view(torch.int8)
+            ref_len = (targets != 0).sum(1).to(torch.int32)
+            counts = _lib.align_counts(seq, seq_len, ref, ref_len).cpu().tolist()
+            seq_h, seq_len_h = seq.cpu().numpy(), seq_len.cpu().tolist()
+            ref_h, ref_len_h = ref.cpu().numpy(), ref_len.cpu().tolist()
+        seqs = [seq_h[i, :n].astype('u1').tobytes().decode() for i, n in enumerate(seq_len_h)]
+        refs = [ref_h[i, :n].astype('u1').tobytes().decode() for i, n in enumerate(ref_len_h)]
+        accs = [_accuracy(c, rl, False, 0.5) if sl else 0. for c, rl, sl in zip(counts, ref_len_h, seq_len_h)]
+        return seqs, refs, accs, losses
+
+    def validate_one_epoch(self):
+        """(mean loss, mean accuracy, median accuracy) over valid_loader."""
+        self.model.eval()
+        with torch.no_grad():
+            seqs, refs, accs, losses = zip(*(self.validate_one_step(batch) for batch in self.valid_loader))
+        accs = sum(accs, [])
+        loss = np.mean([(x['loss'] if isinstance(x, dict) else x) for x in losses])
+        return loss, np.mean(accs), np.median(accs)

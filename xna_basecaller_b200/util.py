@@ -1,7 +1,7 @@
 """Host-side helpers of the basecalling path, with the reference's names and argument meaning
 (ub-bonito/bonito/util.py): chunk (:152-166), stitch (:169-188), batchify / unbatchify (:191-225),
 concat / select_range / size (:66-102), half_supported (:105-112), load_symbol (:228-239),
-match_names (:242-258) and load_model (:261-366).
+match_names (:242-258), load_model (:261-366), decode_ref and accuracy (:402-424).
 
 These are bookkeeping over host arrays (rows a-1, a-2, a-11 of SURVEY.md section 8); the arithmetic of the
 path runs in libxna_b200.so.  The read-sharded GPU pipeline (xna_basecaller_b200.pipeline) does the same
@@ -225,3 +225,48 @@ def load_model(dirname, device, weights=None, half=None, chunksize=None, batchsi
     model.eval()
     model.to(device)
     return model
+
+
+def decode_ref(encoded, labels):
+    """The letters of the non-zero (1-based) labels of one target row."""
+    return ''.join(labels[e] for e in encoded.tolist() if e)
+
+
+def _accuracy(counts, ref_len, balanced, min_coverage):
+    """The reference's accuracy expressions on one pair's (score, eq, x, ins, del), in Python float arithmetic.  The
+    coverage of the reference counts the alignment's columns, gaps included.  An empty alignment, or an empty reference,
+    scores 0 (the reference would divide by zero)."""
+    _, eq, x, ins, dl = (int(c) for c in counts)
+    r_coverage = (eq + x + ins + dl) / ref_len if ref_len else 0.0
+    if r_coverage < min_coverage:
+        return 0.0
+    if balanced:
+        den = eq + x + dl
+        return (eq - ins) / den * 100 if den else 0.0
+    den = eq + ins + x + dl
+    return eq / den * 100 if den else 0.0
+
+
+def accuracy_batch(seq, seq_len, ref, ref_len, balanced=False, min_coverage=0.0):
+    """accuracy() of every row pair of device tensors: seq / ref (N, *) int8 left-packed letter rows, lengths (N,).
+    The alignments run in one xb_align_counts call; only the (N, 5) counts come back.  Returns a list of N floats."""
+    from ._lib import align_counts
+    counts = align_counts(seq, seq_len, ref, ref_len).cpu().tolist()
+    ref_lens = ref_len.cpu().tolist()
+    return [_accuracy(c, rl, balanced, min_coverage) for c, rl in zip(counts, ref_lens)]
+
+
+def accuracy(ref, seq, balanced=False, min_coverage=0.0):
+    """Percent identity of the best local alignment of `seq` against `ref` (host strings), computed on the current CUDA
+    device: 100 * '=' / ('=' + 'I' + 'X' + 'D'), or with balanced 100 * ('=' - 'I') / ('=' + 'X' + 'D'); 0 when the
+    alignment covers less than min_coverage of ref.  Scoring and tie rules: csrc/align.cu."""
+    dev = torch.device('cuda', torch.cuda.current_device()) if torch.cuda.is_available() else None
+    if dev is None:
+        raise RuntimeError('xna_basecaller_b200 needs a CUDA device (sm_100a); there is no CPU fallback')
+    s, r = seq.encode(), ref.encode()
+    rows = torch.zeros(2, max(len(s), len(r), 1), dtype=torch.uint8)
+    rows[0, :len(s)] = torch.frombuffer(bytearray(s), dtype=torch.uint8) if s else rows[0, :0]
+    rows[1, :len(r)] = torch.frombuffer(bytearray(r), dtype=torch.uint8) if r else rows[1, :0]
+    rows = rows.view(torch.int8).to(dev)
+    lens = torch.tensor([[len(s)], [len(r)]], dtype=torch.int32, device=dev)
+    return accuracy_batch(rows[:1], lens[0], rows[1:], lens[1], balanced, min_coverage)[0]
