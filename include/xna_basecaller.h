@@ -192,6 +192,22 @@ int xb_encoder_fwd_train(xb_handle *h, const void *signal, int sig_dtype, int N,
 int xb_encoder_bwd(xb_handle *h, const void *signal, int sig_dtype, const float *scores, const float *dscores,
                    float *const *grads, int n_tensors, void *stream);
 
+/* Dropout in the training step (rnn_encoder(drop_rate_bottom=...), crf/model.py): the forward of xb_encoder_fwd_train with
+ * torch.nn.Dropout(p[s]) applied at XB_DROPOUT_SITES sites, in the order the reference applies them:
+ *   0 conv1 output, 1 conv2 output, 2 conv3 output, 3..6 outputs of LSTM layers 0..3.
+ * p is a host array of XB_DROPOUT_SITES probabilities, each 0 <= p < 1 (else XB_ERR_ARG); NULL or all zero is exactly
+ * xb_encoder_fwd_train (same kernels, same bits).  The mask is a pure function of (seed, site, element index): Philox4x32-10
+ * keyed by the 64-bit seed, written out in csrc/xb_dropout.cuh.  Kept values are scaled by (float)(1 / (1 - p)), dropped
+ * ones are 0 -- torch.nn.Dropout's distribution, not torch's random stream.  The handle records (p, seed), and the next
+ * xb_encoder_bwd regenerates the same masks; its signature does not change. */
+#define XB_DROPOUT_SITES 7
+int xb_encoder_fwd_train_dropout(xb_handle *h, const void *signal, int sig_dtype, int N, int L, const float *p, uint64_t seed,
+                                 float *scores, void *stream);
+
+/* The keep flags (1 kept, 0 dropped) of elements 0 .. n-1 of one dropout site under (seed, p), computed on the current
+ * device by the device function the training kernels use.  keep: n bytes of device memory.  Needs no handle. */
+int xb_dropout_keep(uint64_t seed, int site, float p, int64_t n, uint8_t *keep, void *stream);
+
 /* The optimiser half of Trainer.train_one_step (training.py:112-115): torch.nn.utils.clip_grad_norm_(max_norm) followed by
  * one torch.optim.AdamW step (training.py:183-184; decoupled weight decay, bias-corrected moments) over n_tensors fp32
  * tensors given as host arrays of device pointers.  max_norm <= 0 disables clipping; step >= 1 counts this update;

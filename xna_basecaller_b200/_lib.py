@@ -16,6 +16,7 @@ XB_FLAG_NO_ENCODER = 2
 XB_FLAG_TRAIN = 8
 XB_SIG_F32, XB_SIG_F16, XB_SIG_I16 = 0, 1, 2
 NUM_WEIGHTS = 28
+DROPOUT_SITES = 7       # conv1, conv2, conv3 outputs, outputs of LSTM layers 0..3 (XB_DROPOUT_SITES)
 
 # every symbol include/xna_basecaller.h declares (tests check that the library exports them all)
 SYMBOLS = (
@@ -27,7 +28,7 @@ SYMBOLS = (
     'xb_set_profiling', 'xb_stage_times', 'xb_crf_head_fwd_exp', 'xb_crf_decode_exp', 'xb_basecall_chunks',
     'xb_crf_logz_s', 'xb_crf_forward_scores_s', 'xb_crf_backward_scores_s', 'xb_crf_posteriors_max',
     'xb_encoder_fwd_train', 'xb_encoder_bwd', 'xb_adamw_step', 'xb_crf_beam_search',
-    'xb_align_counts',
+    'xb_align_counts', 'xb_encoder_fwd_train_dropout', 'xb_dropout_keep',
 )
 STAGES = ('conv12_im2col', 'conv3_gemm', 'lstm_inproj_gemm', 'lstm_recurrence', 'crf_head_gemm', 'crf_alpha',
           'crf_backward', 'crf_viterbi', 'train_bptt', 'train_transpose', 'train_weight_grad_gemm', 'train_input_grad_gemm', 'train_head_conv_bwd')
@@ -66,6 +67,8 @@ def load():
     lib.xb_crf_posteriors.argtypes = [vp, vp, ci, ci, vp, vp]
     lib.xb_encoder_fwd_train.argtypes = [vp, vp, ci, ci, ci, vp, vp]
     lib.xb_encoder_bwd.argtypes = [vp, vp, ci, vp, vp, ctypes.POINTER(vp), ci, vp]
+    lib.xb_encoder_fwd_train_dropout.argtypes = [vp, vp, ci, ci, ci, ctypes.POINTER(cf), ctypes.c_uint64, vp, vp]
+    lib.xb_dropout_keep.argtypes = [ctypes.c_uint64, ci, cf, ctypes.c_int64, vp, vp]
     lib.xb_adamw_step.argtypes = [ctypes.POINTER(vp), ctypes.POINTER(vp), ctypes.POINTER(vp), ctypes.POINTER(vp),
                                   ctypes.POINTER(ctypes.c_int64), ci, cf, cf, cf, cf, cf, cf, ctypes.c_int64, vp, vp, vp]
     lib.xb_align_counts.argtypes = [vp, ci, vp, vp, ci, vp, ci, vp, vp]
@@ -136,6 +139,35 @@ def align_counts(seq, seq_len, ref, ref_len):
     if rc != 0:
         raise RuntimeError('xb_align_counts failed (%d): %s' % (rc, lib.xb_last_error(None).decode()))
     return counts
+
+
+def dropout_probabilities(p):
+    """The XB_DROPOUT_SITES probabilities as a list of floats; ValueError unless there are seven, each 0 <= p < 1."""
+    p = [float(v) for v in p]
+    if len(p) != DROPOUT_SITES:
+        raise ValueError('dropout needs %d probabilities (one per site), got %d' % (DROPOUT_SITES, len(p)))
+    for site, v in enumerate(p):
+        if not (0.0 <= v < 1.0 and ctypes.c_float(v).value < 1.0):      # the library takes p as a float
+            raise ValueError('dropout probability of site %d must lie in [0, 1), got %r' % (site, v))
+    return p
+
+
+def dropout_keep(seed, site, p, n, device=None):
+    """xb_dropout_keep: the keep flags (n,) bool on the device of elements 0 .. n-1 of dropout site `site` under (seed, p),
+    from the device function the training kernels use."""
+    if not torch.cuda.is_available():
+        raise RuntimeError('xna_basecaller_b200 needs a CUDA device (sm_100a); there is no CPU fallback')
+    lib = load()
+    if not 0 <= int(site) < DROPOUT_SITES:
+        raise ValueError('dropout site %r out of range' % (site,))
+    p = dropout_probabilities([p if s == int(site) else 0.0 for s in range(DROPOUT_SITES)])[int(site)]
+    dev = torch.device('cuda', torch.cuda.current_device()) if device is None else torch.device(device)
+    keep = torch.empty(int(n), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        rc = lib.xb_dropout_keep(int(seed) & 0xffffffffffffffff, int(site), float(p), int(n), _ptr(keep), _stream(dev))
+    if rc != 0:
+        raise RuntimeError('xb_dropout_keep failed (%d): %s' % (rc, lib.xb_last_error(None).decode()))
+    return keep.bool()
 
 
 class Handle:
@@ -305,13 +337,25 @@ class Handle:
                     for k in ('weight_ih_l0', 'weight_hh_l0', 'bias_ih_l0', 'bias_hh_l0')] +
                    ['encoder.9.linear.weight', 'encoder.9.linear.bias'])
 
-    def encoder_train(self, signal):
-        """Training forward: scores (T, N, C*NZ) fp32; the handle keeps what encoder_backward needs."""
+    def encoder_train(self, signal, dropout_p=None, seed=None):
+        """Training forward: scores (T, N, C*NZ) fp32; the handle keeps what encoder_backward needs.
+        dropout_p: None, or the probabilities of the DROPOUT_SITES dropout sites (xb_encoder_fwd_train_dropout) with the
+        64-bit `seed` of their masks; encoder_backward applies the same masks."""
+        if dropout_p is not None:
+            dropout_p = dropout_probabilities(dropout_p)
+            if seed is None:
+                raise ValueError('dropout needs a seed')
         signal, code = self._sig(signal.to(self.device))
         N, L = signal.shape
         scores = torch.empty(L // 5, N, self.C * self.NZ, dtype=torch.float32, device=self.device)
-        self._check(self.lib.xb_encoder_fwd_train(self.h, _ptr(signal), code, N, L, _ptr(scores), _stream(self.device)),
-                    'xb_encoder_fwd_train')
+        if dropout_p is None:
+            self._check(self.lib.xb_encoder_fwd_train(self.h, _ptr(signal), code, N, L, _ptr(scores), _stream(self.device)),
+                        'xb_encoder_fwd_train')
+        else:
+            p = (ctypes.c_float * DROPOUT_SITES)(*dropout_p)
+            self._check(self.lib.xb_encoder_fwd_train_dropout(self.h, _ptr(signal), code, N, L, p,
+                                                              int(seed) & 0xffffffffffffffff, _ptr(scores),
+                                                              _stream(self.device)), 'xb_encoder_fwd_train_dropout')
         self._train_keep = (signal, code, scores)
         return scores
 

@@ -9,7 +9,12 @@
 // One CTA = one chunk x 32 output steps: stages the 182 input samples it needs (halo included) in shared
 // memory with coalesced loads, computes 178 conv1 and 174 conv2 positions in fp32, keeps conv2 in 16-bit
 // channel-last form in shared memory, and writes the 32 overlapping 640-byte rows with 16-byte stores.
+//
+// DROP (the training forward and backward with dropout sites 0 / 1 active, xb_dropout.cuh): the fp32 conv1 values are
+// masked before conv2 reads them and the conv2 values before they are rounded into the rows.  The mask is a function of
+// the element index alone, so the halo positions a CTA shares with its neighbours get the same bits in both CTAs.
 #include "xb_common.cuh"
+#include "xb_dropout.cuh"
 
 namespace {
 
@@ -26,11 +31,11 @@ template <> __device__ __forceinline__ float load_sig<float>(const float *p, siz
 template <> __device__ __forceinline__ float load_sig<__half>(const __half *p, size_t i) { return __half2float(p[i]); }
 template <> __device__ __forceinline__ float load_sig<int16_t>(const int16_t *p, size_t i) { return (float)p[i]; }
 
-template <bool BF16, typename SIG>
+template <bool BF16, bool DROP, typename SIG>
 __global__ void __launch_bounds__(THREADS)
 conv12_im2col_kernel(const SIG *__restrict__ signal, int L, int T, const float *__restrict__ w1,
                      const float *__restrict__ b1, const float *__restrict__ w2, const float *__restrict__ b2,
-                     uint16_t *__restrict__ rows) {
+                     uint16_t *__restrict__ rows, const xb_dropout drop) {
     using X = xb16<BF16>;
     __shared__ float sx[NPX];
     __shared__ float s1[NP1][4];
@@ -59,6 +64,7 @@ conv12_im2col_kernel(const SIG *__restrict__ signal, int L, int T, const float *
 #pragma unroll
             for (int k = 0; k < 5; k++) v = fmaf(sw1[ch * 5 + k], sx[pos + k], v);
             v = swishf(v);
+            if (DROP && drop.on(0)) v = xb_dropout_apply(drop, 0, ((uint64_t)b * 4 + ch) * L + p, v);
         }
         s1[pos][ch] = v;
     }
@@ -73,6 +79,7 @@ conv12_im2col_kernel(const SIG *__restrict__ signal, int L, int T, const float *
 #pragma unroll
                 for (int k = 0; k < 5; k++) v = fmaf(sw2[(ch * 4 + ci) * 5 + k], s1[pos + k][ci], v);
             v = swishf(v);
+            if (DROP && drop.on(1)) v = xb_dropout_apply(drop, 1, ((uint64_t)b * 16 + ch) * L + p, v);
         }
         typename X::T hv = X::from(v);
         s2[pos][ch] = *reinterpret_cast<uint16_t *>(&hv);
@@ -90,24 +97,29 @@ conv12_im2col_kernel(const SIG *__restrict__ signal, int L, int T, const float *
 }
 
 template <bool BF16, typename SIG>
-int launch(xb_handle *h, const void *signal, int N, int L, cudaStream_t s) {
+int launch(xb_handle *h, const void *signal, int N, int L, const xb_dropout *drop, cudaStream_t s) {
     const int T = L / XB_STRIDE;
     dim3 grid((T + TT - 1) / TT, N);
-    conv12_im2col_kernel<BF16, SIG><<<grid, THREADS, 0, s>>>(reinterpret_cast<const SIG *>(signal), L, T, h->conv1_w,
-                                                             h->conv1_b, h->conv2_w, h->conv2_b,
-                                                             reinterpret_cast<uint16_t *>(h->c2));
+    const SIG *sig = reinterpret_cast<const SIG *>(signal);
+    uint16_t *rows = reinterpret_cast<uint16_t *>(h->c2);
+    if (drop && (drop->on(0) || drop->on(1)))
+        conv12_im2col_kernel<BF16, true, SIG><<<grid, THREADS, 0, s>>>(sig, L, T, h->conv1_w, h->conv1_b, h->conv2_w,
+                                                                      h->conv2_b, rows, *drop);
+    else
+        conv12_im2col_kernel<BF16, false, SIG><<<grid, THREADS, 0, s>>>(sig, L, T, h->conv1_w, h->conv1_b, h->conv2_w,
+                                                                       h->conv2_b, rows, xb_dropout());
     XB_LAUNCH_CHECK(h);
     return XB_OK;
 }
 
 }  // namespace
 
-// signal (N, L) -> h->c2 = im2col rows (N*T, 320) 16-bit
-int xb_conv12_im2col(xb_handle *h, const void *signal, int sig_dtype, int N, int L, cudaStream_t s) {
+// signal (N, L) -> h->c2 = im2col rows (N*T, 320) 16-bit; drop (may be NULL): the masks of dropout sites 0 and 1
+int xb_conv12_im2col(xb_handle *h, const void *signal, int sig_dtype, int N, int L, cudaStream_t s, const xb_dropout *drop) {
     switch (sig_dtype) {        // activations are fp16 in both weight modes
-        case XB_SIG_F32: return launch<false, float>(h, signal, N, L, s);
-        case XB_SIG_F16: return launch<false, __half>(h, signal, N, L, s);
-        case XB_SIG_I16: return launch<false, int16_t>(h, signal, N, L, s);
+        case XB_SIG_F32: return launch<false, float>(h, signal, N, L, drop, s);
+        case XB_SIG_F16: return launch<false, __half>(h, signal, N, L, drop, s);
+        case XB_SIG_I16: return launch<false, int16_t>(h, signal, N, L, drop, s);
     }
     return xb_fail(h, XB_ERR_ARG, "unknown signal dtype %d", sig_dtype);
 }

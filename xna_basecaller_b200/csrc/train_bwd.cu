@@ -24,10 +24,26 @@
 // Measured at N = 512, T = 800 (profiles/r02_config5_train_step_v5.json): 154 ms per training step, of which the 4000 BPTT
 // steps take ~69 ms (17.3 us each: ~10 us of main loop bound by one SM's L2 ingest of its 1.15 MB of operands, the rest
 // epilogue and the kernel hand-over), the K = T*N weight-gradient GEMMs ~20 ms (wgrad_gemm.cu) and the forward ~25 ms.
+//
+// Dropout (xb_encoder_fwd_train_dropout; mask contract in xb_dropout.cuh).  Nothing is stored: every pass that needs a mask
+// regenerates it from (seed, site, element index).
+//   sites 0, 1  conv12_im2col's masked form in the forward and in the backward's recomputation of the rows; conv2_bwd_kernel
+//               masks its recomputed conv1 output (site 0), the incoming conv2 gradient (site 1) and the conv1 gradient
+//               it scatters (site 0).
+//   site 2      applied in place to x[0] (the conv3 backward recomputes its pre-activation from the rows, so the
+//               undropped x[0] is never needed again); the gradient w.r.t. x[0] is masked before EPI_CONV3_BWD.
+//   sites 3..6  x[l+1] keeps the undropped output of LSTM l (dW_hh of layer l reads it through the time-shifted view);
+//               layer l+1's input projection reads a dropped copy in the scratch buffer xd.  The backward transposes x[l+1]
+//               twice: plainly into XT (for dW_hh of layer l) and through the mask into xd (for dW_ih of layer l+1),
+//               and masks dy (the gradient w.r.t. the dropped input) before the BPTT of layer l consumes it.
+// With every p = 0 none of these launches happens and the step is bit for bit the step without dropout.
 #include "xb_common.cuh"
+#include "xb_dropout.cuh"
 #include "xb_gemm.cuh"
 
-int xb_conv12_im2col(xb_handle *h, const void *signal, int sig_dtype, int N, int L, cudaStream_t s);
+int xb_conv12_im2col(xb_handle *h, const void *signal, int sig_dtype, int N, int L, cudaStream_t s, const xb_dropout *drop);
+int xb_conv_stem_fwd_dropout(xb_handle *h, const void *signal, int sig_dtype, int N, int L, void *out_tnc,
+                             const xb_dropout *drop, void *stream);
 int xb_lstm_recurrence_persistent(xb_handle *h, int layer, void *y_tnc, int T, int N, int reverse, cudaStream_t s, void *save);
 int xb_lstm_wgrad_launch(xb_handle *h, const void *dzT, const void *xT, const void *yT, int T, int N, bool reverse, float *g_wih,
                          float *g_whh, cudaStream_t s);
@@ -48,6 +64,9 @@ struct xb_train_ws {
     float *dcstate = nullptr;      // (N,768)
     float *dc2 = nullptr;          // (N, L, 16) fp32: gradient w.r.t. the conv2 output (post-activation)
     float *dc1 = nullptr;          // (N, L, 4) fp32
+    void *xd = nullptr;            // dropout sites 3..6 only: forward (T,N,768) fp16 dropped copy of the next layer's input;
+                                   // backward (768,TN) bf16 transposed dropped input of the layer being differentiated
+    xb_dropout drop;               // (p, seed) of the last forward
 };
 
 namespace {
@@ -89,6 +108,19 @@ __global__ void colsum_kernel(const __nv_bfloat16 *__restrict__ in, int R, int C
         for (int i = 1; i < 8; i++) s += part[i][threadIdx.x];
         atomicAdd(out + c, s);
     }
+}
+
+// dropout of a 16-bit tensor whose element index is its flat offset (sites 2..6): eight elements per iteration; in == out
+// is allowed
+template <bool BF16>
+__global__ void __launch_bounds__(256) dropout16_kernel(const uint4 *in, uint4 *out, size_t n8, const xb_dropout drop, int site) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += (size_t)gridDim.x * blockDim.x)
+        out[i] = xb_dropout8<BF16>(drop, site, i * 8, in[i]);
+}
+
+__global__ void dropout_keep_kernel(const xb_dropout drop, int site, int64_t n, uint8_t *__restrict__ keep) {
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x)
+        keep[e] = xb_dropout_keep(drop, site, (uint64_t)e) ? 1 : 0;
 }
 
 // LinearCRFEncoder backward through scale * tanh and the blank expansion (nn.py:117-129): for head row j = c * n_base + b,
@@ -134,11 +166,12 @@ __device__ __forceinline__ float dswishf(float x) { const float sg = 1.0f / (1.0
 // conv2 backward: recomputes conv1 (and its swish) and the conv2 pre-activation from the signal, turns da2 into
 // d pre2, accumulates dW2 (16,4,5), db2 (16) and scatters the gradient w.r.t. the conv1 output a1 into da1 (N, L, 4).
 // One block per (chunk, tile of 256 positions); block-level reductions, then one atomicAdd per weight and block.
-template <typename SIG>
+// DROP: conv2's input is the masked conv1 output (site 0) and da2 is the gradient w.r.t. the masked conv2 output (site 1).
+template <bool DROP, typename SIG>
 __global__ void __launch_bounds__(256)
 conv2_bwd_kernel(const SIG *__restrict__ signal, int L, const float *__restrict__ w1, const float *__restrict__ b1,
                  const float *__restrict__ w2, const float *__restrict__ b2, const float *__restrict__ da2,
-                 float *__restrict__ da1, float *__restrict__ dw2, float *__restrict__ db2) {
+                 float *__restrict__ da1, float *__restrict__ dw2, float *__restrict__ db2, const xb_dropout drop) {
     constexpr int TP = 256;
     __shared__ float sx[TP + 8];          // signal positions p0-4 .. p0+TP+3
     __shared__ float a1[TP + 4][4];       // conv1 output (post swish) positions p0-2 .. p0+TP+1
@@ -163,6 +196,7 @@ conv2_bwd_kernel(const SIG *__restrict__ signal, int L, const float *__restrict_
 #pragma unroll
             for (int k = 0; k < 5; k++) v = fmaf(sw1[ch * 5 + k], sx[pos + k], v);
             v = swishf(v);
+            if (DROP && drop.on(0)) v = xb_dropout_apply(drop, 0, ((uint64_t)b * 4 + ch) * L + p, v);
         }
         a1[pos][ch] = v;              // zero outside [0, L): conv2's zero padding
     }
@@ -177,7 +211,9 @@ conv2_bwd_kernel(const SIG *__restrict__ signal, int L, const float *__restrict_
             for (int ci = 0; ci < 4; ci++)
 #pragma unroll
                 for (int k = 0; k < 5; k++) pre = fmaf(sw2[(o * 4 + ci) * 5 + k], a1[pos + k][ci], pre);
-            g = da2[((size_t)b * L + p) * 16 + o] * dswishf(pre);
+            g = da2[((size_t)b * L + p) * 16 + o];
+            if (DROP && drop.on(1)) g = xb_dropout_apply(drop, 1, ((uint64_t)b * 16 + o) * L + p, g);
+            g *= dswishf(pre);
         }
         dp2[pos][o] = g;
     }
@@ -207,6 +243,7 @@ conv2_bwd_kernel(const SIG *__restrict__ signal, int L, const float *__restrict_
 #pragma unroll
                 for (int o = 0; o < 16; o++) s = fmaf(sw2[(o * 4 + ci) * 5 + k], dp2[pp][o], s);
         }
+        if (DROP && drop.on(0)) s = xb_dropout_apply(drop, 0, ((uint64_t)b * 4 + ci) * L + q, s);
         atomicAdd(da1 + ((size_t)b * L + q) * 4 + ci, s);
     }
 }
@@ -272,9 +309,12 @@ int colsum(xb_handle *h, const void *in, int R, int C, int ld, float *out, cudaS
 // transposed tile is written and read as words (pitch 33: the read side is conflict free, the write side two-way).  Each
 // CTA walks a slab of row tiles; with COLSUM it also accumulates the column sums of its slab (the bias gradients) and adds
 // them to colsum_out once -- the separate colsum pass over the same 2.5 GB is gone.
-template <bool IN_BF16, bool COLSUM>
+// DROP (fp16 input with ld_in == C): the input is masked by dropout site `site` (element index r * C + c) on the way in,
+// rounded to fp16 as the forward's dropped copy was, then converted -- the transposed dropped copy without storing it.
+template <bool IN_BF16, bool COLSUM, bool DROP = false>
 __global__ void __launch_bounds__(256) transpose16v_kernel(const uint16_t *__restrict__ in, int R, int C, int ld_in,
-                                                           __nv_bfloat16 *__restrict__ out, float *__restrict__ colsum_out) {
+                                                           __nv_bfloat16 *__restrict__ out, float *__restrict__ colsum_out,
+                                                           const xb_dropout drop = xb_dropout(), int site = 0) {
     __shared__ uint32_t tileT[64][33];
     const int t = threadIdx.x;
     const int c0 = blockIdx.x * 64;
@@ -297,6 +337,10 @@ __global__ void __launch_bounds__(256) transpose16v_kernel(const uint16_t *__res
             if (c < C) {
                 if (r < R) a = *reinterpret_cast<const uint4 *>(in + (size_t)r * ld_in + c);
                 if (r + 1 < R) b = *reinterpret_cast<const uint4 *>(in + (size_t)(r + 1) * ld_in + c);
+                if (DROP) {
+                    if (r < R) a = xb_dropout8<IN_BF16>(drop, site, (uint64_t)r * C + c, a);
+                    if (r + 1 < R) b = xb_dropout8<IN_BF16>(drop, site, (uint64_t)(r + 1) * C + c, b);
+                }
             }
             const uint32_t av[4] = {to_bf16(a.x), to_bf16(a.y), to_bf16(a.z), to_bf16(a.w)};
             const uint32_t bv[4] = {to_bf16(b.x), to_bf16(b.y), to_bf16(b.z), to_bf16(b.w)};
@@ -334,30 +378,47 @@ __global__ void __launch_bounds__(256) transpose16v_kernel(const uint16_t *__res
     }
 }
 
-// colsum_out != nullptr: also the column sums of `in` (fp32, zeroed here)
+// colsum_out != nullptr: also the column sums of `in` (fp32, zeroed here).  drop != nullptr: transpose `in` (fp16, ld_in == C)
+// masked by dropout site `site`
 int transpose_to_bf16(xb_handle *h, const void *in, int R, int C, int ld_in, bool in_bf16, void *out, cudaStream_t s,
-                      float *colsum_out = nullptr) {
+                      float *colsum_out = nullptr, const xb_dropout *drop = nullptr, int site = 0) {
     const uint16_t *src = reinterpret_cast<const uint16_t *>(in);
     __nv_bfloat16 *dst = reinterpret_cast<__nv_bfloat16 *>(out);
     xb_stage_timer tm(h, XB_ST_TRAIN_TRANSPOSE, s);
+    if (drop && (in_bf16 || colsum_out || ld_in != C))
+        return xb_fail(h, XB_ERR_ARG, "the masked transposition takes a dense fp16 tensor and takes no column sums");
     if (R % 8 == 0 && C % 8 == 0 && ld_in % 8 == 0 && (reinterpret_cast<uintptr_t>(in) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0) {
         const int tiles = (R + 63) / 64, ctiles = (C + 63) / 64;
         int slabs = (h->num_sms * 12 + ctiles - 1) / ctiles;  // ~12 CTAs per SM over the whole grid
         if (slabs > tiles) slabs = tiles;
         dim3 grid(ctiles, slabs);
         if (colsum_out) XB_CUDA(h, cudaMemsetAsync(colsum_out, 0, (size_t)C * sizeof(float), s));
-        if (in_bf16 && colsum_out) transpose16v_kernel<true, true><<<grid, 256, 0, s>>>(src, R, C, ld_in, dst, colsum_out);
+        if (drop) transpose16v_kernel<false, false, true><<<grid, 256, 0, s>>>(src, R, C, ld_in, dst, nullptr, *drop, site);
+        else if (in_bf16 && colsum_out) transpose16v_kernel<true, true><<<grid, 256, 0, s>>>(src, R, C, ld_in, dst, colsum_out);
         else if (in_bf16) transpose16v_kernel<true, false><<<grid, 256, 0, s>>>(src, R, C, ld_in, dst, nullptr);
         else if (colsum_out) return xb_fail(h, XB_ERR_ARG, "column sums are taken of bf16 gradients only");
         else transpose16v_kernel<false, false><<<grid, 256, 0, s>>>(src, R, C, ld_in, dst, nullptr);
         XB_LAUNCH_CHECK(h);
         return XB_OK;
     }
+    if (drop) return xb_fail(h, XB_ERR_ARG, "the masked transposition needs 16-byte aligned rows");
     dim3 grid((C + 31) / 32, (R + 31) / 32), block(32, 8);
     if (in_bf16) transpose16_kernel<true><<<grid, block, 0, s>>>(src, R, C, ld_in, dst);
     else transpose16_kernel<false><<<grid, block, 0, s>>>(src, R, C, ld_in, dst);
     XB_LAUNCH_CHECK(h);
     if (colsum_out) return colsum(h, in, R, C, ld_in, colsum_out, s);
+    return XB_OK;
+}
+
+// in (n 16-bit elements, n % 8 == 0, flat index = element index of the site) -> out, masked by dropout site `site`
+int dropout16(xb_handle *h, const void *in, void *out, size_t n, bool bf16, const xb_dropout &drop, int site, cudaStream_t s) {
+    const size_t n8 = n / 8;
+    const unsigned blocks = (unsigned)std::min<size_t>((n8 + 255) / 256, (size_t)h->num_sms * 16);
+    const uint4 *src = reinterpret_cast<const uint4 *>(in);
+    uint4 *dst = reinterpret_cast<uint4 *>(out);
+    if (bf16) dropout16_kernel<true><<<blocks, 256, 0, s>>>(src, dst, n8, drop, site);
+    else dropout16_kernel<false><<<blocks, 256, 0, s>>>(src, dst, n8, drop, site);
+    XB_LAUNCH_CHECK(h);
     return XB_OK;
 }
 
@@ -390,7 +451,7 @@ void xb_train_free(xb_handle *h) {
     if (!w) return;
     for (void *p : {w->x[0], w->x[1], w->x[2], w->x[3], w->x[4], w->x[5], w->saved[0], w->saved[1], w->saved[2], w->saved[3],
                     w->saved[4], w->DZ, w->DZT, w->XT[0], w->XT[1], w->dy[0], w->dy[1], w->dzh, w->dzhT, w->colT, w->dcol,
-                    (void *)w->dcstate, (void *)w->dc2, (void *)w->dc1})
+                    (void *)w->dcstate, (void *)w->dc2, (void *)w->dc1, w->xd})
         if (p) cudaFree(p);
     delete w;
     h->train = nullptr;
@@ -420,12 +481,14 @@ static int train_ws(xb_handle *h, int N, int T) {
     return XB_OK;
 }
 
-extern "C" {
-
-// Model.forward in training (training.py:100): scores (T, N, C*NZ) fp32, activations and LSTM step state kept in the handle
-int xb_encoder_fwd_train(xb_handle *h, const void *signal, int sig_dtype, int N, int L, float *scores, void *stream) {
+// Model.forward in training (training.py:100): scores (T, N, C*NZ) fp32, activations and LSTM step state kept in the handle;
+// p (host, XB_DROPOUT_SITES; NULL = none) and seed: the dropout of rnn_encoder(drop_rate_bottom=...)
+static int encoder_fwd_train(xb_handle *h, const void *signal, int sig_dtype, int N, int L, const float *p, uint64_t seed,
+                             float *scores, void *stream) {
     if (!h) return xb_fail(nullptr, XB_ERR_ARG, "NULL handle");
     XB_REQUIRE(h, signal && scores, "NULL buffer");
+    xb_dropout drop;
+    if (int rc = xb_dropout_init(h, &drop, p, seed)) return rc;
     XB_REQUIRE(h, L > 0 && L % XB_STRIDE == 0, "chunk length %d must be a positive multiple of the stride %d", L, XB_STRIDE);
     XB_REQUIRE(h, (h->loaded & 127) == 127, "weights have not been loaded (xb_load_weights)");
     const int T = L / XB_STRIDE;
@@ -438,15 +501,52 @@ int xb_encoder_fwd_train(xb_handle *h, const void *signal, int sig_dtype, int N,
     XB_CUDA(h, cudaSetDevice(h->device));
     if (int rc = train_ws(h, N, T)) return rc;
     xb_train_ws *w = h->train;
+    const size_t TNF = (size_t)T * N * XB_FEATURES;
+    if (drop.active >> 3) {         // a dropped LSTM output: the scratch copy (allocated once, kept with the workspace)
+        const size_t cap = (size_t)w->cap_T * w->cap_N * XB_FEATURES * 2;
+        if (int rc = alloc(h, &w->xd, cap)) return rc;
+    }
     w->N = N; w->T = T;
+    w->drop = drop;
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    if (int rc = xb_conv_stem_fwd(h, signal, sig_dtype, N, L, w->x[0], stream)) return rc;
+    if (int rc = xb_conv_stem_fwd_dropout(h, signal, sig_dtype, N, L, w->x[0], &drop, stream)) return rc;
+    if (drop.on(2)) { if (int rc = dropout16(h, w->x[0], w->x[0], TNF, false, drop, 2, s)) return rc; }
     for (int l = 0; l < 5; l++) {
         const xb_lstm_weights &lw = h->lstm[l];
-        if (int rc = xb_inproj_launch(h, w->x[l], lw.w_ih, lw.bias, h->gates, T * N, s)) return rc;
+        const void *in = (l > 0 && drop.on(l + 2)) ? w->xd : w->x[l];
+        if (int rc = xb_inproj_launch(h, in, lw.w_ih, lw.bias, h->gates, T * N, s)) return rc;
         if (int rc = xb_lstm_recurrence_persistent(h, l, w->x[l + 1], T, N, (l % 2) == 0, s, w->saved[l])) return rc;
+        if (l < 4 && drop.on(l + 3)) { if (int rc = dropout16(h, w->x[l + 1], w->xd, TNF, false, drop, l + 3, s)) return rc; }
     }
     return xb_crf_head_fwd(h, w->x[5], scores, T, N, stream);
+}
+
+extern "C" {
+
+int xb_encoder_fwd_train(xb_handle *h, const void *signal, int sig_dtype, int N, int L, float *scores, void *stream) {
+    return encoder_fwd_train(h, signal, sig_dtype, N, L, nullptr, 0, scores, stream);
+}
+
+int xb_encoder_fwd_train_dropout(xb_handle *h, const void *signal, int sig_dtype, int N, int L, const float *p, uint64_t seed,
+                                 float *scores, void *stream) {
+    return encoder_fwd_train(h, signal, sig_dtype, N, L, p, seed, scores, stream);
+}
+
+int xb_dropout_keep(uint64_t seed, int site, float p, int64_t n, uint8_t *keep, void *stream) {
+    if (site < 0 || site >= XB_DROPOUT_SITES) return xb_fail(nullptr, XB_ERR_ARG, "dropout site %d out of range", site);
+    if (n < 0 || (n > 0 && !keep)) return xb_fail(nullptr, XB_ERR_ARG, "bad keep buffer");
+    float ps[XB_DROPOUT_SITES] = {};
+    ps[site] = p;
+    xb_dropout drop;
+    if (int rc = xb_dropout_init(nullptr, &drop, ps, seed)) return rc;
+    if (n == 0) return XB_OK;
+    int dev = 0, sms = 0;
+    XB_CUDA(nullptr, cudaGetDevice(&dev));
+    XB_CUDA(nullptr, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    const unsigned blocks = (unsigned)std::min<int64_t>((n + 255) / 256, (int64_t)sms * 16);
+    dropout_keep_kernel<<<blocks, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(drop, site, n, keep);
+    XB_CUDA(nullptr, cudaGetLastError());
+    return XB_OK;
 }
 
 // Backward of the last xb_encoder_fwd_train.  signal / scores: the buffers of that forward; dscores (T,N,C*NZ) fp32.
@@ -464,6 +564,8 @@ int xb_encoder_bwd(xb_handle *h, const void *signal, int sig_dtype, const float 
     xb_train_ws *w = h->train;
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     const int N = w->N, T = w->T, TN = T * N, F = XB_FEATURES, HP = h->head_rows_padded, S = h->C * h->NZ, L = T * XB_STRIDE;
+    const xb_dropout &drop = w->drop;
+    const bool drop_stem = drop.on(0) || drop.on(1);
 
     // ---- head
     {
@@ -503,17 +605,23 @@ int xb_encoder_bwd(xb_handle *h, const void *signal, int sig_dtype, const float 
         if (int rc = transpose_to_bf16(h, w->DZ, TN, XB_GATES, XB_GATES, true, w->DZT, s, g_bih)) return rc;   // + db = colsum DZ
         XB_CUDA(h, cudaMemcpyAsync(g_bhh, g_bih, XB_GATES * sizeof(float), cudaMemcpyDeviceToDevice, s));
         if (int rc = transpose_to_bf16(h, w->x[l], TN, F, F, false, w->XT[l & 1], s)) return rc;
+        // layer l > 0 read the dropped copy of x[l] (site l + 2): dW_ih takes that, transposed through the mask into xd
+        const bool drop_in = l > 0 && drop.on(l + 2);
+        if (drop_in) { if (int rc = transpose_to_bf16(h, w->x[l], TN, F, F, false, w->xd, s, nullptr, &drop, l + 2)) return rc; }
         // dW_ih = DZ^T x_l and dW_hh = sum over the steps that had a predecessor of dz_t (x) h_prev (a time shift of N columns
         // between DZ^T and Y^T), one launch over 128 x 256 tiles (wgrad_gemm.cu)
         {
             xb_stage_timer tm(h, XB_ST_TRAIN_WGRAD, s);
-            if (int rc = xb_lstm_wgrad_launch(h, w->DZT, w->XT[l & 1], w->XT[(l + 1) & 1], T, N, reverse, g_wih, g_whh, s)) return rc;
+            if (int rc = xb_lstm_wgrad_launch(h, w->DZT, drop_in ? w->xd : w->XT[l & 1], w->XT[(l + 1) & 1], T, N, reverse, g_wih,
+                                              g_whh, s)) return rc;
         }
         if (int rc = gemm_bf16(h, EPI_BF16OUT, w->DZ, TN, XB_GATES, lw.w_ihT, F, XB_GATES, XB_GATES, w->dy[l & 1], F, s)) return rc;
+        // gradient w.r.t. the dropped input -> w.r.t. the output of the layer below (l == 0: the conv3 output, site 2)
+        if (drop.on(l + 2)) { if (int rc = dropout16(h, w->dy[l & 1], w->dy[l & 1], (size_t)TN * F, true, drop, l + 2, s)) return rc; }
     }
     // ---- convolution stem: dy[0] is the gradient w.r.t. x[0] (T, N, 768)
     {
-        if (int rc = xb_conv12_im2col(h, signal, sig_dtype, N, L, s)) return rc;          // im2col rows of this batch into h->c2
+        if (int rc = xb_conv12_im2col(h, signal, sig_dtype, N, L, s, &drop)) return rc;   // im2col rows of this batch into h->c2
         CUtensorMap tmA, tmB;
         if (int rc = xb_make_tmap_2d(h, &tmA, h->c2, (uint64_t)TN, XB_CONV3_K, XB_CONV3_K)) return rc;
         if (int rc = xb_make_tmap_2d(h, &tmB, h->conv3_w, F, XB_CONV3_K, XB_CONV3_K)) return rc;
@@ -535,14 +643,22 @@ int xb_encoder_bwd(xb_handle *h, const void *signal, int sig_dtype, const float 
         XB_CUDA(h, cudaMemsetAsync(grads[1], 0, 4 * sizeof(float), s));
         dim3 g2((L + 255) / 256, N);
         if (sig_dtype == XB_SIG_F32) {
-            conv2_bwd_kernel<float><<<g2, 256, 0, s>>>(reinterpret_cast<const float *>(signal), L, h->conv1_w, h->conv1_b, h->conv2_w,
-                                                       h->conv2_b, w->dc2, w->dc1, grads[2], grads[3]);
+            if (drop_stem)
+                conv2_bwd_kernel<true, float><<<g2, 256, 0, s>>>(reinterpret_cast<const float *>(signal), L, h->conv1_w, h->conv1_b,
+                                                                 h->conv2_w, h->conv2_b, w->dc2, w->dc1, grads[2], grads[3], drop);
+            else
+                conv2_bwd_kernel<false, float><<<g2, 256, 0, s>>>(reinterpret_cast<const float *>(signal), L, h->conv1_w, h->conv1_b,
+                                                                  h->conv2_w, h->conv2_b, w->dc2, w->dc1, grads[2], grads[3], drop);
             XB_LAUNCH_CHECK(h);
             conv1_bwd_kernel<float><<<dim3(4, N), 256, 0, s>>>(reinterpret_cast<const float *>(signal), L, h->conv1_w, h->conv1_b, w->dc1,
                                                               grads[0], grads[1]);
         } else {
-            conv2_bwd_kernel<int16_t><<<g2, 256, 0, s>>>(reinterpret_cast<const int16_t *>(signal), L, h->conv1_w, h->conv1_b, h->conv2_w,
-                                                         h->conv2_b, w->dc2, w->dc1, grads[2], grads[3]);
+            if (drop_stem)
+                conv2_bwd_kernel<true, int16_t><<<g2, 256, 0, s>>>(reinterpret_cast<const int16_t *>(signal), L, h->conv1_w, h->conv1_b,
+                                                                   h->conv2_w, h->conv2_b, w->dc2, w->dc1, grads[2], grads[3], drop);
+            else
+                conv2_bwd_kernel<false, int16_t><<<g2, 256, 0, s>>>(reinterpret_cast<const int16_t *>(signal), L, h->conv1_w, h->conv1_b,
+                                                                    h->conv2_w, h->conv2_b, w->dc2, w->dc1, grads[2], grads[3], drop);
             XB_LAUNCH_CHECK(h);
             conv1_bwd_kernel<int16_t><<<dim3(4, N), 256, 0, s>>>(reinterpret_cast<const int16_t *>(signal), L, h->conv1_w, h->conv1_b,
                                                                 w->dc1, grads[0], grads[1]);

@@ -20,7 +20,9 @@ int xb_fail(xb_handle *h, int code, const char *fmt, ...) {
     return code;
 }
 
-int xb_conv12_im2col(xb_handle *h, const void *signal, int sig_dtype, int N, int L, cudaStream_t s);
+struct xb_dropout;
+int xb_conv12_im2col(xb_handle *h, const void *signal, int sig_dtype, int N, int L, cudaStream_t s,
+                     const xb_dropout *drop = nullptr);
 int xb_lstm_recurrence_persistent(xb_handle *h, int layer, void *y_tnc, int T, int N, int reverse, cudaStream_t s, void *save = nullptr);
 int xb_inproj_launch(xb_handle *h, const void *x, const void *w_ih, const float *bias, void *gates, int M, cudaStream_t s);
 int xb_head_astationary_launch(xb_handle *h, const void *x, const void *w, int w_rows, const float *bias, int head_rows,
@@ -370,7 +372,11 @@ int xb_load_weights(xb_handle *h, const float *const *w, int n_tensors, float sc
 }
 
 // ------------------------------------------------------------------------------------------ encoder
-int xb_conv_stem_fwd(xb_handle *h, const void *signal, int sig_dtype, int N, int L, void *out_tnc, void *stream) {
+}  // extern "C"
+
+// the stem with the masks of dropout sites 0 and 1 (drop may be NULL); the training forward (train_bwd.cu) calls it
+int xb_conv_stem_fwd_dropout(xb_handle *h, const void *signal, int sig_dtype, int N, int L, void *out_tnc,
+                             const xb_dropout *drop, void *stream) {
     if (!h) return xb_fail(nullptr, XB_ERR_ARG, "NULL handle");
     if (!(h->loaded & 1)) return xb_fail(h, XB_ERR_STATE, "convolution weights have not been loaded (xb_load_weights)");
     XB_REQUIRE(h, signal && out_tnc, "NULL buffer");
@@ -380,10 +386,16 @@ int xb_conv_stem_fwd(xb_handle *h, const void *signal, int sig_dtype, int N, int
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     {
         xb_stage_timer tm(h, XB_ST_CONV12, s);
-        if (int rc = xb_conv12_im2col(h, signal, sig_dtype, N, L, s)) return rc;
+        if (int rc = xb_conv12_im2col(h, signal, sig_dtype, N, L, s, drop)) return rc;
     }
     xb_stage_timer tm(h, XB_ST_CONV3, s);
     return xb_conv3_launch(h, h->c2, h->conv3_w, h->conv3_b, out_tnc, T, N, s);
+}
+
+extern "C" {
+
+int xb_conv_stem_fwd(xb_handle *h, const void *signal, int sig_dtype, int N, int L, void *out_tnc, void *stream) {
+    return xb_conv_stem_fwd_dropout(h, signal, sig_dtype, N, L, out_tnc, nullptr, stream);
 }
 
 int xb_lstm_fwd(xb_handle *h, int layer, const void *x_tnc, void *y_tnc, int T, int N, int reverse, void *stream) {

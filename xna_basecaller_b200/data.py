@@ -16,7 +16,8 @@ lengths) batches Trainer.train_one_step consumes and has the `len()` / `.sampler
 
 Not built: the on-the-fly spliced / spiked unnatural-base augmentation (stitch_chunks.py:323-454, spike_chunks.py:247-297:
 numpy procedures over pandas k-mer tables, driven by one numpy Generator stream per data set item; DESIGN.md section 7).
-Passing spike_kwargs / stitch_kwargs raises NotImplementedError instead of silently training on un-augmented data.
+Passing spike_kwargs / stitch_kwargs raises NotImplementedError instead of silently training on un-augmented data.  (The
+model-side regulariser of the same training setup, rnn_encoder's drop_rate_bottom dropout, is built: training.py.)
 """
 import os
 

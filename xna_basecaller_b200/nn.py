@@ -7,8 +7,10 @@ Parameters are ordinary torch Parameters with the reference's names (conv.weight
 linear.weight ...), so reference checkpoints load unchanged; the arithmetic runs in libxna_b200.so:
 
   Serial.forward   recognises [Convolution(1,4,5) Convolution(4,16,5) Convolution(16,768,19,s5) Permute(2,0,1)]
-                   and runs it as the fused stem (xb_conv_stem_fwd), then LSTM layers (xb_lstm_fwd) and the
-                   CRF head (xb_crf_head_fwd); activations stay 16-bit (T, N, 768) on the device in between.
+                   (with or without rnn_encoder's drop_rate_bottom Dropouts between them) and runs it as the fused
+                   stem (xb_conv_stem_fwd), then LSTM layers (xb_lstm_fwd) and the CRF head (xb_crf_head_fwd);
+                   activations stay 16-bit (T, N, 768) on the device in between.  In training the whole encoder is
+                   one fused step (xb_encoder_fwd_train[_dropout] / xb_encoder_bwd), dropout included.
   LSTM.forward     one layer on a (T, N, 768) CUDA tensor; `reverse` walks time backwards by indexing.
   LinearCRFEncoder.forward   scale * tanh(x W^T + b) with the blank score expanded in the epilogue -> fp32.
 
@@ -99,12 +101,13 @@ class Serial(torch.nn.Sequential):
     def set_engine(self, engine):
         _adopt(self, engine, [0])
 
-    def _stem(self):
-        """The four leading modules when they are the sup@v3.3 convolution stem, else None."""
+    def _stem_end(self):
+        """Index past the Permute when the leading modules, Dropouts skipped, are the sup@v3.3 convolution stem, else None."""
         mods = list(self)
-        if len(mods) < 4:
+        core = [i for i, m in enumerate(mods) if not isinstance(m, torch.nn.Dropout)][:4]
+        if len(core) < 4:
             return None
-        c1, c2, c3, pm = mods[:4]
+        c1, c2, c3, pm = (mods[i] for i in core)
         if not (isinstance(c1, Convolution) and isinstance(c2, Convolution) and isinstance(c3, Convolution)
                 and isinstance(pm, Permute)):
             return None
@@ -115,21 +118,49 @@ class Serial(torch.nn.Sequential):
                 return None
         if list(pm.dims) != [2, 0, 1]:
             return None
+        return core[3] + 1
+
+    def _stem(self):
+        """The three convolutions when the leading modules, Dropouts skipped, are the sup@v3.3 convolution stem, else None.
+        Dropout is the identity outside training, so every inference route runs such a model unchanged."""
+        end = self._stem_end()
+        if end is None:
+            return None
+        c1, c2, c3 = [m for m in list(self)[:end] if isinstance(m, Convolution)]
         return c1, c2, c3
 
     def _training_layout(self):
-        """(stem, five LSTMs, head) when this is the whole sup@v3.3 encoder -- the layout the fused training step
-        (xb_encoder_fwd_train / xb_encoder_bwd) is built for -- else None."""
-        stem = self._stem()
-        mods = [m for m in list(self)[4:] if not isinstance(m, torch.nn.Dropout)] if stem is not None else []
-        if len(mods) != 6 or not all(isinstance(m, LSTM) for m in mods[:5]) or not isinstance(mods[5], LinearCRFEncoder):
+        """(stem, five LSTMs, head, p) when this is the whole sup@v3.3 encoder -- the layout the fused training step
+        (xb_encoder_fwd_train_dropout / xb_encoder_bwd) is built for -- else None.  p lists the dropout probabilities of the
+        seven places rnn_encoder(drop_rate_bottom=...) puts a torch.nn.Dropout: after each convolution and after LSTM
+        layers 0-3 (0.0 where there is none, or where the module is in eval mode).  A Dropout with p > 0 anywhere else
+        makes the layout unknown; one with p == 0 is the identity and may stand anywhere."""
+        core, drops = [], []                 # modules other than Dropout; the active Dropout after each of them
+        for m in self:
+            if isinstance(m, torch.nn.Dropout):
+                p = float(m.p) if m.training else 0.0
+                if p == 0.0:
+                    continue
+                if not core or drops[-1] is not None:
+                    return None
+                drops[-1] = p
+            else:
+                core.append(m)
+                drops.append(None)
+        if self._stem() is None or len(core) != 10:
+            return None
+        stem, mods = self._stem(), core[4:]
+        if not all(isinstance(m, LSTM) for m in mods[:5]) or not isinstance(mods[5], LinearCRFEncoder):
             return None
         if [m.reverse for m in mods[:5]] != [True, False, True, False, True]:
             return None
         head = mods[5]
         if head.extra_linear or not head.expand_blanks or head.blank_score is None or head.linear.bias is None:
             return None
-        return stem, mods[:5], head
+        if any(drops[i] is not None for i in (3, 8, 9)):     # after the Permute, after LSTM layer 4, after the head
+            return None
+        p = [drops[i] or 0.0 for i in (0, 1, 2, 4, 5, 6, 7)]
+        return stem, mods[:5], head, p
 
     def forward(self, x):
         mods = list(self)
@@ -142,15 +173,19 @@ class Serial(torch.nn.Sequential):
             layout = self._training_layout()
             if layout is None or x.dim() != 3 or x.shape[1] != 1:
                 raise RuntimeError('gradients are implemented for the whole sup@v3.3 encoder (conv stem, five LSTMs in the '
-                                   'reference directions, LinearCRFEncoder with expand_blanks); run other layouts under '
-                                   'torch.no_grad()')
-            for m in mods:
-                if isinstance(m, torch.nn.Dropout) and m.training and m.p > 0:
-                    raise RuntimeError('dropout is not part of the B200 path')
+                                   'reference directions, LinearCRFEncoder with expand_blanks, dropout only where '
+                                   'rnn_encoder(drop_rate_bottom=...) puts it); run other layouts under torch.no_grad()')
+            head = layout[2]
+            if head.dropout.training and head.dropout.p > 0:
+                # where the head applies its dropout in the forward is not recorded in this repository: refuse, do not guess
+                raise RuntimeError('LinearCRFEncoder(drop_rate > 0) has no B200 training path; train with drop_rate = 0')
             return _encoder_train_forward(self, layout, x)
         if stem is not None and x.dim() == 3 and x.shape[1] == 1:
+            start = self._stem_end()
+            for m in mods[:start]:
+                if isinstance(m, torch.nn.Dropout) and m.training and m.p > 0:
+                    raise RuntimeError('dropout is not part of the B200 forward path; call model.eval()')
             x = _conv_stem_forward(self, stem, x)
-            start = 4
         for m in mods[start:]:
             if isinstance(m, torch.nn.Dropout):
                 if m.training and m.p > 0:
@@ -177,18 +212,18 @@ class _EncoderTrain(torch.autograd.Function):
     """scores = encoder(x) with a backward that fills the gradients of the 28 parameter tensors (xb_encoder_bwd)."""
 
     @staticmethod
-    def forward(ctx, x, handle, *params):
+    def forward(ctx, x, handle, dropout_p, seed, *params):
         ctx.handle, ctx.dtypes = handle, [p.dtype for p in params]
-        return handle.encoder_train(x)
+        return handle.encoder_train(x, dropout_p=dropout_p, seed=seed)
 
     @staticmethod
     def backward(ctx, dscores):
-        grads = ctx.handle.encoder_backward(dscores)
-        return (None, None) + tuple(grads[k].to(dt) for k, dt in zip(ctx.handle.WEIGHT_KEYS, ctx.dtypes))
+        grads = ctx.handle.encoder_backward(dscores)      # the handle replays the masks of its last forward
+        return (None, None, None, None) + tuple(grads[k].to(dt) for k, dt in zip(ctx.handle.WEIGHT_KEYS, ctx.dtypes))
 
 
 def _encoder_train_forward(owner, layout, x):
-    stem, lstms, head = layout
+    stem, lstms, head, dropout_p = layout
     eng = _engine_of(owner)
     N, _, L = x.shape
     if L % 5:
@@ -199,7 +234,14 @@ def _encoder_train_forward(owner, layout, x):
     for m in lstms:
         params += [m.rnn.weight_ih_l0, m.rnn.weight_hh_l0, m.rnn.bias_ih_l0, m.rnn.bias_hh_l0]
     params += [head.linear.weight, head.linear.bias]
-    return _EncoderTrain.apply(x, h, *params)
+    seed = None
+    if any(dropout_p):
+        # one 63-bit seed per forward from torch's default CPU generator: torch.manual_seed makes the masks repeatable.
+        # Without dropout nothing is drawn, so torch's random stream is the same as without this feature.
+        seed = int(torch.empty((), dtype=torch.int64).random_().item())
+    else:
+        dropout_p = None
+    return _EncoderTrain.apply(x, h, dropout_p, seed, *params)
 
 
 def _sync_stem(eng, stem):

@@ -6,6 +6,12 @@ xb_ctc_crf_loss_fwd / _bwd, xb_encoder_bwd behind torch.autograd.Function nodes)
 multi-tensor call (xb_adamw_step).  Gradients are transported as bf16 with fp32 accumulation, so there is no GradScaler
 (`use_amp` is accepted for signature compatibility and ignored).  Data loading / augmentation stay with the caller.
 
+Models built with rnn_encoder(drop_rate_bottom=p) train with their dropout: the fused step applies it on the GPU
+(xb_encoder_fwd_train_dropout) with masks drawn from one seed per forward that Serial.forward takes from torch's default
+CPU generator, so torch.manual_seed makes a run repeatable.  Not built: the head's dropout (LinearCRFEncoder(drop_rate > 0)
+raises in training: where the reference applies it in the head's forward is not recorded here) and the spliced / spiked
+augmentation (see data.py).
+
 validate_one_step / validate_one_epoch (training.py:159-181) score the validation chunks on the device: forward, loss,
 one CRF decode, and the local alignment of every decode against its reference (xb_align_counts) -- only the strings,
 the loss and 20 bytes of alignment counts per chunk come back to the host.
