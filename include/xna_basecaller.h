@@ -52,7 +52,7 @@ enum xb_flags {
     XB_FLAG_BF16 = 1,            /* weights rounded to bfloat16 (activations stay float16)     */
     XB_FLAG_NO_ENCODER = 2,      /* decode-only handle: no encoder workspace is allocated      */
     XB_FLAG_TRAIN = 8            /* keep transposed bf16 weight copies for xb_encoder_bwd      */
-    /* (4 was the one-launch-per-step LSTM of round 1; it exists only in -DXB_EXPERIMENTS builds) */
+    /* (4 is unused) */
 };
 
 enum xb_signal_dtype { XB_SIG_F32 = 0, XB_SIG_F16 = 1, XB_SIG_I16 = 2 };

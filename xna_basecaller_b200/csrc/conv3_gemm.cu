@@ -3,9 +3,9 @@
 //
 //   out[t, b, :] = swish( col[(b, t), 0:320] . W3^T + b3 )          M = N*T rows, K = 320 (16 channels x 19 taps + pad), 768 columns
 //
-// Why not the generic tile kernel (gemm_tc.cu, EPI_CONV3: 0.48 ms per 512-chunk batch).  With K = 320 a 128 x 128 output
-// tile moves 80 KB of im2col rows and 80 KB of weights for 1280 MMA cycles: 2600 cycles of L2 ingest at ~62 B/clk per SM,
-// and the im2col matrix is read six times (once per column tile).  Here each CTA keeps a 192-column slice of W3 (120 KB)
+// Why not the generic tile kernel (a conv3 epilogue of gemm_tc.cu was measured at 0.48 ms per 512-chunk batch and removed).
+// With K = 320 a 128 x 128 output tile moves 80 KB of im2col rows and 80 KB of weights for 1280 MMA cycles: 2600 cycles of
+// L2 ingest at ~62 B/clk per SM, and the im2col matrix is read six times (once per column tile).  Here each CTA keeps a 192-column slice of W3 (120 KB)
 // in shared memory for its whole life and streams only im2col row tiles (80 KB per 128 x 192 outputs = 1920 MMA cycles):
 // the kernel is bound by the tensor pipe and its epilogue instead of by ingest.
 //

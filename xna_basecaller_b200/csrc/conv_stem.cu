@@ -1,7 +1,7 @@
 // Front of the convolution stem: Convolution(1->4,k5,p2)+swish, Convolution(4->16,k5,p2)+swish fused in one
 // kernel (bonito/nn.py:57-68; built at bonito/crf/model.py:138-139,148-149), with the result emitted directly as
 // the im2col rows of the third convolution (16->768, k19, stride 5, pad 9), so that conv3 runs as a tcgen05
-// GEMM (gemm_tc.cu, EPI_CONV3).  The (N,4,L) and (N,16,L) intermediates of the reference never touch HBM.
+// GEMM (conv3_gemm.cu).  The (N,4,L) and (N,16,L) intermediates of the reference never touch HBM.
 //
 // Row (chunk b, step t) of the im2col matrix holds c2[b, 5t-9+tap, ch] at column tap*16+ch for tap < 19, zero
 // padded to 320 columns.  Padding semantics follow torch Conv1d: each layer sees zeros outside [0, L).

@@ -6,19 +6,14 @@
 // warp 2 = TMEM allocator, warps 4..7 = epilogue (warp q reads TMEM lanes 32q..32q+31 = tile rows).
 //
 // Epilogues
-//   EPI_F32    plain fp32 store (self test)
-//   EPI_CONV3  third Convolution of the stem as an implicit GEMM over im2col rows: + bias, swish, 16-bit store
-//              in (T, N, 768) order, which absorbs nn.Permute([2,0,1])       (bonito/nn.py:57-68,156-167); the product
-//              runs conv3_gemm.cu instead, this form remains in -DXB_EXPERIMENTS builds
-//   EPI_INPROJ LSTM input projection x_t W_ih^T + (b_ih + b_hh) for all t at once, 16-bit store (nn.py:189-193)
-//   EPI_HEAD   LinearCRFEncoder: scale * tanh(x W^T + b), blank score inserted in front of every group of
-//              n_base columns -> fp32 (T, N, C*NZ)                            (bonito/nn.py:112-133)
-//   EPI_LSTM   one LSTM time step: gates = acc (h_{t-1} W_hh^T) + G[t]; c, h update in fp32; h stored 16-bit.
-//              Columns of a tile are [i | f | g | o] x 32 hidden units (weights are row-permuted at load time).
+//   EPI_F32       plain fp32 store, or fp32 atomic adds of split-K slices (weight gradients)
+//   EPI_BF16OUT   plain bf16 store (gradients flowing to the layer below)
+//   EPI_CONV3_BWD recomputed conv3 pre-activation -> dy * swish'(pre), bf16 in im2col row order
+// The forward forms of conv3, the LSTM input projection, the CRF head and a one-launch-per-step LSTM were measured
+// against the dedicated kernels and removed (DESIGN §4.3).
 #include "xb_common.cuh"
 #include "xb_ptx.cuh"
 #include "xb_gemm.cuh"
-#include "xb_head_epilogue.cuh"
 
 using namespace xbptx;
 
@@ -27,26 +22,13 @@ namespace {
 constexpr int BM = 128, BN = 128, BK = 64;
 constexpr int TILE_A_BYTES = BM * BK * 2, TILE_B_BYTES = BN * BK * 2;
 constexpr int STAGE_BYTES = TILE_A_BYTES + TILE_B_BYTES;
-// Pipeline depth.  Three stages (96 KB) leave room for two CTAs per SM, whose epilogues and main loops overlap.  The
-// one-launch-per-step recurrence GEMM of the cross-check builds (a 24-tile grid: one CTA per SM, latency-bound on the TMA
-// round trip) runs six stages instead: 192 KB in flight per SM.
-template <int EPI> struct Pipe {
-    static constexpr int STAGES = (EPI == EPI_LSTM) ? 6 : 3;
-    static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /*align slack*/ + 256 /*barriers*/;
-};
-
-__device__ __forceinline__ float fast_sigmoid(float x) { return __fdividef(1.0f, 1.0f + __expf(-x)); }
-__device__ __forceinline__ float fast_tanh(float x) { return 1.0f - __fdividef(2.0f, __expf(2.0f * x) + 1.0f); }
-__device__ __forceinline__ float tanh_approx(float x) {
-    float y;
-    asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
-    return y;
-}
+// Pipeline depth.  Three stages (96 KB) leave room for two CTAs per SM, whose epilogues and main loops overlap.
+constexpr int STAGES = 3;
+constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /*align slack*/ + 256 /*barriers*/;
 
 template <bool BF16, int EPI>
-__global__ void __launch_bounds__(256, (EPI == EPI_LSTM) ? 1 : 2)
+__global__ void __launch_bounds__(256, 2)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const GemmParams p) {
-    constexpr int STAGES = Pipe<EPI>::STAGES;
     extern __shared__ uint8_t smem_raw[];
     uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     uint64_t *full = reinterpret_cast<uint64_t *>(smem + STAGES * STAGE_BYTES);
@@ -62,7 +44,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const int kb_all = (p.K + BK - 1) / BK;
     const int kb_per = (kb_all + gridDim.z - 1) / gridDim.z;
     const int kb0 = blockIdx.z * kb_per;
-    const int kblocks = (EPI == EPI_LSTM && p.first) ? 0 : max(0, min(kb_all, kb0 + kb_per) - kb0);
+    const int kblocks = max(0, min(kb_all, kb0 + kb_per) - kb0);
 
     if (warp == 0 && lane == 0) {
         prefetch_tmap(&tmA);
@@ -93,7 +75,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                 mbar_wait(&empty[s], ph ^ 1);
                 mbar_expect_tx(&full[s], STAGE_BYTES);
                 uint8_t *sa = smem + s * STAGE_BYTES;
-                tma_load_2d(sa, &tmA, &full[s], (kb0 + kb) * BK, m0 + p.a_row_offset);
+                tma_load_2d(sa, &tmA, &full[s], (kb0 + kb) * BK, m0);
                 tma_load_2d(sa + TILE_A_BYTES, &tmB, &full[s], (kb0 + kb) * BK, n0);
             }
         }
@@ -118,11 +100,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             __syncwarp();
         }
     }
-    // Epilogue: warp w reads TMEM lanes 32*(w%4)..+31 (= tile rows).  The fused LSTM step keeps its four dedicated
-    // warps; every other epilogue runs on all eight warps (the producer / MMA warps are idle once the main loop has
-    // been issued): warps 0-3 take tile columns 0..63, warps 4-7 columns 64..127.  (EPI_F32, the self test, also keeps four.)
+    // Epilogue: warps 4..7; warp w reads TMEM lanes 32*(w%4)..+31 (= tile rows).
     __syncwarp();
-    if ((EPI == EPI_LSTM || EPI == EPI_F32 || EPI == EPI_BF16OUT || EPI == EPI_CONV3_BWD) ? warp >= 4 : true) {
+    if (warp >= 4) {
         const int q = warp & 3;
         const int r = q * 32 + lane;             // tile row == TMEM lane
         const int m = m0 + r;
@@ -132,67 +112,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             mbar_wait(tmem_full, 0);
             tc_fence_after();
         }
-        using X = xb16<BF16>;
-        if constexpr (EPI == EPI_LSTM) {
-            // row = batch element; columns [g*32 + u], g in (i,f,g,o), u = unit within the 32-unit slice
-            const int unit0 = blockIdx.x * 32;
-            const size_t grow = ((size_t)p.t_cur * p.NB + m) * XB_GATES + n0;
-            const uint16_t *G = reinterpret_cast<const uint16_t *>(p.gates) + grow;
-            float *cst = p.cstate + (size_t)m * XB_FEATURES + unit0;
-            uint16_t *hout = reinterpret_cast<uint16_t *>(p.out) + ((size_t)p.t_cur * p.NB + m) * XB_FEATURES + unit0;
-#pragma unroll 1
-            for (int ub = 0; ub < 32; ub += 8) {
-                uint32_t acc[4][8];
-                if (kblocks > 0) {
-#pragma unroll
-                    for (int g = 0; g < 4; g++) tmem_ld_32x32b_x8(taddr + g * 32 + ub, acc[g]);
-                    tmem_ld_wait();
-                } else {
-#pragma unroll
-                    for (int g = 0; g < 4; g++)
-#pragma unroll
-                        for (int j = 0; j < 8; j++) acc[g][j] = 0u;
-                }
-                if (row_ok) {
-                    float gv[4][8];
-#pragma unroll
-                    for (int g = 0; g < 4; g++) {
-                        uint4 raw = *reinterpret_cast<const uint4 *>(G + g * 32 + ub);
-                        const uint32_t rw[4] = {raw.x, raw.y, raw.z, raw.w};
-#pragma unroll
-                        for (int j = 0; j < 4; j++) {
-                            float2 f = X::unpack(rw[j]);
-                            gv[g][2 * j] = __uint_as_float(acc[g][2 * j]) + f.x;
-                            gv[g][2 * j + 1] = __uint_as_float(acc[g][2 * j + 1]) + f.y;
-                        }
-                    }
-                    float cprev[8];
-                    if (p.first) {
-#pragma unroll
-                        for (int j = 0; j < 8; j++) cprev[j] = 0.0f;
-                    } else {
-                        float4 c0 = *reinterpret_cast<const float4 *>(cst + ub);
-                        float4 c1 = *reinterpret_cast<const float4 *>(cst + ub + 4);
-                        cprev[0] = c0.x; cprev[1] = c0.y; cprev[2] = c0.z; cprev[3] = c0.w;
-                        cprev[4] = c1.x; cprev[5] = c1.y; cprev[6] = c1.z; cprev[7] = c1.w;
-                    }
-                    float cn[8], hn[8];
-#pragma unroll
-                    for (int j = 0; j < 8; j++) {
-                        float ig = fast_sigmoid(gv[0][j]), fg = fast_sigmoid(gv[1][j]);
-                        float gg = fast_tanh(gv[2][j]), og = fast_sigmoid(gv[3][j]);
-                        cn[j] = fg * cprev[j] + ig * gg;
-                        hn[j] = og * fast_tanh(cn[j]);
-                    }
-                    *reinterpret_cast<float4 *>(cst + ub) = make_float4(cn[0], cn[1], cn[2], cn[3]);
-                    *reinterpret_cast<float4 *>(cst + ub + 4) = make_float4(cn[4], cn[5], cn[6], cn[7]);
-                    uint4 hv;
-                    hv.x = X::pack(hn[0], hn[1]); hv.y = X::pack(hn[2], hn[3]);
-                    hv.z = X::pack(hn[4], hn[5]); hv.w = X::pack(hn[6], hn[7]);
-                    *reinterpret_cast<uint4 *>(hout + ub) = hv;
-                }
-            }
-        } else if constexpr (EPI == EPI_BF16OUT) {
+        if constexpr (EPI == EPI_BF16OUT) {
             // plain bf16 store of the accumulator (gradients flowing to the layer below)
 #pragma unroll 1
             for (int cb = 0; cb < BN; cb += 32) {
@@ -258,80 +178,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                         for (int j = 0; j < 32; j++)
                             if (nb + j < p.N) o[j] = __uint_as_float(acc[j]);
                     }
-                }
-            }
-        } else {
-            // Coalesced epilogues.  The accumulator arrives one tile ROW per thread; a direct store would touch 32
-            // different output rows per instruction.  Each epilogue warp therefore stages its 32 x 128 block in
-            // the (now idle: every MMA has completed) pipeline buffers and writes whole row segments.
-            uint8_t *stg = smem + warp * (STAGES * STAGE_BYTES / 8);
-            constexpr int HN = BN / 2;                           // columns per warp
-            const int c0 = (warp >> 2) * HN;                     // first tile column of this warp
-            if constexpr (EPI == EPI_CONV3 || EPI == EPI_INPROJ) {
-                constexpr int RSB = HN * 2 + 16;                 // staged row pitch in bytes (16 B pad: conflict free)
-#pragma unroll 1
-                for (int cb = c0; cb < c0 + HN; cb += 32) {
-                    uint32_t acc[32];
-                    tmem_ld_32x32b_x32(taddr + cb, acc);
-                    tmem_ld_wait();
-                    const int nb = n0 + cb;
-                    uint32_t pk[16];
-#pragma unroll
-                    for (int j = 0; j < 16; j++) {
-                        float v0 = __uint_as_float(acc[2 * j]) + __ldg(p.bias + nb + 2 * j);
-                        float v1 = __uint_as_float(acc[2 * j + 1]) + __ldg(p.bias + nb + 2 * j + 1);
-                        if constexpr (EPI == EPI_CONV3) {      // swish with ONE MUFU per element: sigmoid(x) = 0.5 tanh(0.5 x) + 0.5
-                            v0 = v0 * fmaf(tanh_approx(0.5f * v0), 0.5f, 0.5f);      // (the exp + reciprocal form kept this epilogue,
-                            v1 = v1 * fmaf(tanh_approx(0.5f * v1), 0.5f, 0.5f);      // and with it the conv3 GEMM, MUFU-bound)
-                        }
-                        pk[j] = X::pack(v0, v1);
-                    }
-                    uint4 *d = reinterpret_cast<uint4 *>(stg + lane * RSB + (cb - c0) * 2);
-#pragma unroll
-                    for (int j = 0; j < 4; j++) d[j] = make_uint4(pk[4 * j], pk[4 * j + 1], pk[4 * j + 2], pk[4 * j + 3]);
-                }
-                __syncwarp();
-                // 8 lanes x 16 B = one 128-byte row segment; four rows per instruction
-                const int half = lane >> 3, l16 = lane & 7;
-#pragma unroll 4
-                for (int rr = 0; rr < 32; rr += 4) {
-                    const int mm = m0 + q * 32 + rr + half;
-                    if (mm < p.M) {
-                        size_t orow;
-                        if constexpr (EPI == EPI_CONV3) {
-                            const int b = mm / p.T, t = mm - b * p.T;        // im2col rows are (chunk, t)
-                            orow = (size_t)t * p.NB + b;
-                        } else {
-                            orow = (size_t)mm;
-                        }
-                        uint16_t *o = reinterpret_cast<uint16_t *>(p.out) + orow * p.ldo + n0 + c0;
-                        reinterpret_cast<uint4 *>(o)[l16] = *reinterpret_cast<const uint4 *>(stg + (rr + half) * RSB + l16 * 16);
-                    }
-                }
-            } else {   // EPI_HEAD
-                constexpr int RS = 81;                           // staged row pitch in floats (odd: conflict free)
-                float *S = reinterpret_cast<float *>(stg);
-                const int col0 = n0 + c0;                        // head columns of this warp: [col0, col_end)
-                const int col_end = min(col0 + HN, p.head_rows);
-                int seg_start, seg_len;
-                xbhead::segment(col0, col_end, p.n_base, p.expand, seg_start, seg_len);
-#pragma unroll 1
-                for (int cb = c0; cb < c0 + HN; cb += 32) {
-                    if (n0 + cb >= col_end) break;
-                    uint32_t acc[32];
-                    tmem_ld_32x32b_x32(taddr + cb, acc);
-                    tmem_ld_wait();
-                    xbhead::stage32(acc, n0 + cb, col_end, p.n_base, p.expand, p.bias, p.scale, p.blank, S + lane * RS, seg_start);
-                }
-                __syncwarp();
-                float *obase = reinterpret_cast<float *>(p.out) + seg_start;
-#pragma unroll 1
-                for (int rr = 0; rr < 32; rr++) {
-                    const int mm = m0 + q * 32 + rr;
-                    if (mm >= p.M) break;
-                    float *o = obase + (size_t)mm * p.ldo;
-                    const float *Sr = S + rr * RS;
-                    for (int idx = lane; idx < seg_len; idx += 32) o[idx] = Sr[idx];
                 }
             }
         }
@@ -422,16 +268,14 @@ int xb_make_tmap_hview(xb_handle *h, CUtensorMap *out, const void *base, uint64_
 }
 
 template <bool BF16, int EPI>
-static int launch_one(xb_handle *h, const CUtensorMap &tmA, const CUtensorMap &tmB, const GemmParams &p, int rows_a,
-                      cudaStream_t s) {
+static int launch_one(xb_handle *h, const CUtensorMap &tmA, const CUtensorMap &tmB, const GemmParams &p, cudaStream_t s) {
     auto k = gemm_tc_kernel<BF16, EPI>;
-    constexpr int SMEM_BYTES = Pipe<EPI>::SMEM_BYTES;
     static bool configured[64] = {};   // per instantiation and device (function attributes live in the context)
     if (!configured[h->device & 63]) {
         XB_CUDA(h, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
         configured[h->device & 63] = true;
     }
-    dim3 grid((p.N + BN - 1) / BN, (rows_a + BM - 1) / BM, (EPI == EPI_F32 && p.split_k > 1) ? p.split_k : 1);
+    dim3 grid((p.N + BN - 1) / BN, (p.M + BM - 1) / BM, (EPI == EPI_F32 && p.split_k > 1) ? p.split_k : 1);
     k<<<grid, 256, SMEM_BYTES, s>>>(tmA, tmB, p);
     XB_LAUNCH_CHECK(h);
     return XB_OK;
@@ -442,24 +286,14 @@ int xb_gemm_launch(xb_handle *h, int epi, const CUtensorMap &tmA, const CUtensor
     if (p.K <= 0) return xb_fail(h, XB_ERR_ARG, "GEMM K=%d", p.K);
     if (bf16_operands) {      // the training backward: gradients travel as bf16 (range), accumulated in fp32
         switch (epi) {
-            case EPI_F32: return launch_one<true, EPI_F32>(h, tmA, tmB, p, p.M, s);
-            case EPI_BF16OUT: return launch_one<true, EPI_BF16OUT>(h, tmA, tmB, p, p.M, s);
+            case EPI_F32: return launch_one<true, EPI_F32>(h, tmA, tmB, p, s);
+            case EPI_BF16OUT: return launch_one<true, EPI_BF16OUT>(h, tmA, tmB, p, s);
         }
         return xb_fail(h, XB_ERR_ARG, "no bf16 GEMM with epilogue %d", epi);
     }
-#define XB_EPI_CASE(E)                                                                       \
-    case E:                                                                                  \
-        return launch_one<false, E>(h, tmA, tmB, p, p.M, s);      /* fp16 operands in both weight modes (xb_api.cu repack) */
-    switch (epi) {
-        XB_EPI_CASE(EPI_F32)
-        XB_EPI_CASE(EPI_CONV3_BWD)
-#ifdef XB_EXPERIMENTS      // the tile-GEMM forms of conv3, the input projection, the head and the step-wise LSTM (cross-check builds only)
-        XB_EPI_CASE(EPI_CONV3)
-        XB_EPI_CASE(EPI_INPROJ)
-        XB_EPI_CASE(EPI_HEAD)
-        XB_EPI_CASE(EPI_LSTM)
-#endif
+    switch (epi) {      // fp16 operands in both weight modes (xb_api.cu repack)
+        case EPI_F32: return launch_one<false, EPI_F32>(h, tmA, tmB, p, s);
+        case EPI_CONV3_BWD: return launch_one<false, EPI_CONV3_BWD>(h, tmA, tmB, p, s);
     }
-#undef XB_EPI_CASE
     return xb_fail(h, XB_ERR_ARG, "unknown epilogue %d", epi);
 }

@@ -21,26 +21,16 @@
 // of W_ih, fp32 score rows with the blank score inserted leave as coalesced segments, two epilogue warp sets.
 //
 // Warp roles (256 threads; 384 for IP_SCORES): warp 0 TMA producer, warp 1 MMA issuer (+ tcgen05.cp of the x block),
-// warp 2 TMEM allocator, warps 4..7 (and 8..11) run the epilogues (warp % 4 = TMEM lane quarter).  XB_INPROJ_REGLOAD=1
-// selects the earlier x path (epilogue warps load the rows, transpose them through staging rows, tcgen05.st) in builds with
-// -DXB_EXPERIMENTS; the product library reads no environment variables.
-#include <stdlib.h>
-
+// warp 2 TMEM allocator, warps 4..7 (and 8..11) run the epilogues (warp % 4 = TMEM lane quarter).  The earlier x path
+// (epilogue warps load the rows, transpose them through staging rows, tcgen05.st) was measured and removed (DESIGN §4.2).
 #include "xb_common.cuh"
 #include "xb_ptx.cuh"
 #include "xb_gemm.cuh"
-#include "xb_head_epilogue.cuh"
 #include "xb_exact_math.h"
 
 using namespace xbptx;
 
 namespace {
-
-#ifdef XB_EXPERIMENTS
-#define IP_CLK() clock64()       // stall accounting of the MMA thread (XB_INPROJ_DEBUG)
-#else
-#define IP_CLK() 0ll
-#endif
 
 constexpr int BM = 128, BNI = 64, BK = 64;
 constexpr int KB = XB_FEATURES / BK;                 // 12 K blocks
@@ -70,9 +60,24 @@ struct IPParams {
     int n_base, expand;       // IP_SCORES: blank score inserted in front of every n_base columns
     float scale, blank;
     int exp_out;              // IP_SCORES: write E = xb_score_exp(score) (what the linear-domain decode consumes) instead of the score
-    int no_prefetch;
-    long long *dbg;           // optional (XB_INPROJ_DEBUG): stall cycles of the MMA thread of CTA 0: [acc_empty, full, issue, a_ready]
 };
+
+// LinearCRFEncoder (nn.py:117-129): scale * tanh(acc + bias), with the blank score written in front of every group of
+// n_base columns.
+__device__ __forceinline__ float fast_tanh(float x) { return 1.0f - __fdividef(2.0f, __expf(2.0f * x) + 1.0f); }
+
+// Output positions [seg_start, seg_start + seg_len) covered by head columns [col0, col_end).
+__device__ __forceinline__ void segment(int col0, int col_end, int nbs, int expand, int &seg_start, int &seg_len) {
+    seg_start = 0; seg_len = 0;
+    if (col_end <= col0) return;
+    if (expand) {
+        seg_start = col0 + col0 / nbs + ((col0 % nbs) ? 1 : 0);
+        seg_len = (col_end - 1) + (col_end - 1) / nbs + 2 - seg_start;
+    } else {
+        seg_start = col0;
+        seg_len = col_end - col0;
+    }
+}
 
 // LinearCRFEncoder expansion of one thread's 64 activated columns into its staged row (shared address sr, positions
 // relative to the segment start): column jj of the tile goes to pos0 + jj + (e0 + jj) / NB, the blank score in front of
@@ -105,14 +110,14 @@ __device__ __forceinline__ void head_stage64_dyn(const float (&v)[BNI], uint32_t
     }
 }
 
-// XCP: the x block reaches tensor memory as TMA boxes (two K blocks = one 32 KB ring stage, interleaved with the W stages by
+// The x block reaches tensor memory as TMA boxes (two K blocks = one 32 KB ring stage, interleaved with the W stages by
 // the producer) copied with tcgen05.cp by the MMA thread, in issue order with its MMAs -- no register / staging-row detour
 // through the epilogue warps, and the next tile's x stages are already in flight while the current tile finishes
 // (tools/tmem_cp_probe.cu checks the copy's layout: lane = row, column c = elements 2c, 2c+1, as the TS-mode MMA reads A).
-template <bool BF16, int EPI, bool XCP>
+template <int EPI>
 __global__ void __launch_bounds__(IPCfg<EPI>::THREADS, 1)
 inproj_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmX, const IPParams p) {
-    using X = xb16<BF16>;
+    using X = xb16<false>;                    // fp16 operands in both weight modes (xb_api.cu repack)
     constexpr int STAGES = IPCfg<EPI>::STAGES, STG_BYTES = IPCfg<EPI>::STG_BYTES;
     const int NT = p.NT;
     extern __shared__ uint8_t smem_raw[];
@@ -123,8 +128,7 @@ inproj_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ C
     uint64_t *empty = full + STAGES;
     uint64_t *acc_full = empty + STAGES;      // [2]
     uint64_t *acc_empty = acc_full + 2;       // [2]
-    uint64_t *a_ready = acc_empty + 2;        // [SPT]: K blocks ks*KPS .. ks*KPS+KPS-1 of the x block are in tensor memory
-    uint32_t *tmem_holder = reinterpret_cast<uint32_t *>(a_ready + SPT);
+    uint32_t *tmem_holder = reinterpret_cast<uint32_t *>(acc_empty + 2);
 
     const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;
     const int ntiles = (p.M + BM - 1) / BM;
@@ -139,7 +143,6 @@ inproj_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ C
             mbar_init(&acc_full[b], 1);
             mbar_init(&acc_empty[b], 4);
         }
-        for (int ks = 0; ks < SPT; ks++) mbar_init(&a_ready[ks], 4);
         fence_barrier_init();
     }
     if (warp == 2) {
@@ -157,13 +160,12 @@ inproj_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ C
         if (elect_one()) {
             uint32_t it = 0;
             for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-                if (XCP)
-                    for (int xs = 0; xs < KB / 2; xs++, it++) {            // x block: [128 rows x 64 K] x 2 K blocks per stage
-                        const int s = it % STAGES;
-                        mbar_wait(&empty[s], ((it / STAGES) & 1) ^ 1);
-                        mbar_expect_tx(&full[s], STAGE_BYTES);
-                        tma_load_3d(smem + s * STAGE_BYTES, &tmX, &full[s], 0, tile * BM, xs * 2);
-                    }
+                for (int xs = 0; xs < KB / 2; xs++, it++) {                // x block: [128 rows x 64 K] x 2 K blocks per stage
+                    const int s = it % STAGES;
+                    mbar_wait(&empty[s], ((it / STAGES) & 1) ^ 1);
+                    mbar_expect_tx(&full[s], STAGE_BYTES);
+                    tma_load_3d(smem + s * STAGE_BYTES, &tmX, &full[s], 0, tile * BM, xs * 2);
+                }
                 for (int nt = 0; nt < NT; nt++)
                     for (int ks = 0; ks < SPT; ks++, it++) {
                         const int s = it % STAGES;
@@ -175,49 +177,32 @@ inproj_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ C
         }
     } else if (warp == 1) {
         // ------------------------------------------------------------------ MMA issuer
-        constexpr uint32_t idesc = umma_idesc_f16(BF16 ? 1u : 0u, BM, BNI);
-        uint32_t it = 0, nit = 0, tit = 0;
-        long long st_acc = 0, st_full = 0, st_issue = 0, st_a = 0, tt;
-        const bool dbg = p.dbg && blockIdx.x == 0;
-        for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, tit++) {
-            if (XCP) {
-                tt = IP_CLK();
-                for (int xs = 0; xs < KB / 2; xs++, it++) {
-                    const int s = it % STAGES;
-                    mbar_wait(&full[s], (it / STAGES) & 1);
-                    tc_fence_after();
-                    if (elect_one()) {
-                        const uint64_t sdesc = umma_desc_sw128(smem_u32(smem + s * STAGE_BYTES));
+        constexpr uint32_t idesc = umma_idesc_f16(0u, BM, BNI);
+        uint32_t it = 0, nit = 0;
+        for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+            for (int xs = 0; xs < KB / 2; xs++, it++) {
+                const int s = it % STAGES;
+                mbar_wait(&full[s], (it / STAGES) & 1);
+                tc_fence_after();
+                if (elect_one()) {
+                    const uint64_t sdesc = umma_desc_sw128(smem_u32(smem + s * STAGE_BYTES));
 #pragma unroll
-                        for (int kk = 0; kk < 8; kk++)             // 2 K blocks x 4 slices of K = 16: 8 tensor-memory columns each
-                            tmem_cp_128x256b(tmem_base + (xs * 2) * (BK / 2) + kk * 8,
-                                             sdesc + (uint64_t)(((kk >> 2) * (BM * BK * 2) + (kk & 3) * 32) >> 4));
-                        mma_commit(&empty[s]);
-                    }
-                    __syncwarp();
+                    for (int kk = 0; kk < 8; kk++)                 // 2 K blocks x 4 slices of K = 16: 8 tensor-memory columns each
+                        tmem_cp_128x256b(tmem_base + (xs * 2) * (BK / 2) + kk * 8,
+                                         sdesc + (uint64_t)(((kk >> 2) * (BM * BK * 2) + (kk & 3) * 32) >> 4));
+                    mma_commit(&empty[s]);
                 }
-                st_a += IP_CLK() - tt;
+                __syncwarp();
             }
             for (int nt = 0; nt < NT; nt++, nit++) {
                 const int buf = nit & 1;
-                tt = IP_CLK();
                 mbar_wait(&acc_empty[buf], ((nit >> 1) & 1) ^ 1);
                 tc_fence_after();
-                st_acc += IP_CLK() - tt;
                 const uint32_t d = tmem_base + A_COLS + buf * BNI;
                 for (int ks = 0; ks < SPT; ks++, it++) {
                     const int s = it % STAGES;
-                    tt = IP_CLK();
                     mbar_wait(&full[s], (it / STAGES) & 1);
                     tc_fence_after();
-                    st_full += IP_CLK() - tt;
-                    if (!XCP && nt == 0) {                     // first N tile: the x block arrives K-block group by group
-                        tt = IP_CLK();
-                        mbar_wait(&a_ready[ks], tit & 1);
-                        tc_fence_after();
-                        st_a += IP_CLK() - tt;
-                    }
-                    tt = IP_CLK();
                     if (elect_one()) {
                         const uint64_t bdesc = umma_desc_sw128(smem_u32(smem + s * STAGE_BYTES));
                         const uint32_t a0 = tmem_base + ks * KPS * (BK / 2);
@@ -231,15 +216,13 @@ inproj_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ C
                         if (ks == SPT - 1) mma_commit(&acc_full[buf]);
                     }
                     __syncwarp();
-                    st_issue += IP_CLK() - tt;
                 }
             }
         }
-        if (dbg && lane == 0) { p.dbg[0] = st_acc; p.dbg[1] = st_full; p.dbg[2] = st_issue; p.dbg[3] = st_a; p.dbg[4] = tit; }
     } else if (warp >= 4) {
-        // ------------------------------------------------------------------ x block loader + epilogue
+        // ------------------------------------------------------------------ epilogue
         // Scores variant: two sets of four warps; set s runs the epilogues of the accumulators with (N-tile counter & 1) == s,
-        // so consecutive epilogues overlap (each is several times longer than the MMAs of an N tile); set 0 loads the x blocks.
+        // so consecutive epilogues overlap (each is several times longer than the MMAs of an N tile).
         constexpr int SETS = IPCfg<EPI>::SETS;
         const int set = (warp - 4) >> 2;
         const int q = warp & 3, r = q * 32 + lane;
@@ -289,11 +272,9 @@ inproj_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ C
                 // thread's row goes to a staged row (odd pitch: conflict free), rows leave as coalesced fp32 segments
                 constexpr int RS = 81;
                 float *S = reinterpret_cast<float *>(stg);
-                const bool dbg = p.dbg && blockIdx.x == 0 && warp == 4 && lane == 0;
-                const long long te0 = IP_CLK();
                 const int col0 = nt * BNI, col_end = min(col0 + BNI, p.n_valid);
                 int seg_start, seg_len;
-                xbhead::segment(col0, col_end, p.n_base, p.expand, seg_start, seg_len);
+                segment(col0, col_end, p.n_base, p.expand, seg_start, seg_len);
                 if (seg_len > 0) {
                     // activation first (64 independent MUFU chains), then the expansion with running positions: no
                     // compile-time variants per (n_base, group phase) here -- the issue slots are idle anyway, the instruction
@@ -301,7 +282,7 @@ inproj_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ C
                     const float *bs = sbias + col0;
                     float v[BNI];
 #pragma unroll
-                    for (int jj = 0; jj < BNI; jj++) v[jj] = p.scale * xbhead::fast_tanh(__uint_as_float(acc[jj]) + bs[jj]);
+                    for (int jj = 0; jj < BNI; jj++) v[jj] = p.scale * fast_tanh(__uint_as_float(acc[jj]) + bs[jj]);
                     // fused pipeline: hand the decode exp(score) -- the one exponential per edge its three sweeps would
                     // otherwise each compute (bit-reproducible xb_score_exp, the decode contract's own function)
                     if (p.exp_out) {
@@ -328,7 +309,6 @@ inproj_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ C
                             if (jj < ncols) sts_f32(sr + 4u * jj, v[jj]);
                     }
                     __syncwarp();
-                    if (dbg) p.dbg[6] += IP_CLK() - te0;
                     // four rows per round, all shared-memory loads before the stores: with only four epilogue warps per SM
                     // a load -> store chain per row segment leaves the copy-out latency-bound
                     float *obase = reinterpret_cast<float *>(p.out) + seg_start + lane;
@@ -355,7 +335,6 @@ inproj_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ C
                             }
                         }
                     }
-                    if (dbg) p.dbg[7] += IP_CLK() - te0;
                 }
             }
             __syncwarp();
@@ -366,66 +345,12 @@ inproj_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ C
         for (int tile = blockIdx.x; tile < ntiles || pending; tile += gridDim.x) {
             const bool valid = tile < ntiles;
             const int m0 = tile * BM;
-            // all MMAs of the previous tile have completed: its x block may be replaced (set 0), its last accumulator read
-            // (the set that owns it; a set never waits on the other set's barrier, it could fall two phases behind)
-            if (pending && ((!XCP && set == 0) || SETS == 1 || (int)((nit - 1) & 1) == set)) {
+            // all MMAs of the previous tile have completed: its last accumulator may be read (by the set that owns it; a set
+            // never waits on the other set's barrier, it could fall two phases behind)
+            if (pending && (SETS == 1 || (int)((nit - 1) & 1) == set)) {
                 mbar_wait(&acc_full[(nit - 1) & 1], ((nit - 1) >> 1) & 1);
                 tc_fence_after();
             }
-            const long long tl0 = IP_CLK();
-            if (!XCP && valid && set == 0) {   // x block -> tensor memory (lane = row, column c holds elements k = 2c, 2c+1).  The tensor pipe idles
-                // during this, so it has to be quick: a direct row-per-thread read costs one L1 wavefront per lane
-                // (12 k wavefronts per tile, ~20 k cycles).  Instead a warp reads its 32 rows coalesced, 128 bytes
-                // (= one K block) of four rows per instruction, four K blocks in flight, transposes through its
-                // staging rows and hands each thread its own row for tcgen05.st.
-                const int sub = lane >> 3, l8 = lane & 7;
-                const int mrow0 = m0 + q * 32;
-                // Two K blocks per round, two rounds in flight (register double buffer): the global loads of the next round
-                // are issued before the current one is transposed, so only the first round exposes the L2 / HBM latency.
-                constexpr int NBK = 2;
-                static_assert(KPS == 2 * NBK && KB % KPS == 0, "one a_ready group = two rounds");
-                uint4 ldA[NBK][8], ldB[NBK][8];
-                auto issue = [&](uint4 (&ld)[NBK][8], int kb0) {
-#pragma unroll
-                    for (int b = 0; b < NBK; b++)
-#pragma unroll
-                        for (int i = 0; i < 8; i++) {
-                            const int mm = mrow0 + 4 * i + sub;
-                            ld[b][i] = (mm < p.M) ? __ldg(reinterpret_cast<const uint4 *>(p.x + (size_t)mm * XB_FEATURES + (kb0 + b) * BK) + l8)
-                                                  : make_uint4(0, 0, 0, 0);
-                        }
-                };
-                auto consume = [&](uint4 (&ld)[NBK][8], int kb0) {
-#pragma unroll
-                    for (int b = 0; b < NBK; b++) {
-#pragma unroll
-                        for (int i = 0; i < 8; i++)
-                            sts_v4(stg_s + (4 * i + sub) * ROW_PITCH + l8 * 16, ld[b][i]);
-                        __syncwarp();
-                        uint32_t v[32];
-#pragma unroll
-                        for (int i = 0; i < 8; i++) {
-                            const uint4 t4 = lds_v4(stg_s + lane * ROW_PITCH + i * 16);
-                            v[4 * i] = t4.x; v[4 * i + 1] = t4.y; v[4 * i + 2] = t4.z; v[4 * i + 3] = t4.w;
-                        }
-                        __syncwarp();
-                        tmem_st_32x32b_x32(lane_base + (kb0 + b) * (BK / 2), v);
-                    }
-                };
-                issue(ldA, 0);
-#pragma unroll 1
-                for (int kb0 = 0; kb0 < KB; kb0 += KPS) {
-                    issue(ldB, kb0 + NBK);
-                    consume(ldA, kb0);
-                    if (kb0 + KPS < KB) issue(ldA, kb0 + KPS);
-                    consume(ldB, kb0 + NBK);
-                    tmem_st_wait();                            // the MMAs of the first N tile start on this group at once
-                    tc_fence_before();
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive(&a_ready[kb0 / KPS]);
-                }
-            }
-            if (p.dbg && blockIdx.x == 0 && warp == 4 && lane == 0) p.dbg[5] += IP_CLK() - tl0;
             // nt = -1: the previous tile's last N tile (its accumulator was awaited above), then N tiles 0 .. NT-2 of this one
             for (int nt = -1; nt < (valid ? NT - 1 : 0); nt++) {
                 int em0, ent;
@@ -435,7 +360,7 @@ inproj_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ C
                     em0 = pend_m0; ent = NT - 1; eni = nit - 1;
                 } else {
                     if (SETS > 1 && (int)(nit & 1) != set) { nit++; continue; }
-                    if (nt == (NT > 8 ? NT - 8 : 0) && !p.no_prefetch) {      // next tile's x rows into L2 shortly before they are needed (G streams through L2)
+                    if (nt == (NT > 8 ? NT - 8 : 0)) {      // next tile's x rows into L2 shortly before they are needed (G streams through L2)
                         const int mn = m0 + (int)gridDim.x * BM + r;
                         if (mn < p.M) {
                             const char *nx = reinterpret_cast<const char *>(p.x + (size_t)mn * XB_FEATURES);
@@ -451,7 +376,7 @@ inproj_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ C
                 epilogue(em0, ent, eni);
             }
             if (valid) {
-                nit++;                                         // the last N tile is finished after the next x load
+                nit++;                                         // the last N tile is finished in the next round
                 pend_m0 = m0;
             }
             pending = valid;
@@ -473,47 +398,17 @@ static int ip_launch(xb_handle *h, const void *w, int w_rows, IPParams p, cudaSt
     if (int rc = xb_make_tmap_hview(h, &tmW, w, w_rows, BNI, KPS)) return rc;
     if (int rc = xb_make_tmap_hview(h, &tmX, p.x, (uint64_t)p.M, BM, 2)) return rc;
     p.NT = w_rows / BNI;
-    p.dbg = nullptr;
-    p.no_prefetch = 0;
-#ifdef XB_EXPERIMENTS
-    static const bool regload = getenv("XB_INPROJ_REGLOAD") != nullptr;     // the earlier x path through registers / staging rows
-    p.no_prefetch = getenv("XB_INPROJ_NOPF") ? 1 : 0;
-    if (getenv("XB_INPROJ_DEBUG")) {
-        static long long *d = nullptr;
-        if (!d) cudaMalloc(&d, 64);
-        p.dbg = d;
-    }
-#endif
     const int ntiles = (p.M + BM - 1) / BM;
     const int grid = ntiles < h->num_sms ? ntiles : h->num_sms;
     constexpr int SMEM_BYTES = IPCfg<EPI>::SMEM_BYTES;
-    static bool configured[4][64] = {};   // per device: function attributes live in the device's context
-    const int dv = h->device & 63;
-    auto go = [&](auto kernel, int slot) -> int {
-        if (!configured[slot][dv]) {
-            XB_CUDA(h, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-            configured[slot][dv] = true;
-        }
-        kernel<<<grid, IPCfg<EPI>::THREADS, SMEM_BYTES, s>>>(tmW, tmX, p);
-        return XB_OK;
-    };
-    int rc;
-#ifdef XB_EXPERIMENTS
-    if (regload) rc = go(inproj_kernel<false, EPI, false>, 2);
-    else
-#endif
-    rc = go(inproj_kernel<false, EPI, true>, 3);       // fp16 operands in both weight modes (xb_api.cu repack)
-    if (rc) return rc;
-    XB_LAUNCH_CHECK(h);
-#ifdef XB_EXPERIMENTS
-    if (p.dbg) {
-        long long v[8];
-        cudaDeviceSynchronize();
-        cudaMemcpy(v, p.dbg, sizeof v, cudaMemcpyDeviceToHost);
-        fprintf(stderr, "inproj MMA thread of CTA 0: %lld tiles; stall cycles: acc_empty %lld, full %lld, a_ready %lld; issue %lld; x-block load (warp 4) %lld; head epilogue stage %lld, stage+copy %lld\n", v[4], v[0], v[1], v[3], v[2], v[5], v[6], v[7]);
-        cudaMemset(p.dbg, 0, 64);
+    auto kernel = inproj_kernel<EPI>;
+    static bool configured[64] = {};      // per device: function attributes live in the device's context
+    if (!configured[h->device & 63]) {
+        XB_CUDA(h, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+        configured[h->device & 63] = true;
     }
-#endif
+    kernel<<<grid, IPCfg<EPI>::THREADS, SMEM_BYTES, s>>>(tmW, tmX, p);
+    XB_LAUNCH_CHECK(h);
     return XB_OK;
 }
 

@@ -30,22 +30,13 @@
 // Warp roles: warps 0..SUB-1 drive one sub-batch each (one elected thread: counter poll, h boxes, then the step's
 // MMAs part by part as the boxes land, commit; plus the G prefetch), warp SUB allocates tensor memory, epilogue
 // warps start at the next multiple of four, EW (= 8) per sub-batch (warp % 4 = TMEM lane
-// quarter; the second four take the upper half of the chunk columns).  A build with -DXB_EXPERIMENTS adds the measured
-// alternatives behind XB_LSTM_VARIANT (1: four epilogue warps, 2: six sub-batches of 16 chunks, 3: two of 48 chunks with
-// twelve epilogue warps, 4: four of 32 chunks with four epilogue warps each and a single G buffer per sub-batch -- 96 CTAs
-// at N = 512), the per-warp release (XB_LSTM_WARP_RELEASE=1) and the step timeline (XB_LSTM_DEBUG=1); the product
-// library contains the one configuration below and reads no environment variables.
-#include <stdlib.h>
-
+// quarter; the second four take the upper half of the chunk columns).  The other geometries, publish paths and
+// activation forms that were measured against this one are recorded in DESIGN §4.1.
 #include "xb_common.cuh"
 #include "xb_ptx.cuh"
 #include "xb_gemm.cuh"
 
 using namespace xbptx;
-
-#ifndef XB_LSTM_MUFU_TANH
-#define XB_LSTM_MUFU_TANH 1      // 0: exp/rcp activations (7 MUFU + ~45 FP ops per cell), 1: MUFU.TANH (5 MUFU + ~12)
-#endif
 
 namespace {
 
@@ -57,27 +48,28 @@ constexpr int KPB = KCH / HP;              // K blocks per box
 constexpr int D_COL = 384;                 // accumulators start after the 384 columns of W_hh
 constexpr int CTR_STRIDE = 32;             // ints between counters (one 128-byte line each)
 constexpr int MAX_CTRS = 64;
+constexpr int PREFETCH_Y = 4;              // the y rows of step s + PREFETCH_Y are prefetched into L2 at step s
 
-template <int SUB, int NS, int EW, int GB = 2> struct Cfg {  // EW = epilogue warps per sub-batch; GB = G buffers per sub-batch
-    static constexpr int NB = SUB * NS;                       // chunks per group
-    static constexpr int H_BLOCK_BYTES = NS * 64 * 2;         // one K block: NS rows x 128 B
-    static constexpr int H_PART_BYTES = KPB * H_BLOCK_BYTES;
-    static constexpr int H_BYTES = KCH * H_BLOCK_BYTES;
-    static constexpr int G_BYTES = NS * 128 * 2;
-    static constexpr int NBAR = HP + 1 + 4;                   // h_full[HP], d_full, g_full[2], g_empty[2]
-    static constexpr int EPI_WARP0 = ((SUB + 1 + 3) / 4) * 4;
-    static constexpr int THREADS = (EPI_WARP0 + EW * SUB) * 32;
-    static constexpr int NC = NS * 4 / EW;                    // accumulator columns (chunks) per epilogue warp
-    static constexpr int STAGE_BYTES = NC * 16;               // per epilogue warp: [chunk][8 units] 16-bit
-    // GB == 1 (four-chain variant): one G buffer per sub-batch, refilled after the epilogue has consumed it, and the h-slice
-    // staging rows alias the bytes of it that the same warp read -- 4 x (48 + 8) KB + barriers just fit 227 KB
-    static constexpr int SMEM_BYTES = SUB * (H_BYTES + GB * G_BYTES) + (GB == 2 ? SUB * EW * STAGE_BYTES : 0) + 1024 /*align*/ + 1024 /*barriers*/;
-    static_assert(D_COL + SUB * NS <= 512, "tensor memory columns");
-    static_assert(NS % 16 == 0 && NS <= 48, "MMA N");
-    static_assert((EW == 4 || EW == 8 || EW == 12) && NC % 16 == 0, "epilogue split");
-    static_assert(SUB * NBAR * 8 + 16 <= 1024, "barrier block");
-    static_assert(H_BLOCK_BYTES % 1024 == 0, "swizzle atom alignment");
-};
+// Geometry: SUB sub-batches of NS chunks per CTA, EW epilogue warps per sub-batch, two G buffers per sub-batch.
+constexpr int SUB = 3;
+constexpr int NS = 32;
+constexpr int EW = 8;
+constexpr int NB = SUB * NS;                       // chunks per group
+constexpr int H_BLOCK_BYTES = NS * 64 * 2;         // one K block: NS rows x 128 B
+constexpr int H_PART_BYTES = KPB * H_BLOCK_BYTES;
+constexpr int H_BYTES = KCH * H_BLOCK_BYTES;
+constexpr int G_BYTES = NS * 128 * 2;
+constexpr int NBAR = HP + 1 + 4;                   // h_full[HP], d_full, g_full[2], g_empty[2]
+constexpr int EPI_WARP0 = ((SUB + 1 + 3) / 4) * 4;
+constexpr int THREADS = (EPI_WARP0 + EW * SUB) * 32;
+constexpr int NC = NS * 4 / EW;                    // accumulator columns (chunks) per epilogue warp
+constexpr int STAGE_BYTES = NC * 16;               // per epilogue warp: [chunk][8 units] 16-bit
+constexpr int SMEM_BYTES = SUB * (H_BYTES + 2 * G_BYTES + EW * STAGE_BYTES) + 1024 /*align*/ + 1024 /*barriers*/;
+static_assert(D_COL + SUB * NS <= 512, "tensor memory columns");
+static_assert(NS % 16 == 0 && NS <= 48, "MMA N");
+static_assert(EW % 4 == 0 && NC == 16, "epilogue split: one pair of tcgen05.ld.16x256b.x2 per warp and step");
+static_assert(SUB * NBAR * 8 + 16 <= 1024, "barrier block");
+static_assert(H_BLOCK_BYTES % 1024 == 0, "swizzle atom alignment");
 
 struct PLParams {
     int T, N, reverse;
@@ -85,78 +77,44 @@ struct PLParams {
     const uint16_t *w_hh;       // (3072, 768) 16-bit, tile-permuted rows (repack mode 4 in xb_api.cu)
     uint16_t *y;                // (T, N, 768) 16-bit output = hidden states
     int *counters;              // G * SUB counters, CTR_STRIDE ints apart, zeroed before launch
-    int one_release;            // 1: one MEMBAR + counter update per sub-batch and step, 0: one per epilogue warp
-    int prefetch_y;             // d > 0: prefetch the y rows of step s+d into L2
-    long long *dbg;             // optional timeline (XB_EXPERIMENTS, XB_LSTM_DEBUG=1): clock64 stamps of CTA 0, sub-batch 0
-    int tma_store;              // XB_EXPERIMENTS: 1 / 2 = full sub-batches publish h through a TMA tensor store (release / relaxed counter)
     uint16_t *save;             // training forward (SAVE kernels): (T, N, 5, 768) fp16 = activated i, f, g, o and the cell state c
 };
-
-#ifdef XB_EXPERIMENTS
-#define DBG(sub_, ev) do { if (p.dbg && blockIdx.x == 0 && s >= 64 && s < 72) p.dbg[((s - 64) * 8 + (sub_)) * 16 + (ev)] = clock64(); } while (0)
-#else
-#define DBG(sub_, ev) do { } while (0)
-#endif
 
 __device__ __forceinline__ float tanh_approx(float x) {
     float y;
     asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
     return y;
 }
-#if !XB_LSTM_MUFU_TANH
-__device__ __forceinline__ float ex2f(float x) {
-    float y;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-    return y;
-}
-__device__ __forceinline__ float rcpf(float x) {
-    float y;
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-    return y;
-}
-__device__ __forceinline__ float clampf(float x, float lim) { return fminf(fmaxf(x, -lim), lim); }
-#endif
-
-// tcgen05.ld.16x256b.xN: 16 lanes x (N * 8) columns; thread t gets rows t/4 and t/4+8, columns 8k + 2(t%4), +1:
+// tcgen05.ld.16x256b.x2: 16 lanes x 16 columns; thread t gets rows t/4 and t/4+8, columns 8k + 2(t%4), +1:
 // r[4k + {0,1}] = row t/4, r[4k + {2,3}] = row t/4 + 8  (layout checked on hardware: tools/tmem_layout_probe.cu)
-template <int XN> __device__ __forceinline__ void tmem_ld_16x256b(uint32_t taddr, uint32_t (&r)[4 * XN]);
-template <> __device__ __forceinline__ void tmem_ld_16x256b<2>(uint32_t taddr, uint32_t (&r)[8]) {
+__device__ __forceinline__ void tmem_ld_16x256b_x2(uint32_t taddr, uint32_t (&r)[8]) {
     asm volatile("tcgen05.ld.sync.aligned.16x256b.x2.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
                  : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
                  : "r"(taddr) : "memory");
 }
-template <> __device__ __forceinline__ void tmem_ld_16x256b<4>(uint32_t taddr, uint32_t (&r)[16]) {
-    asm volatile("tcgen05.ld.sync.aligned.16x256b.x4.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-                   "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-                 : "r"(taddr) : "memory");
-}
-template <bool BF16, int SUB, int NS, int EW, int GB, bool SAVE = false>
-__global__ void __launch_bounds__(Cfg<SUB, NS, EW, GB>::THREADS, 1)
-lstm_persistent_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_constant__ CUtensorMap tmG,
-                       const __grid_constant__ CUtensorMap tmS, const PLParams p) {
-    using X = xb16<BF16>;
-    using C = Cfg<SUB, NS, EW, GB>;
+template <bool SAVE>
+__global__ void __launch_bounds__(THREADS, 1)
+lstm_persistent_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_constant__ CUtensorMap tmG, const PLParams p) {
+    using X = xb16<false>;                                      // fp16 operands in both weight modes (xb_api.cu repack)
     extern __shared__ uint8_t smem_raw[];
     uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     uint8_t *hbuf = smem;                                       // [SUB][H_BYTES]
-    uint8_t *gbuf = smem + SUB * C::H_BYTES;                    // [SUB][GB][G_BYTES]
-    uint8_t *stage = gbuf + SUB * GB * C::G_BYTES;              // [SUB][EW][STAGE_BYTES] (GB == 2 only)
-    uint64_t *bars = reinterpret_cast<uint64_t *>(stage + (GB == 2 ? SUB * EW * C::STAGE_BYTES : 0));
-    uint32_t *tmem_holder = reinterpret_cast<uint32_t *>(bars + SUB * C::NBAR);
-    auto h_full = [&](int sub, int part) { return bars + sub * C::NBAR + part; };
-    auto d_full = [&](int sub) { return bars + sub * C::NBAR + HP; };
-    auto g_full = [&](int sub, int q) { return bars + sub * C::NBAR + HP + 1 + q; };
-    auto g_empty = [&](int sub, int q) { return bars + sub * C::NBAR + HP + 3 + q; };
+    uint8_t *gbuf = smem + SUB * H_BYTES;                       // [SUB][2][G_BYTES]
+    uint8_t *stage = gbuf + SUB * 2 * G_BYTES;                  // [SUB][EW][STAGE_BYTES]
+    uint64_t *bars = reinterpret_cast<uint64_t *>(stage + SUB * EW * STAGE_BYTES);
+    uint32_t *tmem_holder = reinterpret_cast<uint32_t *>(bars + SUB * NBAR);
+    auto h_full = [&](int sub, int part) { return bars + sub * NBAR + part; };
+    auto d_full = [&](int sub) { return bars + sub * NBAR + HP; };
+    auto g_full = [&](int sub, int q) { return bars + sub * NBAR + HP + 1 + q; };
+    auto g_empty = [&](int sub, int q) { return bars + sub * NBAR + HP + 3 + q; };
 
     // warp index through a shuffle: tells the compiler it is warp-uniform, so the role branches below are
     // non-divergent and the epilogue shuffles need no re-convergence barriers
     const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;
     const int g = blockIdx.x / TILES, j = blockIdx.x % TILES;
     const int T = p.T, N = p.N;
-    // Groups take whole sub-batches of NS chunks (units): every sub-batch but the batch's last is full, which lets a full
-    // sub-batch publish its h tile with ONE TMA store (a box of NS rows); the step time is set by the chain latency, not by
-    // the number of chains per SM, so groups of two and of three sub-batches cost the same.
+    // Groups take whole sub-batches of NS chunks (units): every sub-batch but the batch's last is full; the step time is set
+    // by the chain latency, not by the number of chains per SM, so groups of two and of three sub-batches cost the same.
     const int units = (p.nbatch + NS - 1) / NS;
     const int b0 = p.batch0 + NS * (int)(((long long)g * units) / p.G);
     const int b1 = min(p.batch0 + p.nbatch, p.batch0 + NS * (int)(((long long)(g + 1) * units) / p.G));
@@ -187,7 +145,7 @@ lstm_persistent_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_con
     const uint32_t tmem_base = *tmem_holder;
 
     // W_hh tile -> tensor memory: lane = row of the tile, column c holds elements k = 2c, 2c+1
-    if (warp >= C::EPI_WARP0 && warp < C::EPI_WARP0 + 4) {
+    if (warp >= EPI_WARP0 && warp < EPI_WARP0 + 4) {
         const int q = warp & 3, r = q * 32 + lane;
         const uint4 *src = reinterpret_cast<const uint4 *>(p.w_hh + ((size_t)j * 128 + r) * XB_FEATURES);
         const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16);
@@ -216,35 +174,36 @@ lstm_persistent_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_con
             const int row0 = sub_row0(sub);
             const int cnt_sub = sub_cnt(sub);
             const int *ctr = p.counters + (g * SUB + sub) * CTR_STRIDE;
-            uint8_t *hb = hbuf + sub * C::H_BYTES;
-            constexpr uint32_t idesc = umma_idesc_f16(BF16 ? 1u : 0u, 128, NS);
+            uint8_t *hb = hbuf + sub * H_BYTES;
+            constexpr uint32_t idesc = umma_idesc_f16(0u, 128, NS);
             const uint64_t bdesc0 = umma_desc_sw128(smem_u32(hb));
             const uint32_t dcol = tmem_base + D_COL + sub * NS;
             if (cnt_sub > 0) {
-                mbar_expect_tx(g_full(sub, 0), C::G_BYTES);
-                tma_load_2d(gbuf + (sub * GB) * C::G_BYTES, &tmG, g_full(sub, 0), j * 128, (p.reverse ? T - 1 : 0) * N + row0);
+                mbar_expect_tx(g_full(sub, 0), G_BYTES);
+                tma_load_2d(gbuf + (sub * 2) * G_BYTES, &tmG, g_full(sub, 0), j * 128, (p.reverse ? T - 1 : 0) * N + row0);
             }
             for (int s = 0; s < (cnt_sub > 0 ? T : 0); s++) {      // an empty sub-batch (a short last group) has no chain
                 const int t = p.reverse ? T - 1 - s : s;
-                if (GB == 2 && s + 1 < T) {      // input projection of the next step, one step ahead
+                if (s + 1 < T) {                 // input projection of the next step, one step ahead
                     const int sn = s + 1, q = sn & 1, u = sn >> 1;
                     const int tn = p.reverse ? T - 1 - sn : sn;
                     if (u >= 1) mbar_wait(g_empty(sub, q), (u - 1) & 1);
-                    mbar_expect_tx(g_full(sub, q), C::G_BYTES);
-                    tma_load_2d(gbuf + (sub * 2 + q) * C::G_BYTES, &tmG, g_full(sub, q), j * 128, tn * N + row0);
+                    mbar_expect_tx(g_full(sub, q), G_BYTES);
+                    tma_load_2d(gbuf + (sub * 2 + q) * G_BYTES, &tmG, g_full(sub, q), j * 128, tn * N + row0);
                 }
-                if (p.prefetch_y && s + p.prefetch_y < T) {
-                    // bring the y rows this sub-batch will write two steps from now into L2 (one row per CTA and sub-batch,
-                    // round robin over the group's tiles): a 16-byte store to a line that is not resident is only
-                    // acknowledged after the line was fetched from HBM, which is what the release below waits for
-                    const int t2 = p.reverse ? T - 1 - (s + p.prefetch_y) : s + p.prefetch_y;
+                if (s + PREFETCH_Y < T) {
+                    // bring the y rows this sub-batch will write PREFETCH_Y steps from now into L2 (one row per CTA and
+                    // sub-batch, round robin over the group's tiles): a 16-byte store to a line that is not resident is only
+                    // acknowledged after the line was fetched from HBM, which is what the release below waits for.  At most
+                    // two rows (NS <= 2 * TILES): unrolled, the loop held five more registers than the kernel needs elsewhere.
+                    const int t2 = p.reverse ? T - 1 - (s + PREFETCH_Y) : s + PREFETCH_Y;
+#pragma unroll 1
                     for (int r = j; r < cnt_sub; r += TILES)
                         prefetch_l2_bulk(p.y + ((size_t)t2 * N + row0 + r) * XB_FEATURES, XB_FEATURES * 2);
                 }
                 if (s > 0) {
                     const int tp = p.reverse ? t + 1 : t - 1;
                     const int need = TILES * EW * s;         // every epilogue warp of the group has published step s-1
-                    DBG(sub, 0);
                     // relaxed spin (an acquire load per iteration costs a CCTL.IVALL each time), then ONE acquire load of
                     // the counter once it has been seen at its target: that load synchronises with the producers'
                     // red.release (PTX memory model: a relaxed load alone does not), the proxy fence then orders the
@@ -252,16 +211,14 @@ lstm_persistent_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_con
                     while (ld_relaxed_gpu(ctr) < need) {
                     }
                     (void)ld_acquire_gpu(ctr);
-                    DBG(sub, 1);
                     fence_proxy_async_global();
                     // h_{t-1} of the sub-batch: HP boxes {64 k, NS chunks, KPB k-blocks}, each landing as KPB
                     // swizzled [NS x 128 B] K-major tiles on its own mbarrier
 #pragma unroll
                     for (int part = 0; part < HP; part++) {
-                        mbar_expect_tx(h_full(sub, part), C::H_PART_BYTES);
-                        tma_load_3d(hb + part * C::H_PART_BYTES, &tmY, h_full(sub, part), 0, tp * N + row0, part * KPB);
+                        mbar_expect_tx(h_full(sub, part), H_PART_BYTES);
+                        tma_load_3d(hb + part * H_PART_BYTES, &tmY, h_full(sub, part), 0, tp * N + row0, part * KPB);
                     }
-                    DBG(sub, 2);
                     // ... and the MMAs of the step, part by part as the boxes land (blocking try_wait: ~60 cycles from
                     // completion to wake-up; an earlier single MMA warp scanning all sub-batches with test_wait paid
                     // ~150 cycles per probe and could not keep up with more than one box per step)
@@ -269,47 +226,32 @@ lstm_persistent_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_con
                     for (int part = 0; part < HP; part++) {
                         mbar_wait(h_full(sub, part), (s - 1) & 1);
                         tc_fence_after();
-                        if (part == 0) DBG(sub, 8);
-                        if (part == 0) DBG(sub, 3);
 #pragma unroll
                         for (int kk = 0; kk < KPB * 4; kk++) {
                             const int kc = kk >> 2, k = kk & 3;
                             mma_f16_ts(dcol, tmem_base + part * (KPB * 32) + kk * 8,
-                                       bdesc0 + (uint64_t)((part * C::H_PART_BYTES + kc * C::H_BLOCK_BYTES + k * 32) >> 4), idesc,
+                                       bdesc0 + (uint64_t)((part * H_PART_BYTES + kc * H_BLOCK_BYTES + k * 32) >> 4), idesc,
                                        (part | kk) != 0);
                         }
                     }
                     mma_commit(d_full(sub));
-                    DBG(sub, 4);
-                }
-                if (GB == 1 && s + 1 < T) {      // single G buffer: refill once this step's epilogue is through with it
-                    const int tn = p.reverse ? T - 2 - s : s + 1;
-                    mbar_wait(g_empty(sub, 0), s & 1);
-                    mbar_expect_tx(g_full(sub, 0), C::G_BYTES);
-                    tma_load_2d(gbuf + sub * C::G_BYTES, &tmG, g_full(sub, 0), j * 128, tn * N + row0);
                 }
             }
         }
-    } else if (warp >= C::EPI_WARP0) {
+    } else if (warp >= EPI_WARP0) {
         // ------------------------------------------------------------------ epilogue (EW warps per sub-batch: warp % 4 =
-        // TMEM lane quarter; with EW = 8 the second four take the upper half of the chunk columns)
-        constexpr int NC = C::NC, CELLS = NC / 4;
-        const int ew = (warp - C::EPI_WARP0) % EW, sub = (warp - C::EPI_WARP0) / EW, q = warp & 3;
+        // TMEM lane quarter; the second four take the upper half of the chunk columns)
+        constexpr int CELLS = NC / 4;
+        const int ew = (warp - EPI_WARP0) % EW, sub = (warp - EPI_WARP0) / EW, q = warp & 3;
         const int col0 = (ew >> 2) * NC;                     // first chunk column of this warp
         const int gt = lane & 3, ul = lane >> 2;             // gate held after the TMEM load; unit within the warp
         const int unit = q * 8 + ul;                         // unit within the tile
         const int row0 = sub_row0(sub);
         const int cnt = sub_cnt(sub);                            // valid chunks of this sub-batch (<= NS)
-        // Round-2 experiment (XB_EXPERIMENTS builds, XB_TMAS=1|2): a FULL sub-batch publishes its h tile through the async
-        // proxy -- staged as a dense [NS chunks][32 units] tile, ONE TMA tensor store, cp.async.bulk.wait_group for its
-        // completion, then the counter.  With a release on the counter it is as fast as the generic route below (14.1 ms per
-        // batch); with a relaxed add it is 8-10 % faster (12.5-13.1 ms), but then nothing orders the tile's writes before the
-        // counter in the PTX memory model, so the product publishes through generic stores + red.release.
-#ifdef XB_EXPERIMENTS
-        const bool tma_store = !SAVE && GB == 2 && cnt == NS && p.tma_store;
-#else
-        constexpr bool tma_store = false;
-#endif
+        // h is published through generic stores + red.release.  Publishing a full sub-batch's tile with one TMA tensor store
+        // was measured and removed: with a release on the counter it was as fast as this route (14.1 ms per batch); with a
+        // relaxed add it was 8-10 % faster (12.5-13.1 ms), but then nothing orders the tile's writes before the counter in
+        // the PTX memory model.
         const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + D_COL + sub * NS + col0;
         int *ctr = p.counters + (g * SUB + sub) * CTR_STRIDE;
         float cst[CELLS];
@@ -318,7 +260,7 @@ lstm_persistent_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_con
 
         for (int s = 0; s < (cnt > 0 ? T : 0); s++) {
             const int t = p.reverse ? T - 1 - s : s;
-            const uint16_t *Gs = reinterpret_cast<const uint16_t *>(gbuf + (sub * GB + (GB == 2 ? (s & 1) : 0)) * C::G_BYTES);
+            const uint16_t *Gs = reinterpret_cast<const uint16_t *>(gbuf + (sub * 2 + (s & 1)) * G_BYTES);
             // Accumulator -> registers with tcgen05.ld.16x256b: thread (a = lane/4, b = lane%4) receives rows a, a+8 (first
             // load) and a+16, a+24 (second load, 16 lanes further) of columns 8k+2b, 8k+2b+1.  The rows of a lane quarter are
             // ordered gate*8 + unit, so those four rows are i, f, g, o of unit a: the load itself delivers whole cells
@@ -326,7 +268,7 @@ lstm_persistent_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_con
             // The input projection of the step arrived a step ago: fetch it from shared memory BEFORE waiting for the
             // accumulator, so only the adds remain on the serial chain.
             // cell m of the thread: chunk 8*(m/2) + 2b + m%2 (relative to col0), unit ul
-            mbar_wait(g_full(sub, GB == 2 ? (s & 1) : 0), GB == 2 ? ((s >> 1) & 1) : (s & 1));
+            mbar_wait(g_full(sub, s & 1), (s >> 1) & 1);
             float pre[CELLS][4];
 #pragma unroll
             for (int m = 0; m < CELLS; m++) {
@@ -335,17 +277,14 @@ lstm_persistent_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_con
                 const float2 g01 = X::unpack(graw.x), g23 = X::unpack(graw.y);
                 pre[m][0] = g01.x; pre[m][1] = g01.y; pre[m][2] = g23.x; pre[m][3] = g23.y;
             }
-            if (ew == 0 && lane == 0) DBG(sub, 11);
             if (s > 0) {
                 uint32_t lo[NC / 2], hi[NC / 2];
                 mbar_wait(d_full(sub), (s - 1) & 1);
                 tc_fence_after();
-                if (ew == 0 && lane == 0) DBG(sub, 9);
-                tmem_ld_16x256b<NC / 8>(taddr, lo);
-                tmem_ld_16x256b<NC / 8>(taddr + (16u << 16), hi);
+                tmem_ld_16x256b_x2(taddr, lo);
+                tmem_ld_16x256b_x2(taddr + (16u << 16), hi);
                 tmem_ld_wait();
                 tc_fence_before();
-                if (ew == 0 && lane == 0) DBG(sub, 10);
 #pragma unroll
                 for (int m = 0; m < CELLS; m++) {
                     const int k4 = 4 * (m >> 1), wi = m & 1;
@@ -355,14 +294,13 @@ lstm_persistent_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_con
                     pre[m][3] += __uint_as_float(hi[k4 + 2 + wi]);
                 }
             }
-            if (ew == 0 && lane == 0) DBG(sub, 6);
             // phase B: c' = sig(f) c + sig(i) tanh(g), h = sig(o) tanh(c'), written stage by stage over all cells so
             // that the MUFU latencies overlap.
             float hout[CELLS];
             float sv[SAVE ? 5 : 1][CELLS];           // training forward: what BPTT needs of this step
-#if XB_LSTM_MUFU_TANH
             // Five MUFU.TANH per cell (sigmoid(x) = 0.5 tanh(0.5 x) + 0.5) and a dozen FMAs: a third of the instructions
-            // of the exp/rcp form below.  tanh.approx.f32 has ~2^-11 relative error, the size of the fp16 rounding of h.
+            // of the exp/rcp form (7 MUFU + ~45 FP ops per cell), which was measured and removed.  tanh.approx.f32 has
+            // ~2^-11 relative error, the size of the fp16 rounding of h.
 #pragma unroll
             for (int i = 0; i < CELLS; i++) {
                 const float si = fmaf(tanh_approx(0.5f * pre[i][0]), 0.5f, 0.5f);
@@ -374,77 +312,11 @@ lstm_persistent_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_con
                 hout[i] = so * tanh_approx(cn);
                 if (SAVE) { sv[0][i] = si; sv[SAVE ? 1 : 0][i] = sf; sv[SAVE ? 2 : 0][i] = tg; sv[SAVE ? 3 : 0][i] = so; sv[SAVE ? 4 : 0][i] = cn; }
             }
-#else
-            // Seven MUFU ops per cell: the four gate activations share one reciprocal (1/(d_i d_f d_g d_o) times the
-            // complementary products); inputs are clamped so that the product of the four denominators stays far from
-            // fp32 overflow (sigmoid(-15) = 3e-7, tanh(7.5) = 1 - 6e-7)
-            constexpr float L2E = 1.4426950408889634f;
-            float ei[CELLS], ef[CELLS], eg[CELLS], eo[CELLS], rr[CELLS];
-#pragma unroll
-            for (int i = 0; i < CELLS; i++) {
-                ei[i] = ex2f(-L2E * clampf(pre[i][0], 15.f));
-                ef[i] = ex2f(-L2E * clampf(pre[i][1], 15.f));
-                eg[i] = ex2f(-2.f * L2E * clampf(pre[i][2], 7.5f));
-                eo[i] = ex2f(-L2E * clampf(pre[i][3], 15.f));
-            }
-#pragma unroll
-            for (int i = 0; i < CELLS; i++) {
-                const float di = 1.f + ei[i], df = 1.f + ef[i], dg = 1.f + eg[i], dq = 1.f + eo[i];
-                const float p1 = di * df, p2 = dg * dq;
-                rr[i] = rcpf(p1 * p2);
-                // keep the partial products: sig(i) = r df p2, sig(f) = r di p2, sig(o) = r p1 dg, tanh(g) = (1-eg) r p1 dq
-                ei[i] = df * p2; ef[i] = di * p2; eo[i] = p1 * dg; eg[i] = (1.f - eg[i]) * (p1 * dq);
-            }
-#pragma unroll
-            for (int i = 0; i < CELLS; i++) {
-                const float r = rr[i];
-                const float cn = (r * ef[i]) * cst[i] + (r * ei[i]) * (r * eg[i]);
-                cst[i] = cn;
-                eo[i] = r * eo[i];                             // sig(o)
-                ei[i] = ex2f(-2.f * L2E * clampf(cn, 7.5f));
-            }
-#pragma unroll
-            for (int i = 0; i < CELLS; i++) rr[i] = rcpf(1.f + ei[i]);
-#pragma unroll
-            for (int i = 0; i < CELLS; i++) hout[i] = eo[i] * (1.f - ei[i]) * rr[i];
-#endif
-            if (ew == 0 && lane == 0) DBG(sub, 7);
-            // h slice of the warp (NS chunks x 8 units) through a 16 B-per-chunk staging row: one 16-byte global
+            // h slice of the warp (NS chunks x 8 units) through a private 16 B-per-chunk staging row: one 16-byte global
             // store per chunk instead of eight 2-byte ones
-            // GB == 2: private staging rows.  GB == 1: the rows alias the 16 bytes at the head of the 64-byte G segments this
-            // warp itself read above (chunk rows col0.., unit columns q*8..), so no other warp's data is touched.
-            constexpr int ST_PITCH = GB == 2 ? 8 : 128;          // 16-bit elements between consecutive chunks
-            uint16_t *st = GB == 2 ? reinterpret_cast<uint16_t *>(stage + ((sub * EW + ew) * C::STAGE_BYTES))
-                                   : const_cast<uint16_t *>(Gs) + col0 * 128 + q * 32;
-            if (GB == 1) __syncwarp();                           // every lane has taken its G values
+            constexpr int ST_PITCH = 8;                          // 16-bit elements between consecutive chunks
             // explicit shared-memory instructions: behind the casts the compiler falls back to generic loads / stores
-            const uint32_t st_s = smem_u32(st);
-            if (tma_store) {
-                const uint32_t tile_s = smem_u32(stage + sub * (NS * 64));       // [chunk][32 units] fp16, 64 B per chunk
-#pragma unroll
-                for (int i = 0; i < CELLS; i++) {
-                    typename X::T hv = X::from(hout[i]);
-                    sts_u16(tile_s + 2u * ((col0 + 8 * (i >> 1) + 2 * gt + (i & 1)) * 32 + q * 8 + ul), *reinterpret_cast<uint16_t *>(&hv));
-                }
-                fence_proxy_async();                             // my tile bytes -> visible to the async proxy
-                named_bar_sync(1 + sub, EW * 32);
-                if (ew == 0 && lane == 0) {
-                    tma_store_2d(&tmS, tile_s, j * 32, t * N + row0);
-                    bulk_commit_group();
-                    bulk_wait_group0();                          // the tile's writes are complete (acknowledged by L2)
-                    // Release, not relaxed: wait_group makes the async-proxy writes visible to THIS thread; the consumers'
-                    // acquire needs a release pattern to synchronise with.  The MEMBAR.GPU inside costs ~1 ms per batch
-                    // even with no generic store pending (XB_EXPERIMENTS, XB_TMAS=2 publishes relaxed: 12.5-13.1 ms
-                    // per batch instead of 14.1 -- physically the same, outside the memory model).
-#ifdef XB_EXPERIMENTS
-                    if (p.tma_store >= 2) red_relaxed_gpu_add(ctr, EW); else
-#endif
-                    red_release_gpu_add(ctr, EW);
-                    DBG(sub, 13);
-                }
-                if (lane == 0) mbar_arrive(g_empty(sub, s & 1));
-                continue;
-            }
+            const uint32_t st_s = smem_u32(stage + (sub * EW + ew) * STAGE_BYTES);
 #pragma unroll
             for (int i = 0; i < CELLS; i++) {
                 typename X::T hv = X::from(hout[i]);
@@ -454,29 +326,17 @@ lstm_persistent_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_con
             if (lane < NC && col0 + lane < cnt)
                 *reinterpret_cast<uint4 *>(p.y + ((size_t)t * N + row0 + col0 + lane) * XB_FEATURES + j * 32 + q * 8) =
                     lds_v4(st_s + 2u * (lane * ST_PITCH));
-            if (ew == 0 && lane == 0) DBG(sub, 12);
-            if (p.one_release) {
-                // one release per sub-batch and step instead of one per warp (MEMBAR.GPU instances of one SM appear to
-                // be served one at a time): the sub-batch's warps meet at a named barrier, one thread publishes
-                named_bar_sync(1 + sub, EW * 32);
-                if (ew == 0 && lane == 0) {
-                    red_release_gpu_add(ctr, EW);             // cumulative over the barrier: all the sub-batch's stores
-                    DBG(sub, 13);
-                }
-                if (lane == 0) mbar_arrive(g_empty(sub, GB == 2 ? (s & 1) : 0));
-            } else {
-                __syncwarp();
-                if (lane == 0) {
-                    red_release_gpu_add(ctr, 1);              // publishes the warp's stores (cumulative over __syncwarp)
-                    mbar_arrive(g_empty(sub, GB == 2 ? (s & 1) : 0));
-                    if (ew == 0) DBG(sub, 13);
-                }
-            }
-            // Training forward: i, f, g, o, c of the step through the same (private, GB == 2) staging rows -> (T, N, 5, 768) fp16.
+            // one release per sub-batch and step instead of one per warp (MEMBAR.GPU instances of one SM appear to
+            // be served one at a time; the per-warp release was measured and removed): the sub-batch's warps meet at a
+            // named barrier, one thread publishes
+            named_bar_sync(1 + sub, EW * 32);
+            if (ew == 0 && lane == 0)
+                red_release_gpu_add(ctr, EW);                 // cumulative over the barrier: all the sub-batch's stores
+            if (lane == 0) mbar_arrive(g_empty(sub, s & 1));
+            // Training forward: i, f, g, o, c of the step through the same private staging rows -> (T, N, 5, 768) fp16.
             // AFTER h has been published: these stores feed the backward pass, not the next step, and in front of the release
             // they sat on the step-to-step chain (five staging rounds, and the release's fence waits for every store before it).
             if (SAVE) {
-                static_assert(!SAVE || GB == 2, "the saved-state stores reuse the staging rows after the gate buffer has been released");
 #pragma unroll
                 for (int qn = 0; qn < 5; qn++) {
                     __syncwarp();
@@ -501,21 +361,19 @@ lstm_persistent_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_con
     }
 }
 
-template <bool BF16, int SUB, int NS, int EW, int GB = 2, bool SAVE = false>
-int launch_cfg(xb_handle *h, int layer, void *y_tnc, int T, int N, int reverse, cudaStream_t s, void *save = nullptr) {
-    using C = Cfg<SUB, NS, EW, GB>;
-    CUtensorMap tmY, tmG, tmS;
+template <bool SAVE>
+int launch(xb_handle *h, int layer, void *y_tnc, int T, int N, int reverse, cudaStream_t s, void *save) {
+    CUtensorMap tmY, tmG;
     if (int rc = xb_make_tmap_hview(h, &tmY, y_tnc, (uint64_t)T * N, NS, KPB)) return rc;
-    if (int rc = xb_make_tmap_2d_box(h, &tmS, y_tnc, (uint64_t)T * N, XB_FEATURES, XB_FEATURES, 32, NS, 0)) return rc;
     if (int rc = xb_make_tmap_2d_box(h, &tmG, h->gates, (uint64_t)T * N, XB_GATES, XB_GATES, 128, NS, 0)) return rc;
     const int max_groups = h->num_sms / TILES;                 // 6 on a 148-SM B200
     if (max_groups < 1)
         return xb_fail(h, XB_ERR_UNSUPPORTED, "the persistent LSTM needs %d co-resident CTAs, the device has %d SMs", TILES, h->num_sms);
-    const int block_cap = max_groups * C::NB;
-    auto fn = lstm_persistent_kernel<BF16, SUB, NS, EW, GB, SAVE>;
+    const int block_cap = max_groups * NB;
+    auto fn = lstm_persistent_kernel<SAVE>;
     static bool configured[64] = {};      // per device: function attributes live in the device's context
     if (!configured[h->device & 63]) {
-        XB_CUDA(h, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
+        XB_CUDA(h, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
         configured[h->device & 63] = true;
     }
     for (int batch0 = 0; batch0 < N; batch0 += block_cap) {
@@ -523,26 +381,14 @@ int launch_cfg(xb_handle *h, int layer, void *y_tnc, int T, int N, int reverse, 
         p.T = T; p.N = N; p.reverse = reverse;
         p.batch0 = batch0;
         p.nbatch = (N - batch0 < block_cap) ? N - batch0 : block_cap;
-        p.G = (p.nbatch + C::NB - 1) / C::NB;
+        p.G = (p.nbatch + NB - 1) / NB;
         p.w_hh = reinterpret_cast<const uint16_t *>(h->lstm[layer].w_hh);
         p.y = reinterpret_cast<uint16_t *>(y_tnc);
         p.counters = h->lstm_counters;
-        p.one_release = 1;
-        p.prefetch_y = 4;
-        p.dbg = nullptr;
         p.save = reinterpret_cast<uint16_t *>(save);
-        p.tma_store = 0;
-#ifdef XB_EXPERIMENTS
-        if (getenv("XB_TMAS")) p.tma_store = atoi(getenv("XB_TMAS"));
-#endif
-#ifdef XB_EXPERIMENTS
-        if (getenv("XB_LSTM_WARP_RELEASE")) p.one_release = 0;
-        if (getenv("XB_LSTM_PREFETCH_Y")) p.prefetch_y = atoi(getenv("XB_LSTM_PREFETCH_Y"));
-        if (getenv("XB_LSTM_DEBUG")) p.dbg = reinterpret_cast<long long *>(h->lstm_counters + MAX_CTRS * CTR_STRIDE);
-#endif
         XB_CUDA(h, cudaMemsetAsync(h->lstm_counters, 0, MAX_CTRS * CTR_STRIDE * sizeof(int), s));
-        void *args[] = {(void *)&tmY, (void *)&tmG, (void *)&tmS, (void *)&p};
-        XB_CUDA(h, cudaLaunchCooperativeKernel((const void *)fn, dim3(p.G * TILES), dim3(C::THREADS), args, C::SMEM_BYTES, s));
+        void *args[] = {(void *)&tmY, (void *)&tmG, (void *)&p};
+        XB_CUDA(h, cudaLaunchCooperativeKernel((const void *)fn, dim3(p.G * TILES), dim3(THREADS), args, SMEM_BYTES, s));
         h->launches++;
     }
     return XB_OK;
@@ -550,36 +396,15 @@ int launch_cfg(xb_handle *h, int layer, void *y_tnc, int T, int N, int reverse, 
 
 }  // namespace
 
-#ifdef XB_EXPERIMENTS
-// debug: copy the timeline of the last launch (8 steps x 16 stamps) to the host
-extern "C" int xb_debug_lstm_timeline(xb_handle *h, long long *out_host) {
-    if (!h || !h->lstm_counters) return XB_ERR_STATE;
-    XB_CUDA(h, cudaDeviceSynchronize());
-    XB_CUDA(h, cudaMemcpy(out_host, h->lstm_counters + MAX_CTRS * CTR_STRIDE, 8 * 8 * 16 * sizeof(long long), cudaMemcpyDeviceToHost));
-    return XB_OK;
-}
-#endif
-
 // Recurrent part of one LSTM layer.  h->gates must already hold the input projection (T*N, 3072) with the
 // columns of every 128-wide tile ordered [unit][i,f,g,o] (weight repack mode 3 in xb_api.cu).
 // save != nullptr: the training forward, which also stores (T, N, 5, 768) fp16 = i, f, g, o, c for the backward pass
 int xb_lstm_recurrence_persistent(xb_handle *h, int layer, void *y_tnc, int T, int N, int reverse, cudaStream_t s, void *save) {
     if (!h->lstm_counters) {
         void *q = nullptr;
-        XB_CUDA(h, cudaMalloc(&q, MAX_CTRS * CTR_STRIDE * sizeof(int) + 8 * 8 * 16 * sizeof(long long)));
+        XB_CUDA(h, cudaMalloc(&q, MAX_CTRS * CTR_STRIDE * sizeof(int)));
         h->lstm_counters = reinterpret_cast<int *>(q);
     }
-#ifdef XB_EXPERIMENTS
-    static const int variant = getenv("XB_LSTM_VARIANT") ? atoi(getenv("XB_LSTM_VARIANT")) : 0;
-    if (variant == 1)
-        return launch_cfg<false, 3, 32, 4>(h, layer, y_tnc, T, N, reverse, s);
-    if (variant == 4)      // four chains of 32 chunks on 24 x 4 = 96 CTAs at N = 512 (feasibility of the overlap plan, DESIGN 7)
-        return launch_cfg<false, 4, 32, 4, 1>(h, layer, y_tnc, T, N, reverse, s);
-    if (variant == 3)
-        return launch_cfg<false, 2, 48, 12>(h, layer, y_tnc, T, N, reverse, s);
-    if (variant == 2)
-        return launch_cfg<false, 6, 16, 4>(h, layer, y_tnc, T, N, reverse, s);
-#endif
-    if (save) return launch_cfg<false, 3, 32, 8, 2, true>(h, layer, y_tnc, T, N, reverse, s, save);
-    return launch_cfg<false, 3, 32, 8>(h, layer, y_tnc, T, N, reverse, s);
+    if (save) return launch<true>(h, layer, y_tnc, T, N, reverse, s, save);
+    return launch<false>(h, layer, y_tnc, T, N, reverse, s, nullptr);
 }

@@ -63,7 +63,6 @@ int dev_alloc_bytes(xb_handle *h, void **p, size_t bytes) { return dev_alloc<uin
 
 // ---- weight repacking ------------------------------------------------------------------------------
 // dst (rows_dst, cols_dst) 16-bit <- src fp32; mode 0: plain rows (zero padding past rows_src / cols_src);
-// mode 1: LSTM gate interleave, dst row j*128 + g*32 + u <- src row g*768 + j*32 + u;
 // mode 2: conv3 (768,16,19) -> (768, 320) with column tap*16 + ch;
 // mode 3: LSTM unit-major interleave, dst row j*128 + u*4 + g <- src row g*768 + j*32 + u (the input projection
 //         of the persistent kernel: the four gates of a unit are adjacent in a row of G);
@@ -78,9 +77,6 @@ __global__ void repack_kernel(const float *__restrict__ src, uint16_t *__restric
     float v = 0.0f;
     if (mode == 0) {
         if (r < rows_src && c < cols_src) v = src[(size_t)r * cols_src + c];
-    } else if (mode == 1) {
-        int j = r >> 7, g = (r >> 5) & 3, u = r & 31;
-        v = src[(size_t)(g * XB_FEATURES + j * 32 + u) * cols_src + c];
     } else if (mode == 3) {
         int j = r >> 7, u = (r >> 2) & 31, g = r & 3;
         v = src[(size_t)(g * XB_FEATURES + j * 32 + u) * cols_src + c];
@@ -109,12 +105,11 @@ __global__ void repack_kernel(const float *__restrict__ src, uint16_t *__restric
     __half hv = __float2half_rn(v);
     dst[i] = *reinterpret_cast<uint16_t *>(&hv);
 }
-__global__ void lstm_bias_kernel(const float *__restrict__ b_ih, const float *__restrict__ b_hh, float *__restrict__ dst,
-                                 int mode) {
+// b_ih + b_hh in the row order of repack mode 3
+__global__ void lstm_bias_kernel(const float *__restrict__ b_ih, const float *__restrict__ b_hh, float *__restrict__ dst) {
     int r = blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= XB_GATES) return;
-    int j = r >> 7, g = (r >> 5) & 3, u = r & 31;
-    if (mode == 3) { u = (r >> 2) & 31; g = r & 3; }
+    int j = r >> 7, u = (r >> 2) & 31, g = r & 3;
     int s = g * XB_FEATURES + j * 32 + u;
     dst[r] = b_ih[s] + b_hh[s];
 }
@@ -220,7 +215,6 @@ int xb_create(xb_handle **out, int device, int max_N, int max_T, int n_base, int
         TRY(dev_alloc_bytes(h, &h->act0, TN * XB_FEATURES * 2));
         TRY(dev_alloc_bytes(h, &h->act1, TN * XB_FEATURES * 2));
         TRY(dev_alloc_bytes(h, &h->gates, TN * XB_GATES * 2));
-        TRY(dev_alloc(h, &h->cstate, (size_t)max_N * XB_FEATURES));
         TRY(dev_alloc(h, &h->scores, TN * S));
         TRY(dev_alloc_bytes(h, &h->signal_dev, TN * XB_STRIDE * sizeof(float)));
     }
@@ -238,7 +232,7 @@ int xb_destroy(xb_handle *h) {
     if (!h) return XB_OK;
     cudaSetDevice(h->device);
     void *ptrs[] = {h->conv1_w, h->conv1_b, h->conv2_w, h->conv2_b, h->conv3_w, h->conv3_b, h->head_w, h->head_b, h->c2,
-                    h->act0, h->act1, h->gates, h->cstate, h->hzero, h->scores, h->signal_dev, h->seq_dev, h->lens_dev,
+                    h->act0, h->act1, h->gates, h->scores, h->signal_dev, h->seq_dev, h->lens_dev,
                     h->alpha, h->bmax, h->lp, h->logz, h->ctc_ws, h->lstm_counters};
     for (void *p : ptrs)
         if (p) cudaFree(p);
@@ -318,14 +312,8 @@ int xb_load_lstm_weights(xb_handle *h, int layer, const float *w_ih, const float
     XB_REQUIRE(h, layer >= 0 && layer < 5, "LSTM layer %d out of range", layer);
     XB_REQUIRE(h, w_ih && w_hh && b_ih && b_hh, "NULL LSTM weight");
     const int F = XB_FEATURES;
-#ifdef XB_EXPERIMENTS
-#define XB_FLAG_LSTM_STEPWISE 4
-    const int ih_mode = (h->flags & XB_FLAG_LSTM_STEPWISE) ? 1 : 3;
-#else
-    const int ih_mode = 3;
-#endif
-    if (int rc = repack(h, w_ih, h->lstm[layer].w_ih, XB_GATES, F, XB_GATES, F, ih_mode, s)) return rc;
-    if (int rc = repack(h, w_hh, h->lstm[layer].w_hh, XB_GATES, F, XB_GATES, F, ih_mode == 3 ? 4 : 1, s)) return rc;
+    if (int rc = repack(h, w_ih, h->lstm[layer].w_ih, XB_GATES, F, XB_GATES, F, 3, s)) return rc;
+    if (int rc = repack(h, w_hh, h->lstm[layer].w_hh, XB_GATES, F, XB_GATES, F, 4, s)) return rc;
     if (h->flags & XB_FLAG_TRAIN) {
         xb_lstm_weights &lw = h->lstm[layer];
         if (!lw.w_ihT) { if (int rc = dev_alloc_bytes(h, &lw.w_ihT, (size_t)XB_GATES * F * 2)) return rc; }
@@ -333,7 +321,7 @@ int xb_load_lstm_weights(xb_handle *h, int layer, const float *w_ih, const float
         if (int rc = repack(h, w_ih, lw.w_ihT, F, XB_GATES, XB_GATES, F, 5, s)) return rc;
         if (int rc = repack(h, w_hh, lw.w_hhT, F, XB_GATES, XB_GATES, F, 5, s)) return rc;
     }
-    lstm_bias_kernel<<<(XB_GATES + 255) / 256, 256, 0, s>>>(b_ih, b_hh, h->lstm[layer].bias, ih_mode);
+    lstm_bias_kernel<<<(XB_GATES + 255) / 256, 256, 0, s>>>(b_ih, b_hh, h->lstm[layer].bias);
     XB_LAUNCH_CHECK(h);
     h->loaded |= 2 << layer;
     return XB_OK;
@@ -409,41 +397,10 @@ int xb_lstm_fwd(xb_handle *h, int layer, const void *x_tnc, void *y_tnc, int T, 
     // (a) input projection for all time steps: gates (T*N, 3072) = x W_ih^T + (b_ih + b_hh)
     {
         xb_stage_timer tm(h, XB_ST_INPROJ, s);
-#ifdef XB_EXPERIMENTS
-        static const bool generic = getenv("XB_INPROJ_GENERIC") != nullptr;    // A/B switch: the generic tile kernel
-        if (generic) {
-            CUtensorMap tmA, tmB;
-            if (int rc = xb_make_tmap_2d(h, &tmA, x_tnc, (uint64_t)T * N, XB_FEATURES, XB_FEATURES)) return rc;
-            if (int rc = xb_make_tmap_2d(h, &tmB, lw.w_ih, XB_GATES, XB_FEATURES, XB_FEATURES)) return rc;
-            GemmParams p;
-            p.M = T * N; p.N = XB_GATES; p.K = XB_FEATURES;
-            p.bias = lw.bias; p.out = h->gates; p.ldo = XB_GATES;
-            if (int rc = xb_gemm_launch(h, EPI_INPROJ, tmA, tmB, p, s)) return rc;
-        } else
-#endif
         if (int rc = xb_inproj_launch(h, x_tnc, lw.w_ih, lw.bias, h->gates, T * N, s)) return rc;
     }
     // (b) recurrence: one persistent launch per layer; direction by indexing
     xb_stage_timer tm(h, XB_ST_LSTM_REC, s);
-#ifdef XB_EXPERIMENTS
-    if (h->flags & XB_FLAG_LSTM_STEPWISE) {      // one fused GEMM + cell kernel per time step (independent cross-check)
-        CUtensorMap tmH, tmW;
-        if (int rc = xb_make_tmap_2d(h, &tmH, y_tnc, (uint64_t)T * N, XB_FEATURES, XB_FEATURES)) return rc;
-        if (int rc = xb_make_tmap_2d(h, &tmW, lw.w_hh, XB_GATES, XB_FEATURES, XB_FEATURES)) return rc;
-        for (int i = 0; i < T; i++) {
-            const int t = reverse ? T - 1 - i : i;
-            const int tp = reverse ? t + 1 : t - 1;
-            GemmParams p;
-            p.M = N; p.N = XB_GATES; p.K = XB_FEATURES;
-            p.a_row_offset = (i == 0) ? 0 : tp * N;
-            p.out = y_tnc; p.NB = N;
-            p.gates = h->gates; p.cstate = h->cstate;
-            p.t_cur = t; p.first = (i == 0);
-            if (int rc = xb_gemm_launch(h, EPI_LSTM, tmH, tmW, p, s)) return rc;
-        }
-        return XB_OK;
-    }
-#endif
     return xb_lstm_recurrence_persistent(h, layer, y_tnc, T, N, reverse, s);
 }
 
@@ -467,21 +424,6 @@ static int head_fwd(xb_handle *h, const void *x_tnc, float *scores, int T, int N
     if (int rc = check_tn(h, T, N)) return rc;
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     xb_stage_timer tm(h, XB_ST_HEAD, s);
-#ifdef XB_EXPERIMENTS
-    static const bool tile_gemm = getenv("XB_HEAD_GENERIC") != nullptr;      // the 128x128 tile GEMM, kept for cross-checks
-    if (tile_gemm) {
-        CUtensorMap tmA, tmB;
-        if (int rc = xb_make_tmap_2d(h, &tmA, x_tnc, (uint64_t)T * N, XB_FEATURES, XB_FEATURES)) return rc;
-        if (int rc = xb_make_tmap_2d(h, &tmB, h->head_w, h->head_rows_padded, XB_FEATURES, XB_FEATURES)) return rc;
-        GemmParams p;
-        p.M = T * N; p.N = h->head_rows_padded; p.K = XB_FEATURES;
-        p.bias = h->head_b; p.out = scores;
-        p.ldo = h->expand_blanks ? h->C * h->NZ : h->head_rows;
-        p.n_base = h->n_base; p.head_rows = h->head_rows; p.expand = h->expand_blanks;
-        p.scale = h->scale; p.blank = h->blank_score;
-        return xb_gemm_launch(h, EPI_HEAD, tmA, tmB, p, s);
-    }
-#endif
     return xb_head_astationary_launch(h, x_tnc, h->head_w, h->head_rows_padded, h->head_b, h->head_rows, scores,
                                       h->expand_blanks ? h->C * h->NZ : h->head_rows, T * N, exp_out, s);
 }

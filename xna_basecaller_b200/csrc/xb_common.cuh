@@ -64,8 +64,6 @@ struct xb_handle {
     void *c2 = nullptr;          // (max_N, L + 2*halo (+pad), 16) 16-bit channel-last conv2 output
     void *act0 = nullptr, *act1 = nullptr;   // (max_T, max_N, 768) 16-bit ping-pong
     void *gates = nullptr;       // (max_T, max_N, 3072) 16-bit hoisted input projection
-    float *cstate = nullptr;     // (max_N, 768) fp32 LSTM cell state
-    void *hzero = nullptr;       // (max_N, 768) 16-bit zeros (initial hidden state)
     float *scores = nullptr;     // (max_T, max_N, C*NZ) fp32 (used by the host entry points)
     void *signal_dev = nullptr;  // (max_N, max_T*5) fp32 staging for the host entry points
     int8_t *seq_dev = nullptr;   // (max_N, max_T)

@@ -2,23 +2,15 @@
 #pragma once
 #include "xb_common.cuh"
 
-enum { EPI_F32 = 0, EPI_CONV3 = 1, EPI_INPROJ = 2, EPI_HEAD = 3, EPI_LSTM = 4, EPI_BF16OUT = 5, EPI_CONV3_BWD = 7 };
+enum { EPI_F32 = 0, EPI_BF16OUT = 5, EPI_CONV3_BWD = 7 };
 
 struct GemmParams {
     int M = 0, N = 0, K = 0;       // logical problem (rows of A that are valid, columns = rows of B, depth)
-    int a_row_offset = 0;          // added to the A row coordinate (LSTM: row block of h_{t-1})
     int split_k = 1;               // EPI_F32: K slices (gridDim.z) whose partial tiles are ADDED to a zeroed output
     const float *bias = nullptr;   // (N) fp32
     void *out = nullptr;
     int ldo = 0;                   // output row pitch in elements
-    int T = 0, NB = 0;             // conv3: rows are (chunk, t) -> stored at (t, chunk); LSTM: NB = batch
-    // head
-    int n_base = 0, head_rows = 0, expand = 0;
-    float scale = 0.f, blank = 0.f;
-    // lstm step
-    const void *gates = nullptr;   // (T, NB, 3072) 16-bit input projection (+bias)
-    float *cstate = nullptr;       // (NB, 768) fp32
-    int t_cur = 0, first = 0;
+    int T = 0, NB = 0;             // EPI_CONV3_BWD: rows are (chunk, t), dy is stored at (t, chunk)
     // training backward (EPI_CONV3_BWD: recomputed conv3 pre-activation -> its gradient)
     const void *dy = nullptr;      // (T, NB, 768) bf16: gradient w.r.t. the stem output
 };
