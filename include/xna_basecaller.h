@@ -192,6 +192,17 @@ int xb_encoder_fwd_train(xb_handle *h, const void *signal, int sig_dtype, int N,
 int xb_encoder_bwd(xb_handle *h, const void *signal, int sig_dtype, const float *scores, const float *dscores,
                    float *const *grads, int n_tensors, void *stream);
 
+/* Stages top .. bottom (top >= bottom) of the backward of the last xb_encoder_fwd_train: 6 = CRF head, 5 .. 1 = LSTM
+ * layers 4 .. 0, 0 = convolution stem.  top == 6 starts from dscores; otherwise dy_top (T,N,768) bf16 is the gradient
+ * w.r.t. the OUTPUT of stage top.  bottom >= 1 writes the gradient w.r.t. the INPUT of stage bottom to dy_bottom
+ * (T,N,768) bf16.  Only the gradient tensors of the stages run are written; the others may be NULL.  dy_top / dy_bottom
+ * must be 16-byte aligned; a range the arguments do not cover is XB_ERR_ARG.  After a forward with dropout only the whole
+ * range (6, 0) runs (else XB_ERR_UNSUPPORTED).
+ * xb_encoder_bwd(...) == xb_encoder_bwd_stages(h, 6, 0, ..., NULL, NULL, ...). */
+int xb_encoder_bwd_stages(xb_handle *h, int top, int bottom, const void *signal, int sig_dtype, const float *scores,
+                          const float *dscores, const void *dy_top, void *dy_bottom, float *const *grads, int n_tensors,
+                          void *stream);
+
 /* Dropout in the training step (rnn_encoder(drop_rate_bottom=...), crf/model.py): the forward of xb_encoder_fwd_train with
  * torch.nn.Dropout(p[s]) applied at XB_DROPOUT_SITES sites, in the order the reference applies them:
  *   0 conv1 output, 1 conv2 output, 2 conv3 output, 3..6 outputs of LSTM layers 0..3.

@@ -28,7 +28,7 @@ SYMBOLS = (
     'xb_set_profiling', 'xb_stage_times', 'xb_crf_head_fwd_exp', 'xb_crf_decode_exp', 'xb_basecall_chunks',
     'xb_crf_logz_s', 'xb_crf_forward_scores_s', 'xb_crf_backward_scores_s', 'xb_crf_posteriors_max',
     'xb_encoder_fwd_train', 'xb_encoder_bwd', 'xb_adamw_step', 'xb_crf_beam_search',
-    'xb_align_counts', 'xb_encoder_fwd_train_dropout', 'xb_dropout_keep',
+    'xb_align_counts', 'xb_encoder_fwd_train_dropout', 'xb_dropout_keep', 'xb_encoder_bwd_stages',
 )
 STAGES = ('conv12_im2col', 'conv3_gemm', 'lstm_inproj_gemm', 'lstm_recurrence', 'crf_head_gemm', 'crf_alpha',
           'crf_backward', 'crf_viterbi', 'train_bptt', 'train_transpose', 'train_weight_grad_gemm', 'train_input_grad_gemm', 'train_head_conv_bwd')
@@ -67,6 +67,7 @@ def load():
     lib.xb_crf_posteriors.argtypes = [vp, vp, ci, ci, vp, vp]
     lib.xb_encoder_fwd_train.argtypes = [vp, vp, ci, ci, ci, vp, vp]
     lib.xb_encoder_bwd.argtypes = [vp, vp, ci, vp, vp, ctypes.POINTER(vp), ci, vp]
+    lib.xb_encoder_bwd_stages.argtypes = [vp, ci, ci, vp, ci, vp, vp, vp, vp, ctypes.POINTER(vp), ci, vp]
     lib.xb_encoder_fwd_train_dropout.argtypes = [vp, vp, ci, ci, ci, ctypes.POINTER(cf), ctypes.c_uint64, vp, vp]
     lib.xb_dropout_keep.argtypes = [ctypes.c_uint64, ci, cf, ctypes.c_int64, vp, vp]
     lib.xb_adamw_step.argtypes = [ctypes.POINTER(vp), ctypes.POINTER(vp), ctypes.POINTER(vp), ctypes.POINTER(vp),
@@ -359,21 +360,50 @@ class Handle:
         self._train_keep = (signal, code, scores)
         return scores
 
-    def encoder_backward(self, dscores):
-        """dscores (T, N, C*NZ) fp32 -> {reference state_dict key: fp32 gradient in the reference's layout}."""
-        signal, code, scores = self._train_keep
-        ds = dscores.to(self.device, torch.float32).contiguous()
+    def _grad_buffers(self, stages=range(7)):
+        """Zeroed fp32 gradient tensors of the XB_NUM_WEIGHTS parameters (None for those outside `stages`)."""
         head_rows = self.C * self.n_base
         shapes = [(4, 1, 5), (4,), (16, 4, 5), (16,), (768, 320), (768,)]
         for _ in range(5):
             shapes += [(3072, 768), (3072, 768), (3072,), (3072,)]
         shapes += [(head_rows, 768), (head_rows,)]
-        grads = [torch.zeros(*s, dtype=torch.float32, device=self.device) for s in shapes]
+        stage_of = [0] * 6 + [1 + i // 4 for i in range(20)] + [6, 6]
+        return [torch.zeros(*s, dtype=torch.float32, device=self.device) if stage_of[i] in stages else None
+                for i, s in enumerate(shapes)]
+
+    def _grad_dict(self, grads):
+        if grads[4] is not None:
+            grads[4] = grads[4][:, :304].reshape(768, 19, 16).permute(0, 2, 1).contiguous()  # [out][tap][in] -> (768, 16, 19)
+        return {k: g for k, g in zip(self.WEIGHT_KEYS, grads) if g is not None}
+
+    def encoder_backward(self, dscores):
+        """dscores (T, N, C*NZ) fp32 -> {reference state_dict key: fp32 gradient in the reference's layout}."""
+        signal, code, scores = self._train_keep
+        ds = dscores.to(self.device, torch.float32).contiguous()
+        grads = self._grad_buffers()
         arr = (ctypes.c_void_p * NUM_WEIGHTS)(*[g.data_ptr() for g in grads])
         self._check(self.lib.xb_encoder_bwd(self.h, _ptr(signal), code, _ptr(scores), _ptr(ds), arr, NUM_WEIGHTS,
                                             _stream(self.device)), 'xb_encoder_bwd')
-        grads[4] = grads[4][:, :304].reshape(768, 19, 16).permute(0, 2, 1).contiguous()      # [out][tap][in] -> (768, 16, 19)
-        return dict(zip(self.WEIGHT_KEYS, grads))
+        return self._grad_dict(grads)
+
+    def encoder_backward_stages(self, top, bottom, dscores=None, dy_top=None):
+        """xb_encoder_bwd_stages: stages top .. bottom of encoder_backward (6 CRF head, 5 .. 1 LSTM layers 4 .. 0, 0 stem).
+        top == 6 starts from dscores (T, N, C*NZ) fp32, otherwise from dy_top (T, N, 768) bf16, the gradient w.r.t. the
+        output of stage top.  Returns ({key: gradient} of the stages run, dy_bottom): dy_bottom (T, N, 768) bf16 is the
+        gradient w.r.t. the input of stage bottom, None for bottom == 0."""
+        signal, code, scores = self._train_keep
+        T, N = scores.shape[:2]
+        ds = dscores.to(self.device, torch.float32).contiguous() if dscores is not None else None
+        dy = dy_top.to(self.device).contiguous() if dy_top is not None else None
+        if dy is not None and (dy.dtype != torch.bfloat16 or tuple(dy.shape) != (T, N, 768)):
+            raise ValueError('dy_top must be (%d, %d, 768) bfloat16' % (T, N))
+        out = torch.empty(T, N, 768, dtype=torch.bfloat16, device=self.device) if bottom >= 1 else None
+        grads = self._grad_buffers(range(bottom, top + 1))
+        arr = (ctypes.c_void_p * NUM_WEIGHTS)(*[None if g is None else g.data_ptr() for g in grads])
+        self._check(self.lib.xb_encoder_bwd_stages(self.h, int(top), int(bottom), _ptr(signal), code, _ptr(scores), _ptr(ds),
+                                                   _ptr(dy), _ptr(out), arr, NUM_WEIGHTS, _stream(self.device)),
+                    'xb_encoder_bwd_stages')
+        return self._grad_dict(grads), out
 
     # ------------------------------------------------------------------ CRF
     def _scores(self, scores):

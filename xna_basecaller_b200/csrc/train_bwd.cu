@@ -521,6 +521,121 @@ static int encoder_fwd_train(xb_handle *h, const void *signal, int sig_dtype, in
     return xb_crf_head_fwd(h, w->x[5], scores, T, N, stream);
 }
 
+// ---- the three stages of xb_encoder_bwd.  Each reads the gradient w.r.t. its output and writes the gradient w.r.t. its
+// input (the stem: only parameter gradients); the workspace buffers they share are described in xb_train_ws.
+
+// CRF head: dscores -> grads[26], grads[27] and dy_out = d x5 (T,N,768) bf16.  Leaves x5 transposed in XT[1] for layer 4.
+static int head_bwd(xb_handle *h, xb_train_ws *w, const float *scores, const float *dscores, float *const *grads, void *dy_out,
+                    cudaStream_t s) {
+    const int TN = w->T * w->N, F = XB_FEATURES, HP = h->head_rows_padded, S = h->C * h->NZ;
+    const size_t n = (size_t)TN * HP;
+    head_bwd_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(dscores, scores, (size_t)TN, h->n_base, h->NZ, h->head_rows, HP,
+                                                              h->expand_blanks ? S : h->head_rows, h->expand_blanks,
+                                                              h->scale, reinterpret_cast<__nv_bfloat16 *>(w->dzh));
+    XB_LAUNCH_CHECK(h);
+    if (int rc = colsum(h, w->dzh, TN, h->head_rows, HP, grads[27], s)) return rc;
+    if (int rc = transpose_to_bf16(h, w->dzh, TN, HP, HP, true, w->dzhT, s)) return rc;
+    if (int rc = transpose_to_bf16(h, w->x[5], TN, F, F, false, w->XT[1], s)) return rc;
+    if (int rc = gemm_bf16(h, EPI_F32, w->dzhT, h->head_rows, TN, w->XT[1], F, TN, TN, grads[26], F, s)) return rc;
+    return gemm_bf16(h, EPI_BF16OUT, w->dzh, TN, HP, h->head_wT, F, HP, HP, dy_out, F, s);
+}
+
+// LSTM layer l: dy_in = d (output of layer l) -> grads[6 + 4l .. 9 + 4l] and dy_out = d (input of layer l), both (T,N,768)
+// bf16.  XT[(l+1) & 1] must hold the transposed output of layer l; leaves the transposed input in XT[l & 1].
+static int lstm_layer_bwd(xb_handle *h, xb_train_ws *w, int l, const void *dy_in, void *dy_out, float *const *grads,
+                          cudaStream_t s) {
+    const int N = w->N, T = w->T, TN = T * N, F = XB_FEATURES;
+    const xb_dropout &drop = w->drop;
+    const xb_lstm_weights &lw = h->lstm[l];
+    const bool reverse = (l % 2) == 0;
+    BpttMaps maps;
+    if (int rc = xb_bptt_make_maps(h, &maps, w->DZ, lw.w_hhT, w->saved[l], T, N)) return rc;
+    {
+    xb_stage_timer tm_bptt(h, XB_ST_TRAIN_BPTT, s);
+    for (int i = 0; i < T; i++) {                       // forward ran t = (reverse ? T-1 .. 0 : 0 .. T-1); walk it backwards
+        const int t = reverse ? i : T - 1 - i;
+        const int t_next = reverse ? t - 1 : t + 1;     // the step the forward ran AFTER t (its dz feeds dh_t); i == 0: none
+        const int t_prev = reverse ? t + 1 : t - 1;     // the step the forward ran BEFORE t (its c is c_prev)
+        BpttStep p;
+        p.N = N; p.t_cur = t;
+        p.t_next = (i == 0) ? -1 : t_next;
+        p.t_prev = (t_prev >= 0 && t_prev < T) ? t_prev : -1;
+        p.dy = dy_in; p.dcstate = w->dcstate;
+        if (int rc = xb_bptt_step_launch(h, maps, p, /*dependent=*/i > 0, s)) return rc;
+    }
+    }
+    float *g_wih = grads[6 + 4 * l], *g_whh = grads[7 + 4 * l], *g_bih = grads[8 + 4 * l], *g_bhh = grads[9 + 4 * l];
+    if (int rc = transpose_to_bf16(h, w->DZ, TN, XB_GATES, XB_GATES, true, w->DZT, s, g_bih)) return rc;   // + db = colsum DZ
+    XB_CUDA(h, cudaMemcpyAsync(g_bhh, g_bih, XB_GATES * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    if (int rc = transpose_to_bf16(h, w->x[l], TN, F, F, false, w->XT[l & 1], s)) return rc;
+    // layer l > 0 read the dropped copy of x[l] (site l + 2): dW_ih takes that, transposed through the mask into xd
+    const bool drop_in = l > 0 && drop.on(l + 2);
+    if (drop_in) { if (int rc = transpose_to_bf16(h, w->x[l], TN, F, F, false, w->xd, s, nullptr, &drop, l + 2)) return rc; }
+    // dW_ih = DZ^T x_l and dW_hh = sum over the steps that had a predecessor of dz_t (x) h_prev (a time shift of N columns
+    // between DZ^T and Y^T), one launch over 128 x 256 tiles (wgrad_gemm.cu)
+    {
+        xb_stage_timer tm(h, XB_ST_TRAIN_WGRAD, s);
+        if (int rc = xb_lstm_wgrad_launch(h, w->DZT, drop_in ? w->xd : w->XT[l & 1], w->XT[(l + 1) & 1], T, N, reverse, g_wih,
+                                          g_whh, s)) return rc;
+    }
+    if (int rc = gemm_bf16(h, EPI_BF16OUT, w->DZ, TN, XB_GATES, lw.w_ihT, F, XB_GATES, XB_GATES, dy_out, F, s)) return rc;
+    // gradient w.r.t. the dropped input -> w.r.t. the output of the layer below (l == 0: the conv3 output, site 2)
+    if (drop.on(l + 2)) { if (int rc = dropout16(h, dy_out, dy_out, (size_t)TN * F, true, drop, l + 2, s)) return rc; }
+    return XB_OK;
+}
+
+// convolution stem: dy_in = d x0 (T,N,768) bf16 -> grads[0 .. 5]
+static int stem_bwd(xb_handle *h, xb_train_ws *w, const void *signal, int sig_dtype, const void *dy_in, float *const *grads,
+                    cudaStream_t s) {
+    const int N = w->N, T = w->T, TN = T * N, F = XB_FEATURES, L = T * XB_STRIDE;
+    const xb_dropout &drop = w->drop;
+    const bool drop_stem = drop.on(0) || drop.on(1);
+    if (int rc = xb_conv12_im2col(h, signal, sig_dtype, N, L, s, &drop)) return rc;   // im2col rows of this batch into h->c2
+    CUtensorMap tmA, tmB;
+    if (int rc = xb_make_tmap_2d(h, &tmA, h->c2, (uint64_t)TN, XB_CONV3_K, XB_CONV3_K)) return rc;
+    if (int rc = xb_make_tmap_2d(h, &tmB, h->conv3_w, F, XB_CONV3_K, XB_CONV3_K)) return rc;
+    GemmParams p;
+    p.M = TN; p.N = F; p.K = XB_CONV3_K; p.bias = h->conv3_b; p.out = w->dpre; p.ldo = F; p.T = T; p.NB = N; p.dy = dy_in;
+    if (int rc = xb_gemm_launch(h, EPI_CONV3_BWD, tmA, tmB, p, s, false)) return rc;
+    if (int rc = transpose_to_bf16(h, w->dpre, TN, F, F, true, w->dpreT, s, grads[5])) return rc;       // + db3 = colsum d pre
+    if (int rc = transpose_to_bf16(h, h->c2, TN, XB_CONV3_K, XB_CONV3_K, false, w->colT, s)) return rc;
+    // dW3 in im2col column order (768, 320): the caller drops the 16 padding columns and permutes to (768, 16, 19)
+    if (int rc = gemm_bf16(h, EPI_F32, w->dpreT, F, TN, w->colT, XB_CONV3_K, TN, TN, grads[4], XB_CONV3_K, s)) return rc;
+    if (int rc = gemm_bf16(h, EPI_BF16OUT, w->dpre, TN, F, h->conv3_wT, XB_CONV3_K, F, F, w->dcol, XB_CONV3_K, s)) return rc;
+    const size_t n2 = (size_t)N * L * XB_C2_CH;
+    col2im_kernel<<<(unsigned)((n2 + 255) / 256), 256, 0, s>>>(reinterpret_cast<const __nv_bfloat16 *>(w->dcol), N, T, L, w->dc2);
+    XB_LAUNCH_CHECK(h);
+    XB_CUDA(h, cudaMemsetAsync(w->dc1, 0, (size_t)N * L * 4 * sizeof(float), s));
+    XB_CUDA(h, cudaMemsetAsync(grads[2], 0, 320 * sizeof(float), s));
+    XB_CUDA(h, cudaMemsetAsync(grads[3], 0, 16 * sizeof(float), s));
+    XB_CUDA(h, cudaMemsetAsync(grads[0], 0, 20 * sizeof(float), s));
+    XB_CUDA(h, cudaMemsetAsync(grads[1], 0, 4 * sizeof(float), s));
+    dim3 g2((L + 255) / 256, N);
+    if (sig_dtype == XB_SIG_F32) {
+        if (drop_stem)
+            conv2_bwd_kernel<true, float><<<g2, 256, 0, s>>>(reinterpret_cast<const float *>(signal), L, h->conv1_w, h->conv1_b,
+                                                             h->conv2_w, h->conv2_b, w->dc2, w->dc1, grads[2], grads[3], drop);
+        else
+            conv2_bwd_kernel<false, float><<<g2, 256, 0, s>>>(reinterpret_cast<const float *>(signal), L, h->conv1_w, h->conv1_b,
+                                                              h->conv2_w, h->conv2_b, w->dc2, w->dc1, grads[2], grads[3], drop);
+        XB_LAUNCH_CHECK(h);
+        conv1_bwd_kernel<float><<<dim3(4, N), 256, 0, s>>>(reinterpret_cast<const float *>(signal), L, h->conv1_w, h->conv1_b, w->dc1,
+                                                          grads[0], grads[1]);
+    } else {
+        if (drop_stem)
+            conv2_bwd_kernel<true, int16_t><<<g2, 256, 0, s>>>(reinterpret_cast<const int16_t *>(signal), L, h->conv1_w, h->conv1_b,
+                                                               h->conv2_w, h->conv2_b, w->dc2, w->dc1, grads[2], grads[3], drop);
+        else
+            conv2_bwd_kernel<false, int16_t><<<g2, 256, 0, s>>>(reinterpret_cast<const int16_t *>(signal), L, h->conv1_w, h->conv1_b,
+                                                                h->conv2_w, h->conv2_b, w->dc2, w->dc1, grads[2], grads[3], drop);
+        XB_LAUNCH_CHECK(h);
+        conv1_bwd_kernel<int16_t><<<dim3(4, N), 256, 0, s>>>(reinterpret_cast<const int16_t *>(signal), L, h->conv1_w, h->conv1_b,
+                                                            w->dc1, grads[0], grads[1]);
+    }
+    XB_LAUNCH_CHECK(h);
+    return XB_OK;
+}
+
 extern "C" {
 
 int xb_encoder_fwd_train(xb_handle *h, const void *signal, int sig_dtype, int N, int L, float *scores, void *stream) {
@@ -555,116 +670,52 @@ int xb_dropout_keep(uint64_t seed, int site, float p, int64_t n, uint8_t *keep, 
 // columns are padding; the caller reshapes to (768, 16, 19)).
 int xb_encoder_bwd(xb_handle *h, const void *signal, int sig_dtype, const float *scores, const float *dscores, float *const *grads,
                    int n_tensors, void *stream) {
+    return xb_encoder_bwd_stages(h, 6, 0, signal, sig_dtype, scores, dscores, nullptr, nullptr, grads, n_tensors, stream);
+}
+
+// Stages top .. bottom of the same backward (6 head, 5 .. 1 LSTM layers 4 .. 0, 0 stem); include/xna_basecaller.h.
+int xb_encoder_bwd_stages(xb_handle *h, int top, int bottom, const void *signal, int sig_dtype, const float *scores,
+                          const float *dscores, const void *dy_top, void *dy_bottom, float *const *grads, int n_tensors,
+                          void *stream) {
     if (!h) return xb_fail(nullptr, XB_ERR_ARG, "NULL handle");
     XB_REQUIRE(h, h->train && h->train->T > 0, "xb_encoder_bwd needs a preceding xb_encoder_fwd_train");
-    XB_REQUIRE(h, signal && scores && dscores && grads && n_tensors == XB_NUM_WEIGHTS, "bad arguments");
-    for (int i = 0; i < n_tensors; i++) XB_REQUIRE(h, grads[i] != nullptr, "gradient tensor %d is NULL", i);
-    XB_REQUIRE(h, sig_dtype == XB_SIG_F32 || sig_dtype == XB_SIG_I16, "the backward reads fp32 or int16 signal");
+    XB_REQUIRE(h, 0 <= bottom && bottom <= top && top <= 6, "bad stage range %d .. %d (need 6 >= top >= bottom >= 0)", top, bottom);
+    XB_REQUIRE(h, grads && n_tensors == XB_NUM_WEIGHTS, "bad arguments");
+    XB_REQUIRE(h, top < 6 || (scores && dscores), "the head stage needs scores and dscores");
+    XB_REQUIRE(h, top == 6 || (dy_top && (reinterpret_cast<uintptr_t>(dy_top) & 15) == 0),
+               "stage %d needs dy_top, 16-byte aligned", top);
+    XB_REQUIRE(h, bottom == 0 || (dy_bottom && (reinterpret_cast<uintptr_t>(dy_bottom) & 15) == 0),
+               "stage %d needs dy_bottom, 16-byte aligned", bottom);
+    XB_REQUIRE(h, bottom > 0 || signal, "the stem stage needs the signal");
+    XB_REQUIRE(h, bottom > 0 || sig_dtype == XB_SIG_F32 || sig_dtype == XB_SIG_I16, "the backward reads fp32 or int16 signal");
+    // parameter tensors of stage k: 6 -> 26, 27; k in 1..5 (LSTM layer k-1) -> 4k+2 .. 4k+5; 0 -> 0 .. 5
+    for (int k = bottom; k <= top; k++) {
+        const int lo = k == 6 ? 26 : k == 0 ? 0 : 4 * k + 2, hi = k == 6 ? 27 : 4 * k + 5;
+        for (int i = lo; i <= hi; i++) XB_REQUIRE(h, grads[i] != nullptr, "gradient tensor %d is NULL", i);
+    }
+    if (h->train->drop.active && !(top == 6 && bottom == 0))
+        return xb_fail(h, XB_ERR_UNSUPPORTED, "the last forward applied dropout: only the whole backward (stages 6 .. 0) runs");
     XB_CUDA(h, cudaSetDevice(h->device));
     xb_train_ws *w = h->train;
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    const int N = w->N, T = w->T, TN = T * N, F = XB_FEATURES, HP = h->head_rows_padded, S = h->C * h->NZ, L = T * XB_STRIDE;
-    const xb_dropout &drop = w->drop;
-    const bool drop_stem = drop.on(0) || drop.on(1);
-
-    // ---- head
-    {
-        const size_t n = (size_t)TN * HP;
-        head_bwd_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(dscores, scores, (size_t)TN, h->n_base, h->NZ, h->head_rows, HP,
-                                                                  h->expand_blanks ? S : h->head_rows, h->expand_blanks,
-                                                                  h->scale, reinterpret_cast<__nv_bfloat16 *>(w->dzh));
-        XB_LAUNCH_CHECK(h);
-        if (int rc = colsum(h, w->dzh, TN, h->head_rows, HP, grads[27], s)) return rc;
-        if (int rc = transpose_to_bf16(h, w->dzh, TN, HP, HP, true, w->dzhT, s)) return rc;
-        if (int rc = transpose_to_bf16(h, w->x[5], TN, F, F, false, w->XT[1], s)) return rc;
-        if (int rc = gemm_bf16(h, EPI_F32, w->dzhT, h->head_rows, TN, w->XT[1], F, TN, TN, grads[26], F, s)) return rc;
-        if (int rc = gemm_bf16(h, EPI_BF16OUT, w->dzh, TN, HP, h->head_wT, F, HP, HP, w->dy[1], F, s)) return rc;
+    // stage k's outgoing gradient: dy_bottom for the last stage, else the workspace buffer the next stage reads
+    const void *dy = dy_top;
+    if (top == 6) {
+        void *out = bottom == 6 ? dy_bottom : w->dy[1];
+        if (int rc = head_bwd(h, w, scores, dscores, grads, out, s)) return rc;
+        dy = out;
+    } else if (top >= 1) {
+        // layer top-1 reads its own output transposed, which the stage above it leaves behind in a chained backward
+        const int l = top - 1;
+        if (int rc = transpose_to_bf16(h, w->x[l + 1], w->T * w->N, XB_FEATURES, XB_FEATURES, false, w->XT[(l + 1) & 1], s)) return rc;
     }
-    // ---- LSTM layers 4 .. 0.  XT[(l+1) & 1] holds the transposed OUTPUT of layer l, dy[(l+1) & 1] the gradient w.r.t. it.
-    for (int l = 4; l >= 0; l--) {
-        const xb_lstm_weights &lw = h->lstm[l];
-        const bool reverse = (l % 2) == 0;
-        const void *dy = w->dy[(l + 1) & 1];
-        BpttMaps maps;
-        if (int rc = xb_bptt_make_maps(h, &maps, w->DZ, lw.w_hhT, w->saved[l], T, N)) return rc;
-        {
-        xb_stage_timer tm_bptt(h, XB_ST_TRAIN_BPTT, s);
-        for (int i = 0; i < T; i++) {                       // forward ran t = (reverse ? T-1 .. 0 : 0 .. T-1); walk it backwards
-            const int t = reverse ? i : T - 1 - i;
-            const int t_next = reverse ? t - 1 : t + 1;     // the step the forward ran AFTER t (its dz feeds dh_t); i == 0: none
-            const int t_prev = reverse ? t + 1 : t - 1;     // the step the forward ran BEFORE t (its c is c_prev)
-            BpttStep p;
-            p.N = N; p.t_cur = t;
-            p.t_next = (i == 0) ? -1 : t_next;
-            p.t_prev = (t_prev >= 0 && t_prev < T) ? t_prev : -1;
-            p.dy = dy; p.dcstate = w->dcstate;
-            if (int rc = xb_bptt_step_launch(h, maps, p, /*dependent=*/i > 0, s)) return rc;
-        }
-        }
-        float *g_wih = grads[6 + 4 * l], *g_whh = grads[7 + 4 * l], *g_bih = grads[8 + 4 * l], *g_bhh = grads[9 + 4 * l];
-        if (int rc = transpose_to_bf16(h, w->DZ, TN, XB_GATES, XB_GATES, true, w->DZT, s, g_bih)) return rc;   // + db = colsum DZ
-        XB_CUDA(h, cudaMemcpyAsync(g_bhh, g_bih, XB_GATES * sizeof(float), cudaMemcpyDeviceToDevice, s));
-        if (int rc = transpose_to_bf16(h, w->x[l], TN, F, F, false, w->XT[l & 1], s)) return rc;
-        // layer l > 0 read the dropped copy of x[l] (site l + 2): dW_ih takes that, transposed through the mask into xd
-        const bool drop_in = l > 0 && drop.on(l + 2);
-        if (drop_in) { if (int rc = transpose_to_bf16(h, w->x[l], TN, F, F, false, w->xd, s, nullptr, &drop, l + 2)) return rc; }
-        // dW_ih = DZ^T x_l and dW_hh = sum over the steps that had a predecessor of dz_t (x) h_prev (a time shift of N columns
-        // between DZ^T and Y^T), one launch over 128 x 256 tiles (wgrad_gemm.cu)
-        {
-            xb_stage_timer tm(h, XB_ST_TRAIN_WGRAD, s);
-            if (int rc = xb_lstm_wgrad_launch(h, w->DZT, drop_in ? w->xd : w->XT[l & 1], w->XT[(l + 1) & 1], T, N, reverse, g_wih,
-                                              g_whh, s)) return rc;
-        }
-        if (int rc = gemm_bf16(h, EPI_BF16OUT, w->DZ, TN, XB_GATES, lw.w_ihT, F, XB_GATES, XB_GATES, w->dy[l & 1], F, s)) return rc;
-        // gradient w.r.t. the dropped input -> w.r.t. the output of the layer below (l == 0: the conv3 output, site 2)
-        if (drop.on(l + 2)) { if (int rc = dropout16(h, w->dy[l & 1], w->dy[l & 1], (size_t)TN * F, true, drop, l + 2, s)) return rc; }
+    for (int k = std::min(top, 5); k >= std::max(bottom, 1); k--) {
+        const int l = k - 1;
+        void *out = k == bottom ? dy_bottom : w->dy[l & 1];
+        if (int rc = lstm_layer_bwd(h, w, l, dy, out, grads, s)) return rc;
+        dy = out;
     }
-    // ---- convolution stem: dy[0] is the gradient w.r.t. x[0] (T, N, 768)
-    {
-        if (int rc = xb_conv12_im2col(h, signal, sig_dtype, N, L, s, &drop)) return rc;   // im2col rows of this batch into h->c2
-        CUtensorMap tmA, tmB;
-        if (int rc = xb_make_tmap_2d(h, &tmA, h->c2, (uint64_t)TN, XB_CONV3_K, XB_CONV3_K)) return rc;
-        if (int rc = xb_make_tmap_2d(h, &tmB, h->conv3_w, F, XB_CONV3_K, XB_CONV3_K)) return rc;
-        GemmParams p;
-        p.M = TN; p.N = F; p.K = XB_CONV3_K; p.bias = h->conv3_b; p.out = w->dpre; p.ldo = F; p.T = T; p.NB = N; p.dy = w->dy[0];
-        if (int rc = xb_gemm_launch(h, EPI_CONV3_BWD, tmA, tmB, p, s, false)) return rc;
-        if (int rc = transpose_to_bf16(h, w->dpre, TN, F, F, true, w->dpreT, s, grads[5])) return rc;       // + db3 = colsum d pre
-        if (int rc = transpose_to_bf16(h, h->c2, TN, XB_CONV3_K, XB_CONV3_K, false, w->colT, s)) return rc;
-        // dW3 in im2col column order (768, 320): the caller drops the 16 padding columns and permutes to (768, 16, 19)
-        if (int rc = gemm_bf16(h, EPI_F32, w->dpreT, F, TN, w->colT, XB_CONV3_K, TN, TN, grads[4], XB_CONV3_K, s)) return rc;
-        if (int rc = gemm_bf16(h, EPI_BF16OUT, w->dpre, TN, F, h->conv3_wT, XB_CONV3_K, F, F, w->dcol, XB_CONV3_K, s)) return rc;
-        const size_t n2 = (size_t)N * L * XB_C2_CH;
-        col2im_kernel<<<(unsigned)((n2 + 255) / 256), 256, 0, s>>>(reinterpret_cast<const __nv_bfloat16 *>(w->dcol), N, T, L, w->dc2);
-        XB_LAUNCH_CHECK(h);
-        XB_CUDA(h, cudaMemsetAsync(w->dc1, 0, (size_t)N * L * 4 * sizeof(float), s));
-        XB_CUDA(h, cudaMemsetAsync(grads[2], 0, 320 * sizeof(float), s));
-        XB_CUDA(h, cudaMemsetAsync(grads[3], 0, 16 * sizeof(float), s));
-        XB_CUDA(h, cudaMemsetAsync(grads[0], 0, 20 * sizeof(float), s));
-        XB_CUDA(h, cudaMemsetAsync(grads[1], 0, 4 * sizeof(float), s));
-        dim3 g2((L + 255) / 256, N);
-        if (sig_dtype == XB_SIG_F32) {
-            if (drop_stem)
-                conv2_bwd_kernel<true, float><<<g2, 256, 0, s>>>(reinterpret_cast<const float *>(signal), L, h->conv1_w, h->conv1_b,
-                                                                 h->conv2_w, h->conv2_b, w->dc2, w->dc1, grads[2], grads[3], drop);
-            else
-                conv2_bwd_kernel<false, float><<<g2, 256, 0, s>>>(reinterpret_cast<const float *>(signal), L, h->conv1_w, h->conv1_b,
-                                                                  h->conv2_w, h->conv2_b, w->dc2, w->dc1, grads[2], grads[3], drop);
-            XB_LAUNCH_CHECK(h);
-            conv1_bwd_kernel<float><<<dim3(4, N), 256, 0, s>>>(reinterpret_cast<const float *>(signal), L, h->conv1_w, h->conv1_b, w->dc1,
-                                                              grads[0], grads[1]);
-        } else {
-            if (drop_stem)
-                conv2_bwd_kernel<true, int16_t><<<g2, 256, 0, s>>>(reinterpret_cast<const int16_t *>(signal), L, h->conv1_w, h->conv1_b,
-                                                                   h->conv2_w, h->conv2_b, w->dc2, w->dc1, grads[2], grads[3], drop);
-            else
-                conv2_bwd_kernel<false, int16_t><<<g2, 256, 0, s>>>(reinterpret_cast<const int16_t *>(signal), L, h->conv1_w, h->conv1_b,
-                                                                    h->conv2_w, h->conv2_b, w->dc2, w->dc1, grads[2], grads[3], drop);
-            XB_LAUNCH_CHECK(h);
-            conv1_bwd_kernel<int16_t><<<dim3(4, N), 256, 0, s>>>(reinterpret_cast<const int16_t *>(signal), L, h->conv1_w, h->conv1_b,
-                                                                w->dc1, grads[0], grads[1]);
-        }
-        XB_LAUNCH_CHECK(h);
-    }
+    if (bottom == 0) return stem_bwd(h, w, signal, sig_dtype, dy, grads, s);
     return XB_OK;
 }
 
