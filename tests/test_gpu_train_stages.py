@@ -301,3 +301,20 @@ def test_stage_ranges_are_checked():
     with pytest.raises(RuntimeError, match=r'\(-4\)'):
         h.encoder_backward_stages(3, 3, dy_top=dy)
     h.close()
+
+
+def test_backward_times_the_head_and_stem_kernels():
+    """xb_stage_times row train_head_conv_bwd: the CRF head's and the convolution stem's own kernels, timed in every
+    backward (the transpositions and GEMMs around them have rows of their own)."""
+    from xna_basecaller_b200._lib import Handle
+    h = Handle(ALPHABETS[5], 3, max_N=8, max_T=20, train=True)
+    h.load_weights(bo.reference_state_dict(n_base=5, seed=12, **REF_SCALE))
+    scores = h.encoder_train(synthetic_signal(3, 8, 100).cuda())
+    ds = torch.randn(scores.shape, generator=torch.Generator().manual_seed(6)).cuda() * 1e-2
+    h.set_profiling(True)
+    h.stage_times()
+    h.encoder_backward(ds)
+    ms, spans = h.stage_times()['train_head_conv_bwd']
+    h.set_profiling(False)
+    h.close()
+    assert spans > 0 and ms > 0

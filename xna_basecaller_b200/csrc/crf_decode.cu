@@ -1,5 +1,5 @@
 // CTC-CRF scans on RAW scores for sm_100a, in the log domain: Log-semiring forward (alpha / logZ), backward scans in
-// either semiring, Max-semiring forward sweep with arg-max, labels and left-packing (CTC_CRF.logZ / forward_scores /
+// either semiring, Max-semiring forward sweep with arg-max edges and labels (CTC_CRF.logZ / forward_scores /
 // backward_scores / viterbi).  decode_batch (posteriors + max-marginal Viterbi) lives in crf_decode_lin.cu.
 //
 // Reference semantics: bonito/crf/model.py:26-46 (idx, logZ), :51-61 (forward/backward scores), :92-100
@@ -152,14 +152,12 @@ crf_bscan_kernel(const float *__restrict__ scores, int T, int N, float *__restri
 }
 
 // --------------------------------------------------------------------------------------------------
-// Forward sweep, Max semiring, over lp with the stored Max-beta: arg-max edge per step -> label
-// (edge % NZ), then path_to_str + left-pack for the row.   dynamic smem tail holds T labels.
+// Forward sweep, Max semiring, over the scores with the stored Max-beta: arg-max edge per step -> edges_out and / or
+// its label (edge % NZ) -> labels_out.
 template <int NB, int SL>
 __global__ void __launch_bounds__(Lat<NB, SL>::NT)
-crf_viterbi_fwd_kernel(const float *__restrict__ lp, const float *__restrict__ bmax, int T, int N,
-                       int8_t *__restrict__ labels_out, int8_t *__restrict__ seq_out,
-                       int8_t *__restrict__ qs_out, int32_t *__restrict__ lens_out, int32_t *__restrict__ edges_out,
-                       Alphabet abc) {
+crf_viterbi_fwd_kernel(const float *__restrict__ scores, const float *__restrict__ bmax, int T, int N,
+                       int8_t *__restrict__ labels_out, int32_t *__restrict__ edges_out) {
     using L = Lat<NB, SL>;
     constexpr int C = L::C, NZ = L::NZ, S = L::S, NT = L::NT, W = L::W, D = L::D;
     extern __shared__ __align__(16) float smem[];
@@ -168,14 +166,25 @@ crf_viterbi_fwd_kernel(const float *__restrict__ lp, const float *__restrict__ b
     float *am = ringB + D * NT;          // 2 * NT
     float *bval = am + 2 * NT;           // 2 * W
     int *bidx = reinterpret_cast<int *>(bval + 2 * W);      // 2 * W
-    int *scan = bidx + 2 * W;            // NT + 1
-    int8_t *lab = reinterpret_cast<int8_t *>(scan + NT + 1);   // T
     const int n = blockIdx.x, c = threadIdx.x, lane = c & 31, w = c >> 5;
     const bool act = c < C;
-    const float *base = lp + (size_t)n * S;
+    const float *base = scores + (size_t)n * S;
     const size_t row = (size_t)N * S;
     const float *bbase = bmax + (size_t)n * C;
     const size_t brow = (size_t)N * C;
+    // thread 0: step t's arg-max over the per-warp candidates (first index on ties)
+    auto finish = [&](int t) {
+        const int q = t & 1;
+        float bv = bval[q * W];
+        int bi = bidx[q * W];
+        for (int j = 1; j < W; j++) {
+            float v = bval[q * W + j];
+            int ix = bidx[q * W + j];
+            if (v > bv || (v == bv && ix < bi)) { bv = v; bi = ix; }
+        }
+        if (labels_out) labels_out[(size_t)n * T + t] = (int8_t)(bi % NZ);
+        if (edges_out) edges_out[(size_t)n * T + t] = bi;
+    };
 
 #pragma unroll
     for (int j = 0; j < D - 1; j++) {
@@ -206,18 +215,7 @@ crf_viterbi_fwd_kernel(const float *__restrict__ lp, const float *__restrict__ b
             fetchB += brow;
             cp_async_commit();
         }
-        if (c == 0 && t > 0) {           // finish step t-1: reduce the per-warp candidates
-            const int q = (t - 1) & 1;
-            float bv = bval[q * W];
-            int bi = bidx[q * W];
-            for (int j = 1; j < W; j++) {
-                float v = bval[q * W + j];
-                int ix = bidx[q * W + j];
-                if (v > bv || (v == bv && ix < bi)) { bv = v; bi = ix; }
-            }
-            lab[t - 1] = (int8_t)(bi % NZ);
-            if (edges_out) edges_out[(size_t)n * T + t - 1] = bi;
-        }
+        if (c == 0 && t > 0) finish(t - 1);
         const float *M = ring + (t % D) * S + c * NZ;
         const float *ac = am + (t & 1) * NT;
         float *an = am + ((t + 1) & 1) * NT;
@@ -250,21 +248,7 @@ crf_viterbi_fwd_kernel(const float *__restrict__ lp, const float *__restrict__ b
         if (lane == 0) { bval[(t & 1) * W + w] = best; bidx[(t & 1) * W + w] = besti; }
     }
     __syncthreads();
-    if (c == 0 && T > 0) {
-        const int q = (T - 1) & 1;
-        float bv = bval[q * W];
-        int bi = bidx[q * W];
-        for (int j = 1; j < W; j++) {
-            float v = bval[q * W + j];
-            int ix = bidx[q * W + j];
-            if (v > bv || (v == bv && ix < bi)) { bv = v; bi = ix; }
-        }
-        lab[T - 1] = (int8_t)(bi % NZ);
-        if (edges_out) edges_out[(size_t)n * T + T - 1] = bi;
-    }
-    __syncthreads();
-
-    pack_labels<NT>(lab, scan, T, n, labels_out, seq_out, qs_out, lens_out, abc);
+    if (c == 0 && T > 0) finish(T - 1);
 }
 
 template <int NB, int SL> size_t smem_alpha() {
@@ -275,18 +259,14 @@ template <int NB, int SL> size_t smem_bscan() {
     using L = Lat<NB, SL>;
     return sizeof(float) * (L::D * L::S + 2 * L::NT);
 }
-template <int NB, int SL> size_t smem_vit(int T) {
+template <int NB, int SL> size_t smem_vit() {
     using L = Lat<NB, SL>;
-    return sizeof(float) * (L::D * L::S + L::D * L::NT + 2 * L::NT + 4 * L::W + L::NT + 1) + ((T + 15) / 16) * 16;
-}
-
-template <typename K> int set_smem(xb_handle *h, K kernel, size_t bytes) {
-    if (bytes > 48 * 1024) XB_CUDA(h, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    return XB_OK;
+    return sizeof(float) * (L::D * L::S + L::D * L::NT + 2 * L::NT + 4 * L::W);
 }
 
 template <int NB, int SL>
-int alpha_impl(xb_handle *h, const float *scores, int T, int N, float *alpha, float *logz, int use_max, cudaStream_t s) {
+int alpha_impl(Lat<NB, SL>, xb_handle *h, const float *scores, int T, int N, float *alpha, float *logz, int use_max,
+               cudaStream_t s) {
     using L = Lat<NB, SL>;
     size_t sm = smem_alpha<NB, SL>();
     if (use_max) {
@@ -302,7 +282,8 @@ int alpha_impl(xb_handle *h, const float *scores, int T, int N, float *alpha, fl
     return XB_OK;
 }
 template <int NB, int SL>
-int backward_impl(xb_handle *h, const float *scores, int T, int N, float *bmax, float *beta, int mode, cudaStream_t s) {
+int backward_impl(Lat<NB, SL>, xb_handle *h, const float *scores, int T, int N, float *bmax, float *beta, int mode,
+                  cudaStream_t s) {
     using L = Lat<NB, SL>;
     if (mode == 1) {
         auto k = crf_bscan_kernel<NB, SL, true>;
@@ -319,52 +300,32 @@ int backward_impl(xb_handle *h, const float *scores, int T, int N, float *bmax, 
     return XB_OK;
 }
 template <int NB, int SL>
-int vit_impl(xb_handle *h, const float *lp, const float *bmax, int T, int N, int8_t *labels, int8_t *seq,
-             int8_t *qs, int32_t *lens, int32_t *edges, cudaStream_t s) {
+int vit_impl(Lat<NB, SL>, xb_handle *h, const float *scores, const float *bmax, int T, int N, int8_t *labels, int32_t *edges,
+             cudaStream_t s) {
     using L = Lat<NB, SL>;
     auto k = crf_viterbi_fwd_kernel<NB, SL>;
-    size_t sm = smem_vit<NB, SL>(T);
+    size_t sm = smem_vit<NB, SL>();
     if (int rc = set_smem(h, k, sm)) return rc;
-    Alphabet abc;
-    for (int i = 0; i < 16; i++) abc.ch[i] = h->alphabet[i];
-    k<<<N, L::NT, sm, s>>>(lp, bmax, T, N, labels, seq, qs, lens, edges, abc);
+    k<<<N, L::NT, sm, s>>>(scores, bmax, T, N, labels, edges);
     XB_LAUNCH_CHECK(h);
     return XB_OK;
 }
-
-#define XB_LATTICE_DISPATCH(h, CALL)                                                               \
-    switch ((h)->n_base * 10 + (h)->state_len) {                                                   \
-        case 43: return CALL(4, 3);                                                                \
-        case 53: return CALL(5, 3);                                                                \
-        case 63: return CALL(6, 3);                                                                \
-        case 44: return CALL(4, 4);                                                                \
-        case 22: return CALL(2, 2);                                                                \
-        default:                                                                                   \
-            return xb_fail((h), XB_ERR_UNSUPPORTED, "no CRF kernel compiled for n_base=%d state_len=%d", \
-                           (h)->n_base, (h)->state_len);                                           \
-    }
 
 }  // namespace
 
 int xb_decode_alpha(xb_handle *h, const float *scores, int T, int N, float *alpha, float *logz, int use_max, cudaStream_t s) {
     xb_stage_timer tm(h, XB_ST_CRF_ALPHA, s);
-#define CALL(NB, SL) alpha_impl<NB, SL>(h, scores, T, N, alpha, logz, use_max, s)
-    XB_LATTICE_DISPATCH(h, CALL)
-#undef CALL
+    return lattice_dispatch(h, [&](auto lat) { return alpha_impl(lat, h, scores, T, N, alpha, logz, use_max, s); });
 }
 
 // mode 1: Max-semiring backward scan of the raw scores into bmax;  mode 2: Log-semiring scan into beta
 int xb_decode_backward(xb_handle *h, const float *scores, int T, int N, float *bmax, float *beta, int mode, cudaStream_t s) {
     xb_stage_timer tm(h, XB_ST_CRF_BACKWARD, s);
-#define CALL(NB, SL) backward_impl<NB, SL>(h, scores, T, N, bmax, beta, mode, s)
-    XB_LATTICE_DISPATCH(h, CALL)
-#undef CALL
+    return lattice_dispatch(h, [&](auto lat) { return backward_impl(lat, h, scores, T, N, bmax, beta, mode, s); });
 }
 
-int xb_decode_viterbi_fwd(xb_handle *h, const float *lp, const float *bmax, int T, int N, int8_t *labels,
-                          int8_t *seq, int8_t *qstring, int32_t *lens, int32_t *edges, cudaStream_t s) {
+int xb_decode_viterbi_fwd(xb_handle *h, const float *scores, const float *bmax, int T, int N, int8_t *labels, int32_t *edges,
+                          cudaStream_t s) {
     xb_stage_timer tm(h, XB_ST_CRF_VITERBI, s);
-#define CALL(NB, SL) vit_impl<NB, SL>(h, lp, bmax, T, N, labels, seq, qstring, lens, edges, s)
-    XB_LATTICE_DISPATCH(h, CALL)
-#undef CALL
+    return lattice_dispatch(h, [&](auto lat) { return vit_impl(lat, h, scores, bmax, T, N, labels, edges, s); });
 }

@@ -465,20 +465,15 @@ crf_lin_viterbi_kernel(const float *__restrict__ scores, const float *__restrict
     pack_labels<NTT>(lab, scan, T, n, labels_out, seq_out, qs_out, lens_out, abc);
 }
 
-template <typename K> int set_smem(xb_handle *h, K kernel, size_t bytes) {
-    if (bytes > 48 * 1024) XB_CUDA(h, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    return XB_OK;
-}
-
-template <int NB, int SL, bool LIN>
-int lin_impl(xb_handle *h, const float *scores, int T, int N, int8_t *labels, int8_t *seq, int8_t *qs, int32_t *lens,
-             float *post, cudaStream_t s) {
+template <bool LIN, int NB, int SL>
+int lin_impl(Lat<NB, SL>, xb_handle *h, const float *scores, int T, int N, int8_t *labels, int8_t *seq, int8_t *qs,
+             int32_t *lens, float *post, cudaStream_t s) {
     using L = Lat<NB, SL>;
     using R = Ring<NB, SL>;
     constexpr int NTT = L::NT + 32;
     XB_REQUIRE(h, (reinterpret_cast<uintptr_t>(scores) & 15) == 0, "scores must be 16-byte aligned");
     // state vectors with pitch VP in handle workspace (xb_create sizes the three buffers for it)
-    float *alpha = h->alpha, *beta = h->lp, *bmax = h->bmax;
+    float *alpha = h->alpha, *beta = h->beta, *bmax = h->bmax;
     {
         xb_stage_timer tm(h, XB_ST_CRF_ALPHA, s);
         auto k = crf_lin_alpha_kernel<NB, SL, LIN>;
@@ -514,33 +509,14 @@ int lin_impl(xb_handle *h, const float *scores, int T, int N, int8_t *labels, in
     return XB_OK;
 }
 
-// elementwise E = xb_score_exp(M): the conversion the fused head applies in its epilogue, as a stand-alone kernel for tests
-__global__ void score_exp_kernel(const float *__restrict__ in, float *__restrict__ out, size_t n) {
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
-        out[i] = xb_score_exp(in[i]);
-}
-
 }  // namespace
 
 // Decode of (T, N, C*NZ) scores: labels / left-packed letters / lengths and, optionally, the posteriors.
 // lin_input: the buffer holds E = exp(scores) (the fused head's output) instead of the scores.
 int xb_decode_lin(xb_handle *h, const float *scores, int lin_input, int T, int N, int8_t *labels, int8_t *seq, int8_t *qs,
                   int32_t *lens, float *post, cudaStream_t s) {
-#define CALL(NB, SL) (lin_input ? lin_impl<NB, SL, true>(h, scores, T, N, labels, seq, qs, lens, post, s) \
-                                : lin_impl<NB, SL, false>(h, scores, T, N, labels, seq, qs, lens, post, s))
-    switch (h->n_base * 10 + h->state_len) {
-        case 43: return CALL(4, 3);
-        case 53: return CALL(5, 3);
-        case 63: return CALL(6, 3);
-        case 44: return CALL(4, 4);
-        case 22: return CALL(2, 2);
-    }
-#undef CALL
-    return xb_fail(h, XB_ERR_UNSUPPORTED, "no CRF kernel compiled for n_base=%d state_len=%d", h->n_base, h->state_len);
-}
-
-int xb_score_exp_launch(xb_handle *h, const float *in, float *out, size_t n, cudaStream_t s) {
-    score_exp_kernel<<<h->num_sms * 8, 256, 0, s>>>(in, out, n);
-    XB_LAUNCH_CHECK(h);
-    return XB_OK;
+    return lattice_dispatch(h, [&](auto lat) {
+        return lin_input ? lin_impl<true>(lat, h, scores, T, N, labels, seq, qs, lens, post, s)
+                         : lin_impl<false>(lat, h, scores, T, N, labels, seq, qs, lens, post, s);
+    });
 }

@@ -1,5 +1,6 @@
 // Shared pieces of the CRF scan kernels (crf_decode.cu: Log / Max semiring scans on raw scores; crf_decode_lin.cu: the
-// linear-domain decode): lattice constants, the cp.async score-row ring, warp reductions with a fixed evaluation order.
+// linear-domain decode): lattice constants, the list of supported lattices and the dispatch over it, the cp.async
+// score-row ring, warp reductions with a fixed evaluation order.
 #pragma once
 #include "xb_common.cuh"
 #include "xb_exact_math.h"
@@ -18,6 +19,35 @@ template <int NB, int SL> struct Lat {
     static constexpr int D = D0 < 2 ? 2 : (D0 > 8 ? 8 : D0);   // ring depth (rows in flight + 1)
     static_assert(S % 2 == 0, "row must be a whole number of 8-byte chunks");
 };
+
+// The lattices (n_base, state_len) the CRF kernels are compiled for -- the one list of them: f(Lat<NB, SL>()) for one of
+// these, unsupported() for any other.
+template <typename F, typename U> int for_lattice(int n_base, int state_len, F &&f, U &&unsupported) {
+    switch (n_base * 10 + state_len) {
+        case 43: return f(Lat<4, 3>());
+        case 53: return f(Lat<5, 3>());
+        case 63: return f(Lat<6, 3>());
+        case 44: return f(Lat<4, 4>());
+        case 22: return f(Lat<2, 2>());
+    }
+    return unsupported();
+}
+
+inline bool lattice_supported(int n_base, int state_len) {
+    return for_lattice(n_base, state_len, [](auto) { return 1; }, [] { return 0; });
+}
+
+// f(Lat<NB, SL>()) for the handle's lattice
+template <typename F> int lattice_dispatch(xb_handle *h, F &&f) {
+    return for_lattice(h->n_base, h->state_len, f, [h] {
+        return xb_fail(h, XB_ERR_UNSUPPORTED, "no CRF kernel compiled for n_base=%d state_len=%d", h->n_base, h->state_len);
+    });
+}
+
+template <typename K> int set_smem(xb_handle *h, K kernel, size_t bytes) {
+    if (bytes > 48 * 1024) XB_CUDA(h, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    return XB_OK;
+}
 
 __device__ __forceinline__ void cp_async4(float *dst, const float *src) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"((uint32_t)__cvta_generic_to_shared(dst)), "l"(src));

@@ -17,8 +17,8 @@
 //   LSTM l   T launches of the BPTT step kernel (lstm_bptt.cu), one per time step in reverse forward order, chained with
 //            programmatic dependent launches: dh_t = dz_{next} W_hh + dy_t, then the cell backward -> DZ[t] (T*N, 3072)
 //            and the running dc;  dW_ih = DZ^T x_l,  dW_hh = DZ^T h_prev (time-shifted view of the layer output),
-//            db = colsum DZ (taken inside the transposition),  dy_{l-1} = DZ W_ih.   The K = T*N contractions run on
-//            K-major transposed copies (transpose16v_kernel).
+//            db = colsum DZ,  dy_{l-1} = DZ W_ih.   The K = T*N contractions run on K-major transposed copies
+//            (transpose16v_kernel), which also take every bias gradient's column sum on the way.
 //   conv3    pre-activation recomputed from the im2col rows (EPI_CONV3_BWD) -> d pre;  dW3 = d pre^T col;  db3;
 //            d col = d pre W3 -> col2im -> conv2 / conv1 backward (conv_stem_bwd kernels below).
 // Measured at N = 512, T = 800 (profiles/r02_config5_train_step_v5.json): 154 ms per training step, of which the 4000 BPTT
@@ -70,45 +70,6 @@ struct xb_train_ws {
 };
 
 namespace {
-
-// (R, C) 16-bit row-major (row pitch ld_in elements; fp16 or bf16) -> (C, R) bf16 row-major
-template <bool IN_BF16>
-__global__ void transpose16_kernel(const uint16_t *__restrict__ in, int R, int C, int ld_in, __nv_bfloat16 *__restrict__ out) {
-    __shared__ uint16_t tile[32][33];
-    const int r0 = blockIdx.y * 32, c0 = blockIdx.x * 32;
-    for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-        const int r = r0 + i, c = c0 + threadIdx.x;
-        tile[i][threadIdx.x] = (r < R && c < C) ? in[(size_t)r * ld_in + c] : (uint16_t)0;
-    }
-    __syncthreads();
-    for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-        const int c = c0 + i, r = r0 + threadIdx.x;
-        if (c < C && r < R) {
-            const uint16_t v = tile[threadIdx.x][i];
-            __nv_bfloat16 o;
-            if (IN_BF16) o = *reinterpret_cast<const __nv_bfloat16 *>(&v);
-            else o = __float2bfloat16_rn(__half2float(*reinterpret_cast<const __half *>(&v)));
-            out[(size_t)c * R + r] = o;
-        }
-    }
-}
-
-// column sums of a (R, C) bf16 matrix into fp32 out[C] (out zeroed by the caller); grid (C/32, row slabs)
-__global__ void colsum_kernel(const __nv_bfloat16 *__restrict__ in, int R, int C, int ld, float *__restrict__ out) {
-    __shared__ float part[8][33];
-    const int c = blockIdx.x * 32 + threadIdx.x;
-    const int rows_per = (R + gridDim.y - 1) / gridDim.y;
-    const int r_lo = blockIdx.y * rows_per, r_hi = min(R, r_lo + rows_per);
-    float s = 0.0f;
-    if (c < C)
-        for (int r = r_lo + threadIdx.y; r < r_hi; r += 8) s += __bfloat162float(in[(size_t)r * ld + c]);
-    part[threadIdx.y][threadIdx.x] = s;
-    __syncthreads();
-    if (threadIdx.y == 0 && c < C) {
-        for (int i = 1; i < 8; i++) s += part[i][threadIdx.x];
-        atomicAdd(out + c, s);
-    }
-}
 
 // dropout of a 16-bit tensor whose element index is its flat offset (sites 2..6): eight elements per iteration; in == out
 // is allowed
@@ -295,26 +256,23 @@ int alloc(xb_handle *h, void **p, size_t bytes) {
     return XB_OK;
 }
 
-int colsum(xb_handle *h, const void *in, int R, int C, int ld, float *out, cudaStream_t s) {
-    XB_CUDA(h, cudaMemsetAsync(out, 0, (size_t)C * sizeof(float), s));
-    int slabs = (R + 2047) / 2048;
-    if (slabs > 256) slabs = 256;
-    colsum_kernel<<<dim3((C + 31) / 32, slabs), dim3(32, 8), 0, s>>>(reinterpret_cast<const __nv_bfloat16 *>(in), R, C, ld, out);
-    XB_LAUNCH_CHECK(h);
-    return XB_OK;
-}
+// The three forms of the training step's transpositions (R, C) 16-bit -> (C, R) bf16:
+//   TR_BF16_COLSUM  a bf16 gradient, plus the column sums of its first nsum columns (a bias gradient)
+//   TR_F16          an fp16 activation
+//   TR_F16_DROP     an fp16 activation masked by a dropout site
+enum TrForm { TR_BF16_COLSUM, TR_F16, TR_F16_DROP };
 
-// Vector form of the same transposition for shapes whose rows are 16-byte multiples (all of the training step's): 64 x 64
-// tiles, 16-byte global loads and stores on both sides.  Two input rows are packed into one 32-bit word per column, so the
-// transposed tile is written and read as words (pitch 33: the read side is conflict free, the write side two-way).  Each
-// CTA walks a slab of row tiles; with COLSUM it also accumulates the column sums of its slab (the bias gradients) and adds
-// them to colsum_out once -- the separate colsum pass over the same 2.5 GB is gone.
-// DROP (fp16 input with ld_in == C): the input is masked by dropout site `site` (element index r * C + c) on the way in,
-// rounded to fp16 as the forward's dropped copy was, then converted -- the transposed dropped copy without storing it.
-template <bool IN_BF16, bool COLSUM, bool DROP = false>
-__global__ void __launch_bounds__(256) transpose16v_kernel(const uint16_t *__restrict__ in, int R, int C, int ld_in,
+// 64 x 64 tiles, 16-byte global loads and stores on both sides (R, C multiples of 8, 16-byte aligned buffers).  Two input
+// rows are packed into one 32-bit word per column, so the transposed tile is written and read as words (pitch 33: the read
+// side is conflict free, the write side two-way).  Each CTA walks a slab of row tiles; TR_BF16_COLSUM also accumulates the
+// column sums of its slab and adds them to colsum_out once -- no separate column-sum pass over the same matrix.
+// TR_F16_DROP: the input is masked by dropout site `site` (element index r * C + c) on the way in, rounded to fp16 as the
+// forward's dropped copy was, then converted -- the transposed dropped copy without storing it.
+template <TrForm FORM>
+__global__ void __launch_bounds__(256) transpose16v_kernel(const uint16_t *__restrict__ in, int R, int C,
                                                            __nv_bfloat16 *__restrict__ out, float *__restrict__ colsum_out,
-                                                           const xb_dropout drop = xb_dropout(), int site = 0) {
+                                                           int nsum, const xb_dropout drop, int site) {
+    constexpr bool IN_BF16 = FORM == TR_BF16_COLSUM, COLSUM = FORM == TR_BF16_COLSUM, DROP = FORM == TR_F16_DROP;
     __shared__ uint32_t tileT[64][33];
     const int t = threadIdx.x;
     const int c0 = blockIdx.x * 64;
@@ -335,11 +293,11 @@ __global__ void __launch_bounds__(256) transpose16v_kernel(const uint16_t *__res
             const int r = r0 + 2 * rp, c = c0 + cg * 8;
             uint4 a = make_uint4(0, 0, 0, 0), b = make_uint4(0, 0, 0, 0);
             if (c < C) {
-                if (r < R) a = *reinterpret_cast<const uint4 *>(in + (size_t)r * ld_in + c);
-                if (r + 1 < R) b = *reinterpret_cast<const uint4 *>(in + (size_t)(r + 1) * ld_in + c);
+                if (r < R) a = *reinterpret_cast<const uint4 *>(in + (size_t)r * C + c);
+                if (r + 1 < R) b = *reinterpret_cast<const uint4 *>(in + (size_t)(r + 1) * C + c);
                 if (DROP) {
-                    if (r < R) a = xb_dropout8<IN_BF16>(drop, site, (uint64_t)r * C + c, a);
-                    if (r + 1 < R) b = xb_dropout8<IN_BF16>(drop, site, (uint64_t)(r + 1) * C + c, b);
+                    if (r < R) a = xb_dropout8<false>(drop, site, (uint64_t)r * C + c, a);
+                    if (r + 1 < R) b = xb_dropout8<false>(drop, site, (uint64_t)(r + 1) * C + c, b);
                 }
             }
             const uint32_t av[4] = {to_bf16(a.x), to_bf16(a.y), to_bf16(a.z), to_bf16(a.w)};
@@ -374,39 +332,28 @@ __global__ void __launch_bounds__(256) transpose16v_kernel(const uint16_t *__res
     if (COLSUM) {
         csum += __shfl_xor_sync(0xffffffffu, csum, 1);
         csum += __shfl_xor_sync(0xffffffffu, csum, 2);
-        if (wq == 0 && c0 + oc < C) atomicAdd(colsum_out + c0 + oc, csum);
+        if (wq == 0 && c0 + oc < nsum) atomicAdd(colsum_out + c0 + oc, csum);
     }
 }
 
-// colsum_out != nullptr: also the column sums of `in` (fp32, zeroed here).  drop != nullptr: transpose `in` (fp16, ld_in == C)
-// masked by dropout site `site`
-int transpose_to_bf16(xb_handle *h, const void *in, int R, int C, int ld_in, bool in_bf16, void *out, cudaStream_t s,
-                      float *colsum_out = nullptr, const xb_dropout *drop = nullptr, int site = 0) {
+// in (R, C) -> out (C, R) bf16 in one of the forms of TrForm.  TR_BF16_COLSUM: colsum_out[0 .. nsum) = the sums of the
+// first nsum columns (zeroed here).  TR_F16_DROP: masked by dropout site `site` of *drop.
+int transpose_to_bf16(xb_handle *h, TrForm form, const void *in, int R, int C, void *out, cudaStream_t s,
+                      float *colsum_out = nullptr, int nsum = 0, const xb_dropout *drop = nullptr, int site = 0) {
     const uint16_t *src = reinterpret_cast<const uint16_t *>(in);
     __nv_bfloat16 *dst = reinterpret_cast<__nv_bfloat16 *>(out);
     xb_stage_timer tm(h, XB_ST_TRAIN_TRANSPOSE, s);
-    if (drop && (in_bf16 || colsum_out || ld_in != C))
-        return xb_fail(h, XB_ERR_ARG, "the masked transposition takes a dense fp16 tensor and takes no column sums");
-    if (R % 8 == 0 && C % 8 == 0 && ld_in % 8 == 0 && (reinterpret_cast<uintptr_t>(in) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0) {
-        const int tiles = (R + 63) / 64, ctiles = (C + 63) / 64;
-        int slabs = (h->num_sms * 12 + ctiles - 1) / ctiles;  // ~12 CTAs per SM over the whole grid
-        if (slabs > tiles) slabs = tiles;
-        dim3 grid(ctiles, slabs);
-        if (colsum_out) XB_CUDA(h, cudaMemsetAsync(colsum_out, 0, (size_t)C * sizeof(float), s));
-        if (drop) transpose16v_kernel<false, false, true><<<grid, 256, 0, s>>>(src, R, C, ld_in, dst, nullptr, *drop, site);
-        else if (in_bf16 && colsum_out) transpose16v_kernel<true, true><<<grid, 256, 0, s>>>(src, R, C, ld_in, dst, colsum_out);
-        else if (in_bf16) transpose16v_kernel<true, false><<<grid, 256, 0, s>>>(src, R, C, ld_in, dst, nullptr);
-        else if (colsum_out) return xb_fail(h, XB_ERR_ARG, "column sums are taken of bf16 gradients only");
-        else transpose16v_kernel<false, false><<<grid, 256, 0, s>>>(src, R, C, ld_in, dst, nullptr);
-        XB_LAUNCH_CHECK(h);
-        return XB_OK;
-    }
-    if (drop) return xb_fail(h, XB_ERR_ARG, "the masked transposition needs 16-byte aligned rows");
-    dim3 grid((C + 31) / 32, (R + 31) / 32), block(32, 8);
-    if (in_bf16) transpose16_kernel<true><<<grid, block, 0, s>>>(src, R, C, ld_in, dst);
-    else transpose16_kernel<false><<<grid, block, 0, s>>>(src, R, C, ld_in, dst);
+    if (R % 8 || C % 8 || (reinterpret_cast<uintptr_t>(in) & 15) || (reinterpret_cast<uintptr_t>(out) & 15))
+        return xb_fail(h, XB_ERR_ARG, "transposition of (%d, %d): rows must be multiples of 8 and buffers 16-byte aligned", R, C);
+    const int tiles = (R + 63) / 64, ctiles = (C + 63) / 64;
+    int slabs = (h->num_sms * 12 + ctiles - 1) / ctiles;  // ~12 CTAs per SM over the whole grid
+    if (slabs > tiles) slabs = tiles;
+    if (form == TR_BF16_COLSUM) XB_CUDA(h, cudaMemsetAsync(colsum_out, 0, (size_t)nsum * sizeof(float), s));
+    auto k = form == TR_BF16_COLSUM ? transpose16v_kernel<TR_BF16_COLSUM>
+             : form == TR_F16       ? transpose16v_kernel<TR_F16>
+                                    : transpose16v_kernel<TR_F16_DROP>;
+    k<<<dim3(ctiles, slabs), 256, 0, s>>>(src, R, C, dst, colsum_out, nsum, drop ? *drop : xb_dropout(), site);
     XB_LAUNCH_CHECK(h);
-    if (colsum_out) return colsum(h, in, R, C, ld_in, colsum_out, s);
     return XB_OK;
 }
 
@@ -446,36 +393,44 @@ int gemm_bf16(xb_handle *h, int epi, const void *A, int M, int lda, const void *
 
 }  // namespace
 
+// Every buffer the workspace owns, with its size at the workspace's capacity: train_ws allocates this list and
+// xb_train_free frees it.  dpre / dpreT are not in it (aliases of DZ / DZT).
+struct ws_buffer { void **p; size_t bytes; };
+static std::vector<ws_buffer> ws_buffers(const xb_handle *h, xb_train_ws *w) {
+    const size_t TN = (size_t)w->cap_T * w->cap_N, F = XB_FEATURES, HP = h->head_rows_padded ? h->head_rows_padded : 3072;
+    const size_t NL = (size_t)w->cap_N * w->cap_T * XB_STRIDE;
+    std::vector<ws_buffer> b;
+    for (void *&p : w->x) b.push_back({&p, TN * F * 2});
+    for (void *&p : w->saved) b.push_back({&p, TN * 5 * F * 2});
+    for (void *&p : w->XT) b.push_back({&p, TN * F * 2});
+    for (void *&p : w->dy) b.push_back({&p, TN * F * 2});
+    b.insert(b.end(), {{&w->DZ, TN * XB_GATES * 2}, {&w->DZT, TN * XB_GATES * 2}, {&w->dzh, TN * HP * 2}, {&w->dzhT, TN * HP * 2},
+                       {&w->colT, TN * XB_CONV3_K * 2}, {&w->dcol, TN * XB_CONV3_K * 2},
+                       {reinterpret_cast<void **>(&w->dcstate), (size_t)w->cap_N * F * 4},
+                       {reinterpret_cast<void **>(&w->dc2), NL * XB_C2_CH * 4},
+                       {reinterpret_cast<void **>(&w->dc1), NL * 4 * 4},
+                       {&w->xd, TN * F * 2}});
+    return b;
+}
+
 void xb_train_free(xb_handle *h) {
     xb_train_ws *w = h->train;
     if (!w) return;
-    for (void *p : {w->x[0], w->x[1], w->x[2], w->x[3], w->x[4], w->x[5], w->saved[0], w->saved[1], w->saved[2], w->saved[3],
-                    w->saved[4], w->DZ, w->DZT, w->XT[0], w->XT[1], w->dy[0], w->dy[1], w->dzh, w->dzhT, w->colT, w->dcol,
-                    (void *)w->dcstate, (void *)w->dc2, (void *)w->dc1, w->xd})
-        if (p) cudaFree(p);
+    for (const ws_buffer &b : ws_buffers(h, w))
+        if (*b.p) cudaFree(*b.p);
     delete w;
     h->train = nullptr;
 }
 
-static int train_ws(xb_handle *h, int N, int T) {
+// with_xd: also the scratch copy xd, which only a forward with an active LSTM dropout site needs (kept once allocated)
+static int train_ws(xb_handle *h, int N, int T, bool with_xd) {
     if (!(h->flags & XB_FLAG_TRAIN)) return xb_fail(h, XB_ERR_STATE, "the handle was created without XB_FLAG_TRAIN");
     if (h->train && (h->train->cap_N < N || h->train->cap_T < T)) xb_train_free(h);
     if (!h->train) { h->train = new xb_train_ws(); h->train->cap_N = N; h->train->cap_T = T; }
     xb_train_ws *w = h->train;
-    const size_t TN = (size_t)w->cap_T * w->cap_N, F = XB_FEATURES, HP = h->head_rows_padded ? h->head_rows_padded : 3072;
-    const size_t L = (size_t)w->cap_T * XB_STRIDE;
-    for (int i = 0; i < 6; i++) if (int rc = alloc(h, &w->x[i], TN * F * 2)) return rc;
-    for (int i = 0; i < 5; i++) if (int rc = alloc(h, &w->saved[i], TN * 5 * F * 2)) return rc;
-    if (int rc = alloc(h, &w->DZ, TN * XB_GATES * 2)) return rc;
-    if (int rc = alloc(h, &w->DZT, TN * XB_GATES * 2)) return rc;
-    for (int i = 0; i < 2; i++) { if (int rc = alloc(h, &w->XT[i], TN * F * 2)) return rc; if (int rc = alloc(h, &w->dy[i], TN * F * 2)) return rc; }
-    if (int rc = alloc(h, &w->dzh, TN * HP * 2)) return rc;
-    if (int rc = alloc(h, &w->dzhT, TN * HP * 2)) return rc;
-    if (int rc = alloc(h, &w->colT, TN * XB_CONV3_K * 2)) return rc;
-    if (int rc = alloc(h, &w->dcol, TN * XB_CONV3_K * 2)) return rc;
-    if (int rc = alloc(h, reinterpret_cast<void **>(&w->dcstate), (size_t)w->cap_N * F * 4)) return rc;
-    if (int rc = alloc(h, reinterpret_cast<void **>(&w->dc2), (size_t)w->cap_N * L * XB_C2_CH * 4)) return rc;
-    if (int rc = alloc(h, reinterpret_cast<void **>(&w->dc1), (size_t)w->cap_N * L * 4 * 4)) return rc;
+    for (const ws_buffer &b : ws_buffers(h, w))
+        if (b.p != &w->xd || with_xd)
+            if (int rc = alloc(h, b.p, b.bytes)) return rc;
     w->dpre = w->DZ;            // conv3's (TN,768) gradients reuse the LSTM buffers (the LSTM layers are done by then)
     w->dpreT = w->DZT;
     return XB_OK;
@@ -499,13 +454,9 @@ static int encoder_fwd_train(xb_handle *h, const void *signal, int sig_dtype, in
     XB_REQUIRE(h, N % 8 == 0, "the training path needs a batch that is a multiple of 8 (16-byte TMA alignment of the time-shifted "
                               "operand views); got %d", N);
     XB_CUDA(h, cudaSetDevice(h->device));
-    if (int rc = train_ws(h, N, T)) return rc;
+    if (int rc = train_ws(h, N, T, drop.active >> 3)) return rc;    // a dropped LSTM output needs the scratch copy xd
     xb_train_ws *w = h->train;
     const size_t TNF = (size_t)T * N * XB_FEATURES;
-    if (drop.active >> 3) {         // a dropped LSTM output: the scratch copy (allocated once, kept with the workspace)
-        const size_t cap = (size_t)w->cap_T * w->cap_N * XB_FEATURES * 2;
-        if (int rc = alloc(h, &w->xd, cap)) return rc;
-    }
     w->N = N; w->T = T;
     w->drop = drop;
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
@@ -529,13 +480,16 @@ static int head_bwd(xb_handle *h, xb_train_ws *w, const float *scores, const flo
                     cudaStream_t s) {
     const int TN = w->T * w->N, F = XB_FEATURES, HP = h->head_rows_padded, S = h->C * h->NZ;
     const size_t n = (size_t)TN * HP;
-    head_bwd_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(dscores, scores, (size_t)TN, h->n_base, h->NZ, h->head_rows, HP,
-                                                              h->expand_blanks ? S : h->head_rows, h->expand_blanks,
-                                                              h->scale, reinterpret_cast<__nv_bfloat16 *>(w->dzh));
-    XB_LAUNCH_CHECK(h);
-    if (int rc = colsum(h, w->dzh, TN, h->head_rows, HP, grads[27], s)) return rc;
-    if (int rc = transpose_to_bf16(h, w->dzh, TN, HP, HP, true, w->dzhT, s)) return rc;
-    if (int rc = transpose_to_bf16(h, w->x[5], TN, F, F, false, w->XT[1], s)) return rc;
+    {
+        xb_stage_timer tm(h, XB_ST_TRAIN_HEAD_CONV, s);
+        head_bwd_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(dscores, scores, (size_t)TN, h->n_base, h->NZ, h->head_rows,
+                                                                  HP, h->expand_blanks ? S : h->head_rows, h->expand_blanks,
+                                                                  h->scale, reinterpret_cast<__nv_bfloat16 *>(w->dzh));
+        XB_LAUNCH_CHECK(h);
+    }
+    // + db = colsum dz over the head_rows real columns
+    if (int rc = transpose_to_bf16(h, TR_BF16_COLSUM, w->dzh, TN, HP, w->dzhT, s, grads[27], h->head_rows)) return rc;
+    if (int rc = transpose_to_bf16(h, TR_F16, w->x[5], TN, F, w->XT[1], s)) return rc;
     if (int rc = gemm_bf16(h, EPI_F32, w->dzhT, h->head_rows, TN, w->XT[1], F, TN, TN, grads[26], F, s)) return rc;
     return gemm_bf16(h, EPI_BF16OUT, w->dzh, TN, HP, h->head_wT, F, HP, HP, dy_out, F, s);
 }
@@ -565,12 +519,13 @@ static int lstm_layer_bwd(xb_handle *h, xb_train_ws *w, int l, const void *dy_in
     }
     }
     float *g_wih = grads[6 + 4 * l], *g_whh = grads[7 + 4 * l], *g_bih = grads[8 + 4 * l], *g_bhh = grads[9 + 4 * l];
-    if (int rc = transpose_to_bf16(h, w->DZ, TN, XB_GATES, XB_GATES, true, w->DZT, s, g_bih)) return rc;   // + db = colsum DZ
+    // + db = colsum DZ
+    if (int rc = transpose_to_bf16(h, TR_BF16_COLSUM, w->DZ, TN, XB_GATES, w->DZT, s, g_bih, XB_GATES)) return rc;
     XB_CUDA(h, cudaMemcpyAsync(g_bhh, g_bih, XB_GATES * sizeof(float), cudaMemcpyDeviceToDevice, s));
-    if (int rc = transpose_to_bf16(h, w->x[l], TN, F, F, false, w->XT[l & 1], s)) return rc;
+    if (int rc = transpose_to_bf16(h, TR_F16, w->x[l], TN, F, w->XT[l & 1], s)) return rc;
     // layer l > 0 read the dropped copy of x[l] (site l + 2): dW_ih takes that, transposed through the mask into xd
     const bool drop_in = l > 0 && drop.on(l + 2);
-    if (drop_in) { if (int rc = transpose_to_bf16(h, w->x[l], TN, F, F, false, w->xd, s, nullptr, &drop, l + 2)) return rc; }
+    if (drop_in) { if (int rc = transpose_to_bf16(h, TR_F16_DROP, w->x[l], TN, F, w->xd, s, nullptr, 0, &drop, l + 2)) return rc; }
     // dW_ih = DZ^T x_l and dW_hh = sum over the steps that had a predecessor of dz_t (x) h_prev (a time shift of N columns
     // between DZ^T and Y^T), one launch over 128 x 256 tiles (wgrad_gemm.cu)
     {
@@ -584,24 +539,42 @@ static int lstm_layer_bwd(xb_handle *h, xb_train_ws *w, int l, const void *dy_in
     return XB_OK;
 }
 
+// conv2 and conv1 backward of the stem (SIG: the signal's element type): w->dc2 -> grads[0 .. 3], through w->dc1
+template <typename SIG>
+static int conv12_bwd(xb_handle *h, xb_train_ws *w, const void *signal, float *const *grads, cudaStream_t s) {
+    const int N = w->N, L = w->T * XB_STRIDE;
+    const xb_dropout &drop = w->drop;
+    const SIG *sig = reinterpret_cast<const SIG *>(signal);
+    auto conv2 = drop.on(0) || drop.on(1) ? conv2_bwd_kernel<true, SIG> : conv2_bwd_kernel<false, SIG>;
+    conv2<<<dim3((L + 255) / 256, N), 256, 0, s>>>(sig, L, h->conv1_w, h->conv1_b, h->conv2_w, h->conv2_b, w->dc2, w->dc1,
+                                                  grads[2], grads[3], drop);
+    XB_LAUNCH_CHECK(h);
+    conv1_bwd_kernel<SIG><<<dim3(4, N), 256, 0, s>>>(sig, L, h->conv1_w, h->conv1_b, w->dc1, grads[0], grads[1]);
+    XB_LAUNCH_CHECK(h);
+    return XB_OK;
+}
+
 // convolution stem: dy_in = d x0 (T,N,768) bf16 -> grads[0 .. 5]
 static int stem_bwd(xb_handle *h, xb_train_ws *w, const void *signal, int sig_dtype, const void *dy_in, float *const *grads,
                     cudaStream_t s) {
     const int N = w->N, T = w->T, TN = T * N, F = XB_FEATURES, L = T * XB_STRIDE;
-    const xb_dropout &drop = w->drop;
-    const bool drop_stem = drop.on(0) || drop.on(1);
-    if (int rc = xb_conv12_im2col(h, signal, sig_dtype, N, L, s, &drop)) return rc;   // im2col rows of this batch into h->c2
+    if (int rc = xb_conv12_im2col(h, signal, sig_dtype, N, L, s, &w->drop)) return rc;   // im2col rows of this batch into h->c2
     CUtensorMap tmA, tmB;
     if (int rc = xb_make_tmap_2d(h, &tmA, h->c2, (uint64_t)TN, XB_CONV3_K, XB_CONV3_K)) return rc;
     if (int rc = xb_make_tmap_2d(h, &tmB, h->conv3_w, F, XB_CONV3_K, XB_CONV3_K)) return rc;
     GemmParams p;
     p.M = TN; p.N = F; p.K = XB_CONV3_K; p.bias = h->conv3_b; p.out = w->dpre; p.ldo = F; p.T = T; p.NB = N; p.dy = dy_in;
-    if (int rc = xb_gemm_launch(h, EPI_CONV3_BWD, tmA, tmB, p, s, false)) return rc;
-    if (int rc = transpose_to_bf16(h, w->dpre, TN, F, F, true, w->dpreT, s, grads[5])) return rc;       // + db3 = colsum d pre
-    if (int rc = transpose_to_bf16(h, h->c2, TN, XB_CONV3_K, XB_CONV3_K, false, w->colT, s)) return rc;
+    {
+        xb_stage_timer tm(h, XB_ST_TRAIN_HEAD_CONV, s);
+        if (int rc = xb_gemm_launch(h, EPI_CONV3_BWD, tmA, tmB, p, s, false)) return rc;
+    }
+    // + db3 = colsum d pre
+    if (int rc = transpose_to_bf16(h, TR_BF16_COLSUM, w->dpre, TN, F, w->dpreT, s, grads[5], F)) return rc;
+    if (int rc = transpose_to_bf16(h, TR_F16, h->c2, TN, XB_CONV3_K, w->colT, s)) return rc;
     // dW3 in im2col column order (768, 320): the caller drops the 16 padding columns and permutes to (768, 16, 19)
     if (int rc = gemm_bf16(h, EPI_F32, w->dpreT, F, TN, w->colT, XB_CONV3_K, TN, TN, grads[4], XB_CONV3_K, s)) return rc;
     if (int rc = gemm_bf16(h, EPI_BF16OUT, w->dpre, TN, F, h->conv3_wT, XB_CONV3_K, F, F, w->dcol, XB_CONV3_K, s)) return rc;
+    xb_stage_timer tm(h, XB_ST_TRAIN_HEAD_CONV, s);
     const size_t n2 = (size_t)N * L * XB_C2_CH;
     col2im_kernel<<<(unsigned)((n2 + 255) / 256), 256, 0, s>>>(reinterpret_cast<const __nv_bfloat16 *>(w->dcol), N, T, L, w->dc2);
     XB_LAUNCH_CHECK(h);
@@ -610,30 +583,7 @@ static int stem_bwd(xb_handle *h, xb_train_ws *w, const void *signal, int sig_dt
     XB_CUDA(h, cudaMemsetAsync(grads[3], 0, 16 * sizeof(float), s));
     XB_CUDA(h, cudaMemsetAsync(grads[0], 0, 20 * sizeof(float), s));
     XB_CUDA(h, cudaMemsetAsync(grads[1], 0, 4 * sizeof(float), s));
-    dim3 g2((L + 255) / 256, N);
-    if (sig_dtype == XB_SIG_F32) {
-        if (drop_stem)
-            conv2_bwd_kernel<true, float><<<g2, 256, 0, s>>>(reinterpret_cast<const float *>(signal), L, h->conv1_w, h->conv1_b,
-                                                             h->conv2_w, h->conv2_b, w->dc2, w->dc1, grads[2], grads[3], drop);
-        else
-            conv2_bwd_kernel<false, float><<<g2, 256, 0, s>>>(reinterpret_cast<const float *>(signal), L, h->conv1_w, h->conv1_b,
-                                                              h->conv2_w, h->conv2_b, w->dc2, w->dc1, grads[2], grads[3], drop);
-        XB_LAUNCH_CHECK(h);
-        conv1_bwd_kernel<float><<<dim3(4, N), 256, 0, s>>>(reinterpret_cast<const float *>(signal), L, h->conv1_w, h->conv1_b, w->dc1,
-                                                          grads[0], grads[1]);
-    } else {
-        if (drop_stem)
-            conv2_bwd_kernel<true, int16_t><<<g2, 256, 0, s>>>(reinterpret_cast<const int16_t *>(signal), L, h->conv1_w, h->conv1_b,
-                                                               h->conv2_w, h->conv2_b, w->dc2, w->dc1, grads[2], grads[3], drop);
-        else
-            conv2_bwd_kernel<false, int16_t><<<g2, 256, 0, s>>>(reinterpret_cast<const int16_t *>(signal), L, h->conv1_w, h->conv1_b,
-                                                                h->conv2_w, h->conv2_b, w->dc2, w->dc1, grads[2], grads[3], drop);
-        XB_LAUNCH_CHECK(h);
-        conv1_bwd_kernel<int16_t><<<dim3(4, N), 256, 0, s>>>(reinterpret_cast<const int16_t *>(signal), L, h->conv1_w, h->conv1_b,
-                                                            w->dc1, grads[0], grads[1]);
-    }
-    XB_LAUNCH_CHECK(h);
-    return XB_OK;
+    return sig_dtype == XB_SIG_F32 ? conv12_bwd<float>(h, w, signal, grads, s) : conv12_bwd<int16_t>(h, w, signal, grads, s);
 }
 
 extern "C" {
@@ -707,7 +657,7 @@ int xb_encoder_bwd_stages(xb_handle *h, int top, int bottom, const void *signal,
     } else if (top >= 1) {
         // layer top-1 reads its own output transposed, which the stage above it leaves behind in a chained backward
         const int l = top - 1;
-        if (int rc = transpose_to_bf16(h, w->x[l + 1], w->T * w->N, XB_FEATURES, XB_FEATURES, false, w->XT[(l + 1) & 1], s)) return rc;
+        if (int rc = transpose_to_bf16(h, TR_F16, w->x[l + 1], w->T * w->N, XB_FEATURES, w->XT[(l + 1) & 1], s)) return rc;
     }
     for (int k = std::min(top, 5); k >= std::max(bottom, 1); k--) {
         const int l = k - 1;

@@ -6,6 +6,7 @@
 
 #include "xb_common.cuh"
 #include "xb_gemm.cuh"
+#include "crf_lattice.cuh"
 
 thread_local std::string xb_global_err;
 
@@ -173,8 +174,7 @@ int xb_create(xb_handle **out, int device, int max_N, int max_T, int n_base, int
     if (max_N <= 0 || max_T <= 0) return xb_fail(nullptr, XB_ERR_ARG, "xb_create: max_N and max_T must be positive");
     if (!alphabet || (int)strlen(alphabet) != n_base + 1 || n_base + 1 > 15)
         return xb_fail(nullptr, XB_ERR_ARG, "xb_create: alphabet must have n_base+1 letters (blank first)");
-    int key = n_base * 10 + state_len;
-    if (!(key == 43 || key == 53 || key == 63 || key == 44 || key == 22))
+    if (!xbcrf::lattice_supported(n_base, state_len))
         return xb_fail(nullptr, XB_ERR_UNSUPPORTED, "xb_create: no kernels for n_base=%d state_len=%d", n_base, state_len);
     int ndev = 0;
     cudaError_t e = cudaGetDeviceCount(&ndev);
@@ -206,7 +206,7 @@ int xb_create(xb_handle **out, int device, int max_N, int max_T, int n_base, int
     const size_t VP = (size_t)((h->C + 31) / 32) * 32 + 4;
     TRY(dev_alloc(h, &h->alpha, (TN + max_N) * VP));
     TRY(dev_alloc(h, &h->bmax, (TN + max_N) * VP));
-    TRY(dev_alloc(h, &h->lp, (TN + max_N) * VP));
+    TRY(dev_alloc(h, &h->beta, (TN + max_N) * VP));
     TRY(dev_alloc(h, &h->logz, (size_t)max_N));
     TRY(dev_alloc(h, &h->seq_dev, TN));
     TRY(dev_alloc(h, &h->lens_dev, (size_t)max_N));
@@ -233,7 +233,7 @@ int xb_destroy(xb_handle *h) {
     cudaSetDevice(h->device);
     void *ptrs[] = {h->conv1_w, h->conv1_b, h->conv2_w, h->conv2_b, h->conv3_w, h->conv3_b, h->head_w, h->head_b, h->c2,
                     h->act0, h->act1, h->gates, h->scores, h->signal_dev, h->seq_dev, h->lens_dev,
-                    h->alpha, h->bmax, h->lp, h->logz, h->ctc_ws, h->lstm_counters};
+                    h->alpha, h->bmax, h->beta, h->logz, h->lstm_counters};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     for (void *p : {(void *)h->signal_dev2, (void *)h->seq_dev2, (void *)h->lens_dev2})
@@ -512,7 +512,7 @@ int xb_crf_posteriors_max(xb_handle *h, const float *scores, int T, int N, int32
     XB_CRF_PROLOGUE();
     XB_REQUIRE(h, edges_nt != nullptr, "edges is NULL");
     if (int rc = xb_decode_backward(h, scores, T, N, h->bmax, nullptr, 1, s)) return rc;
-    if (int rc = xb_decode_viterbi_fwd(h, scores, h->bmax, T, N, nullptr, nullptr, nullptr, nullptr, edges_nt, s)) return rc;
+    if (int rc = xb_decode_viterbi_fwd(h, scores, h->bmax, T, N, nullptr, edges_nt, s)) return rc;
     if (post) return xb_onehot_edges(h, edges_nt, T, N, h->C * h->NZ, post, s);
     return XB_OK;
 }
@@ -527,7 +527,7 @@ int xb_crf_viterbi(xb_handle *h, const float *scores, int T, int N, int8_t *labe
     XB_CRF_PROLOGUE();
     XB_REQUIRE(h, labels_nt != nullptr, "labels is NULL");
     if (int rc = xb_decode_backward(h, scores, T, N, h->bmax, nullptr, 1, s)) return rc;
-    return xb_decode_viterbi_fwd(h, scores, h->bmax, T, N, labels_nt, nullptr, nullptr, nullptr, nullptr, s);
+    return xb_decode_viterbi_fwd(h, scores, h->bmax, T, N, labels_nt, nullptr, s);
 }
 
 int xb_crf_decode(xb_handle *h, const float *scores, int T, int N, int8_t *seq, int8_t *qstring, int32_t *lens,
@@ -542,8 +542,8 @@ int xb_crf_beam_search(xb_handle *h, const float *scores, int T, int N, int beam
                        int8_t *qstring, int8_t *moves, int32_t *lens, void *stream) {
     XB_CRF_PROLOGUE();
     XB_REQUIRE(h, seq != nullptr && lens != nullptr, "seq / lens is NULL");
-    if (int rc = xb_decode_backward(h, scores, T, N, nullptr, h->lp, 2, s)) return rc;
-    return xb_beam_search_impl(h, scores, h->lp, T, N, beam_width, beam_cut, seq, qstring, moves, lens, s);
+    if (int rc = xb_decode_backward(h, scores, T, N, nullptr, h->beta, 2, s)) return rc;
+    return xb_beam_search_impl(h, scores, h->beta, T, N, beam_width, beam_cut, seq, qstring, moves, lens, s);
 }
 
 int xb_crf_decode_exp(xb_handle *h, const float *scores, int T, int N, int8_t *seq, int8_t *qstring, int32_t *lens,

@@ -79,12 +79,11 @@ struct xb_handle {
 
     // decode workspace
     // three (max_T+1, max_N, VP) state-vector buffers, VP = round_up(C, 32) + 4 floats (16-byte aligned rows for the
-    // bulk-copy ring of crf_decode_lin.cu: a_hat, bm_hat, b_hat); the log-domain scans use alpha / bmax with pitch C
-    float *alpha = nullptr;
-    float *bmax = nullptr;
-    float *lp = nullptr;
+    // bulk-copy ring of crf_decode_lin.cu); the log-domain scans use them with pitch C
+    float *alpha = nullptr;      // linear decode: a_hat;  log-domain scans: alpha
+    float *bmax = nullptr;       // linear decode: bm_hat; log-domain scans: Max-semiring beta
+    float *beta = nullptr;       // linear decode: b_hat;  beam search: Log-semiring beta
     float *logz = nullptr;       // (max_N)
-    float *ctc_ws = nullptr;
     int *lstm_counters = nullptr; // per-group step counters of the persistent LSTM kernel
 
     // training (XB_FLAG_TRAIN; workspace allocated by the first xb_encoder_fwd_train, see train_bwd.cu)
@@ -171,6 +170,5 @@ int xb_decode_alpha(xb_handle *h, const float *scores, int T, int N, float *alph
 int xb_decode_backward(xb_handle *h, const float *scores, int T, int N, float *bmax, float *beta, int mode, cudaStream_t s);
 int xb_decode_lin(xb_handle *h, const float *scores, int lin_input, int T, int N, int8_t *labels, int8_t *seq, int8_t *qs,
                   int32_t *lens, float *post, cudaStream_t s);
-int xb_score_exp_launch(xb_handle *h, const float *in, float *out, size_t n, cudaStream_t s);
-int xb_decode_viterbi_fwd(xb_handle *h, const float *lp, const float *bmax, int T, int N, int8_t *labels,
-                          int8_t *seq, int8_t *qstring, int32_t *lens, int32_t *edges, cudaStream_t s);
+int xb_decode_viterbi_fwd(xb_handle *h, const float *scores, const float *bmax, int T, int N, int8_t *labels, int32_t *edges,
+                          cudaStream_t s);
