@@ -166,7 +166,10 @@ int xb_basecall_chunks(xb_handle *h, const void *signal, int sig_dtype, int N, i
                        int32_t *lens, void *stream);
 
 /* CTC_CRF.ctc_loss(reduction='none') forward (crf/model.py:118-131): targets (N, Lmax) int32 1-based
- * 0-padded, lengths (N) int32 -> loss (N) fp32 = -logz / length.  normalise as in the reference. */
+ * 0-padded, lengths (N) int32 -> loss (N) fp32 = -logz / length.  normalise as in the reference.
+ * 1 <= Lmax - state_len + 1 <= 1024, else XB_ERR_ARG before anything is launched (both directions).  A target no
+ * alignment reaches (length < state_len, length > Lmax, or more moves than steps) scores seqdist's zero:
+ * loss = 1e38 / length, and the backward below has no P_target term for it. */
 int xb_ctc_crf_loss_fwd(xb_handle *h, const float *scores, int T, int N, const int32_t *targets,
                         int Lmax, const int32_t *lengths, int normalise, float *loss, void *stream);
 

@@ -228,11 +228,12 @@ class CRF:
         """crf/model.py:48-49."""
         return scores - self.logZ(scores)[:, None] / len(scores)
 
-    def prepare_ctc_scores(self, scores, targets):
-        """crf/model.py:102-116.  targets are 1-based labels, 0-padded."""
+    def prepare_ctc_scores(self, scores, targets, dtype=torch.float32):
+        """crf/model.py:102-116.  targets are 1-based labels, 0-padded.  The reference casts to float32; the float64
+        references pass dtype=torch.float64."""
         tg = torch.clamp(targets - 1, 0)
         T = scores.shape[0]
-        scores = scores.to(torch.float32)
+        scores = scores.to(dtype)
         n = tg.size(1) - (self.state_len - 1)
         state = torch.zeros_like(tg[:, :n])
         for i in range(self.state_len):

@@ -1,5 +1,6 @@
-"""float64 references of the three stages of the encoder backward (xb_encoder_bwd_stages): the CRF head, one LSTM layer
-and the convolution stem.  TEST INFRASTRUCTURE ONLY (see oracle/__init__.py).
+"""float64 references of the training gradient one part at a time: the CTC-CRF loss and its gradient w.r.t. the scores
+(xb_ctc_crf_loss_fwd / _bwd), and the three stages of the encoder backward (xb_encoder_bwd_stages): the CRF head, one
+LSTM layer and the convolution stem.  TEST INFRASTRUCTURE ONLY (see oracle/__init__.py).
 
 Every function is plain torch and runs on whatever device its inputs live on: the GPU tests run them there, because a
 T = 800 LSTM layer in float64 on the CPU takes minutes.  Inputs are the stage's exact 16-bit inputs as float64 and the
@@ -32,6 +33,70 @@ def held_bwd(w):
 def _grads(out, cot, inputs):
     gs = torch.autograd.grad(out, inputs, cot, allow_unused=True)
     return [torch.zeros_like(i) if g is None else g for i, g in zip(inputs, gs)]
+
+
+# ----------------------------------------------------------------------------------------------------------- CTC-CRF loss
+def ctc_loss_backward(scores, targets, lengths, grad_loss, n_base, normalise=True, state_len=3):
+    """CTC_CRF.ctc_loss(reduction='none') (bonito/crf/model.py:102-131) and its gradient, in float64.
+
+    scores (T, N, S = n_base^state_len * (n_base + 1)), targets (N, Lmax) 1-based labels, lengths (N,), grad_loss (N,)
+    -> (loss (N,), dscores (T, N, S)): loss[n] = -logZ_n / lengths[n], logZ_n the log-sum over the alignments of target n
+    (of the scores less logZ / T with normalise), and dscores = d(sum_n grad_loss[n] * loss[n]) / d scores in the closed
+    form (P_den - P_num) * grad_loss / length: P_den the edge posteriors of the full lattice (only with normalise), P_num
+    those of the target's alignment lattice, from explicit alpha / beta recursions over the target positions.
+
+    A target no alignment reaches follows the kernels' contract, which is seqdist's semiring zero (-1e38): its loss is
+    1e38 / length and it has no P_num term.  That is the case for length < state_len (no end position), length > Lmax,
+    and more moves than steps (length - state_len > T).  Autograd through the reference would instead spread a numerator
+    over paths of score ~-1e38, and index the end position with a negative number when length < state_len."""
+    dev = scores.device
+    T, N, S = scores.shape
+    NZ = n_base + 1
+    crf = bo.CRF(state_len, range(NZ))
+    crf.idx, crf.src_edges, crf.src_dst = (t.to(dev) for t in (crf.idx, crf.src_edges, crf.src_dst))
+    s = scores.to(F64)
+    p_den = None
+    if normalise:
+        p_den = crf.posteriors(s)
+        s = crf.normalise(s)
+    # the alignment lattice (crf/model.py:102-116): stay edge of every position and the move edge into positions 1..
+    tg = targets.to(dev, torch.int64).clamp_min(1) - 1
+    npos = tg.shape[1] - (state_len - 1)
+    state = torch.zeros_like(tg[:, :npos])
+    for i in range(state_len):
+        state = state * n_base + tg[:, i:npos + i]
+    stay_idx = state * NZ
+    move_idx = stay_idx[:, 1:] + tg[:, :npos - 1] + 1
+    stay = s.gather(2, stay_idx.expand(T, -1, -1))
+    move = s.gather(2, move_idx.expand(T, -1, -1))
+    alpha = s.new_full((T + 1, N, npos), bo.NEG)
+    alpha[0, :, 0] = 0.0
+    for t in range(T):
+        a = stay[t] + alpha[t]
+        a[:, 1:] = torch.logaddexp(a[:, 1:], move[t] + alpha[t, :, :-1])
+        alpha[t + 1] = a
+    length = lengths.to(dev, torch.int64)
+    last = length - state_len
+    reach = (last >= 0) & (last < npos)
+    end = last.clamp(0, npos - 1)
+    z = torch.where(reach, alpha[T, torch.arange(N, device=dev), end], torch.full_like(alpha[T, :, 0], bo.NEG))
+    feasible = reach & (z > -1e37)
+    loss = -z / length
+    beta = s.new_full((T + 1, N, npos), bo.NEG)
+    beta[T, torch.arange(N, device=dev)[feasible], end[feasible]] = 0.0
+    for t in range(T - 1, -1, -1):
+        b = stay[t] + beta[t + 1]
+        b[:, :-1] = torch.logaddexp(b[:, :-1], move[t] + beta[t + 1, :, 1:])
+        beta[t] = b
+    zf = torch.where(feasible, z, 0.0)[:, None]
+    keep = feasible[:, None]
+    p_stay = torch.where(keep, torch.exp(alpha[:-1] + stay + beta[1:] - zf), 0.0)
+    p_move = torch.where(keep, torch.exp(alpha[:-1, :, :-1] + move + beta[1:, :, 1:] - zf), 0.0)
+    p_num = s.new_zeros(T, N, S)
+    p_num.scatter_add_(2, stay_idx.expand(T, -1, -1), p_stay)
+    p_num.scatter_add_(2, move_idx.expand(T, -1, -1), p_move)
+    d = -p_num if p_den is None else p_den - p_num
+    return loss, d * (grad_loss.to(dev, F64) / length)[:, None]
 
 
 # ----------------------------------------------------------------------------------------------------------- CRF head

@@ -322,7 +322,7 @@ int xb_ctc_loss_impl(xb_handle *h, const float *scores, int T, int N, const int3
     return XB_OK;
 }
 
-// grad (T, N, S) must hold the Log posteriors of `scores` on entry when normalise != 0 (xb_ctc_crf_loss_bwd puts them there).
+// Every argument is checked before the first launch, so a refused call leaves `grad` and the handle's logZ untouched.
 int xb_ctc_loss_bwd_impl(xb_handle *h, const float *scores, int T, int N, const int32_t *targets, int Lmax,
                          const int32_t *lengths, int normalise, const float *grad_loss, float *alpha_ws, float *grad,
                          cudaStream_t s) {
@@ -332,6 +332,10 @@ int xb_ctc_loss_bwd_impl(xb_handle *h, const float *scores, int T, int N, const 
     int NT = ((npos + 31) / 32) * 32;
     if (NT * 4 < S) NT = ((S + 127) / 128) * 32;      // the kernel keeps a score row in four registers per thread
     XB_REQUIRE(h, NT <= 1024, "score rows of %d elements are not supported by the loss backward", S);
+    if (normalise) {       // logZ (for the shift) and the posteriors of the full lattice, straight into grad
+        if (int rc = xb_decode_lin(h, scores, 0, T, N, nullptr, nullptr, nullptr, nullptr, grad, s)) return rc;
+        if (int rc = xb_decode_alpha(h, scores, T, N, nullptr, h->logz, 0, s)) return rc;
+    }
     size_t smem = sizeof(float) * (3 * NT + 1 + 2 * S);
     if (smem > 48 * 1024)
         XB_CUDA(h, cudaFuncSetAttribute(ctc_simple_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));

@@ -565,10 +565,6 @@ int xb_ctc_crf_loss_bwd(xb_handle *h, const float *scores, int T, int N, const i
                         float *grad_scores, void *stream) {
     XB_CRF_PROLOGUE();
     XB_REQUIRE(h, targets && lengths && grad_loss && alpha_ws && grad_scores, "NULL buffer");
-    if (normalise) {       // logZ (for the shift) and the posteriors of the full lattice, straight into grad_scores
-        if (int rc = xb_decode_lin(h, scores, 0, T, N, nullptr, nullptr, nullptr, nullptr, grad_scores, s)) return rc;
-        if (int rc = xb_decode_alpha(h, scores, T, N, nullptr, h->logz, 0, s)) return rc;
-    }
     return xb_ctc_loss_bwd_impl(h, scores, T, N, targets, Lmax, lengths, normalise, grad_loss, alpha_ws, grad_scores, s);
 }
 
