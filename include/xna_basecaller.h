@@ -271,7 +271,8 @@ int xb_preprocess_reads(xb_handle *h, const int16_t *raw, const int64_t *read_of
 
 /* crf.basecall.compute_scores end to end with HOST buffers (crf/basecall.py:27-82): H2D of the
  * chunk batch, encoder, decode, D2H of the packed sequences; synchronises.  signal_host (N, L) fp32,
- * seq_host (N, T) int8, lens_host (N).  Pinned host memory makes the copies asynchronous. */
+ * seq_host (N, T) int8, lens_host (N).  Pinned host memory makes the copies asynchronous.  The same as
+ * xb_compute_scores_submit into slot 0 followed by xb_compute_scores_wait(h, 0). */
 int xb_compute_scores_host(xb_handle *h, const float *signal_host, int N, int L, int8_t *seq_host,
                            int32_t *lens_host, void *stream);
 

@@ -253,10 +253,14 @@ def test_batch_position_independence_odd_sizes():
 
 
 def test_pipelined_host_entry_points_match_the_blocking_one(enc5):
-    """xb_compute_scores_submit / _wait over five different batches in two slots == xb_compute_scores_host per batch."""
+    """xb_compute_scores_submit / _wait over five different batches in two slots == xb_basecall_chunks on device copies of
+    the same batches."""
     h, _ = enc5
     batches = [synthetic_signal(40 + i, 3, 500)[:, 0, :].contiguous().pin_memory() for i in range(5)]
-    want = [tuple(t.clone() for t in h.compute_scores_host(b)) for b in batches]
+    want = []
+    for b in batches:
+        seq, _, lens = h.basecall_chunks(b.cuda())
+        want.append((seq.cpu(), lens.cpu()))
     seqs = [torch.empty(3, 100, dtype=torch.int8).pin_memory() for _ in range(2)]
     lens = [torch.empty(3, dtype=torch.int32).pin_memory() for _ in range(2)]
     got = []

@@ -1,9 +1,9 @@
 """CRF basecalling with the reference's call surface (ub-bonito/bonito/crf/basecall.py): stitch_results
 (:15-24), compute_scores (:27-82, Viterbi branch), apply_stride_to_moves (:85-93), basecall (:96-119).
 
-compute_scores is one C-ABI call with HOST buffers (xb_compute_scores_host): pinned H2D of the chunk batch,
-fused stem, five persistent LSTM layers, CRF head, posteriors, max-marginal Viterbi and left-packing on the
-GPU, D2H of the packed (N, T) int8 letters and their lengths.  The Python loops of the reference (ord() per
+compute_scores runs a host batch through the host-buffer C ABI (xb_compute_scores_submit / _wait in slot 0): pinned H2D
+of the chunk batch, fused stem, five persistent LSTM layers, CRF head, posteriors, max-marginal Viterbi and left-packing
+on the GPU, D2H of the packed (N, T) int8 letters and their lengths.  The Python loops of the reference (ord() per
 base, per-row padding) are gone; the returned dict has the same keys, dtypes and contents.
 """
 import numpy as np
@@ -48,41 +48,25 @@ def compute_scores(model, batch, beam_width=32, beam_cut=100.0, scale=1.0, offse
             scores = model.seqdist.reverse_complement(scores)
         seq, qs, moves, _ = model.seqdist.beam_search(scores, beam_width=beam_width, beam_cut=beam_cut)
         return {'qstring': qs.cpu(), 'sequence': seq.cpu(), 'moves': moves.cpu().numpy()}
-    if reverse or batch.device.type != 'cpu':
-        # reverse complement permutes the score tensor between encoder and decode: two device calls
-        with torch.no_grad():
-            scores = model(batch.to(device))
-        if reverse:
-            scores = model.seqdist.reverse_complement(scores)
-        seq, qs, lens = model.seqdist.decode_packed(scores)
-        sequence, qstring = seq.cpu(), qs.cpu()
-    else:
-        eng = model.seqdist.engine
-        stem = model.encoder._stem()
-        if stem is None:
-            raise RuntimeError('compute_scores needs the sup@v3.3 encoder layout')
-        h = eng.get(device, N, T, bf16=next(model.parameters()).dtype == torch.bfloat16)
-        model.encoder.sync_weights(h)
-        staged = _pinned(model, 'signal', (N, L), torch.float32)
-        staged.copy_(batch[:, 0, :])
-        sequence = torch.empty(N, T, dtype=torch.int8)
-        lens = torch.empty(N, dtype=torch.int32)
-        seq_pin, lens_pin = _pinned(model, 'seq', (N, T), torch.int8), _pinned(model, 'lens', (N,), torch.int32)
-        h.compute_scores_host(staged, seq_pin, lens_pin)
-        sequence.copy_(seq_pin)
-        lens.copy_(lens_pin)
-        qstring = torch.where(sequence != 0, torch.tensor(ord('O'), dtype=torch.int8), torch.tensor(0, dtype=torch.int8))
+    if not reverse and batch.device.type == 'cpu':
+        return _collect_scores(*_submit_scores(model, batch, 0))
+    # reverse complement permutes the score tensor between encoder and decode: two device calls
+    with torch.no_grad():
+        scores = model(batch.to(device))
+    if reverse:
+        scores = model.seqdist.reverse_complement(scores)
+    seq, qs, lens = model.seqdist.decode_packed(scores)
     return {
-        'qstring': qstring,
-        'sequence': sequence,
+        'qstring': qs.cpu(),
+        'sequence': seq.cpu(),
         'moves': np.zeros((N, T), dtype=bool),
     }
 
 
 def _submit_scores(model, batch, slot):
-    """Pipelined half of compute_scores: stage the batch in the slot's pinned buffer and enqueue it."""
+    """Host-buffer half of compute_scores: stage the batch in the slot's pinned buffer and enqueue it."""
     if not model.encoder[-1].expand_blanks or model.encoder._stem() is None:
-        raise RuntimeError('the pipelined path needs the sup@v3.3 encoder layout with expand_blanks')
+        raise RuntimeError('the host-buffer path needs the sup@v3.3 encoder layout with expand_blanks')
     device = next(model.parameters()).device
     if device.type == 'cuda':
         torch.cuda.set_device(device)

@@ -217,7 +217,7 @@ int xb_beam_search_impl(xb_handle *h, const float *scores, const float *beta, in
     a.seq = seq; a.qstring = qstring; a.moves = moves; a.lens = lens;
     for (int i = 0; i < 16; i++) a.abc.ch[i] = h->alphabet[i];
     const size_t sm = 2 * BW_MAX * (4 + 4 + 8) + NT_BEAM * (4 + 4 + 4 + 4 + 8) + 16 + BW_MAX * 4 + (size_t)T * BW_MAX + 2 * (size_t)T + 16;
-    if (sm > 48 * 1024) XB_CUDA(h, cudaFuncSetAttribute(beam_search_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+    if (int rc = xb_smem_attr(h, beam_search_kernel, sm)) return rc;
     XB_REQUIRE(h, sm <= 227 * 1024, "T=%d is too long for the beam search's shared-memory traceback", T);
     beam_search_kernel<<<N, NT_BEAM, sm, s>>>(a);
     XB_LAUNCH_CHECK(h);

@@ -232,18 +232,18 @@ int xb_conv3_launch(xb_handle *h, const void *col, const void *w3, const float *
     const uint64_t M = (uint64_t)N * T;
     CUtensorMap tmA, tmB, tmO;
     if (int rc = xb_make_tmap_2d(h, &tmA, col, M, XB_CONV3_K, XB_CONV3_K)) return rc;
-    if (int rc = xb_make_tmap_2d_box(h, &tmB, w3, XB_FEATURES, XB_CONV3_K, XB_CONV3_K, BK, BN, 1)) return rc;
+    {
+        const uint64_t dims[2] = {XB_CONV3_K, XB_FEATURES}, st[1] = {XB_CONV3_K * 2};
+        const uint32_t box[2] = {BK, BN};
+        if (int rc = xb_make_tmap_nd(h, &tmB, w3, 2, 2, dims, st, box, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
+    }
     {
         const uint64_t dims[3] = {XB_FEATURES, (uint64_t)T, (uint64_t)N};
         const uint64_t st[2] = {(uint64_t)N * XB_FEATURES * 2, XB_FEATURES * 2};
         const uint32_t box[3] = {64, 32, 1};
-        if (int rc = xb_make_tmap_nd(h, &tmO, out_tnc, 3, 2, dims, st, box)) return rc;
+        if (int rc = xb_make_tmap_nd(h, &tmO, out_tnc, 3, 2, dims, st, box, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
     }
-    static bool configured[64] = {};
-    if (!configured[h->device & 63]) {
-        XB_CUDA(h, cudaFuncSetAttribute(conv3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-        configured[h->device & 63] = true;
-    }
+    if (int rc = xb_smem_attr(h, conv3_kernel, SMEM_BYTES)) return rc;
     Conv3Params p;
     p.M = (int)M; p.T = T; p.NB = N; p.bias = bias; p.col = col; p.out = reinterpret_cast<uint16_t *>(out_tnc);
     const int ntiles = (int)((M + BM - 1) / BM);

@@ -271,11 +271,11 @@ int alpha_impl(Lat<NB, SL>, xb_handle *h, const float *scores, int T, int N, flo
     size_t sm = smem_alpha<NB, SL>();
     if (use_max) {
         auto k = crf_alpha_kernel<NB, SL, true>;
-        if (int rc = set_smem(h, k, sm)) return rc;
+        if (int rc = xb_smem_attr(h, k, sm)) return rc;
         k<<<N, L::NT, sm, s>>>(scores, T, N, alpha, logz);
     } else {
         auto k = crf_alpha_kernel<NB, SL, false>;
-        if (int rc = set_smem(h, k, sm)) return rc;
+        if (int rc = xb_smem_attr(h, k, sm)) return rc;
         k<<<N, L::NT, sm, s>>>(scores, T, N, alpha, logz);
     }
     XB_LAUNCH_CHECK(h);
@@ -288,12 +288,12 @@ int backward_impl(Lat<NB, SL>, xb_handle *h, const float *scores, int T, int N, 
     if (mode == 1) {
         auto k = crf_bscan_kernel<NB, SL, true>;
         size_t sm = smem_bscan<NB, SL>();
-        if (int rc = set_smem(h, k, sm)) return rc;
+        if (int rc = xb_smem_attr(h, k, sm)) return rc;
         k<<<N, L::NT, sm, s>>>(scores, T, N, bmax);
     } else {
         auto k = crf_bscan_kernel<NB, SL, false>;
         size_t sm = smem_bscan<NB, SL>();
-        if (int rc = set_smem(h, k, sm)) return rc;
+        if (int rc = xb_smem_attr(h, k, sm)) return rc;
         k<<<N, L::NT, sm, s>>>(scores, T, N, beta);
     }
     XB_LAUNCH_CHECK(h);
@@ -305,7 +305,7 @@ int vit_impl(Lat<NB, SL>, xb_handle *h, const float *scores, const float *bmax, 
     using L = Lat<NB, SL>;
     auto k = crf_viterbi_fwd_kernel<NB, SL>;
     size_t sm = smem_vit<NB, SL>();
-    if (int rc = set_smem(h, k, sm)) return rc;
+    if (int rc = xb_smem_attr(h, k, sm)) return rc;
     k<<<N, L::NT, sm, s>>>(scores, bmax, T, N, labels, edges);
     XB_LAUNCH_CHECK(h);
     return XB_OK;

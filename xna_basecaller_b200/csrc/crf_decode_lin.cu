@@ -478,7 +478,7 @@ int lin_impl(Lat<NB, SL>, xb_handle *h, const float *scores, int T, int N, int8_
         xb_stage_timer tm(h, XB_ST_CRF_ALPHA, s);
         auto k = crf_lin_alpha_kernel<NB, SL, LIN>;
         const size_t sm = sizeof(float) * (L::D * R::ROWF + 2 * L::NT + 2 * L::W + 2) + 16 * L::D;
-        if (int rc = set_smem(h, k, sm)) return rc;
+        if (int rc = xb_smem_attr(h, k, sm)) return rc;
         k<<<N, NTT, sm, s>>>(scores, T, N, alpha);
         XB_LAUNCH_CHECK(h);
     }
@@ -486,7 +486,7 @@ int lin_impl(Lat<NB, SL>, xb_handle *h, const float *scores, int T, int N, int8_
         xb_stage_timer tm(h, XB_ST_CRF_BACKWARD, s);
         auto k = crf_lin_backward_kernel<NB, SL, LIN>;
         const size_t sm = sizeof(float) * (L::D * R::ROWF + L::D * R::VP + 4 * L::NT + 6 * L::W + 2) + 16 * L::D;
-        if (int rc = set_smem(h, k, sm)) return rc;
+        if (int rc = xb_smem_attr(h, k, sm)) return rc;
         k<<<N, NTT, sm, s>>>(scores, alpha, T, N, beta, bmax);
         XB_LAUNCH_CHECK(h);
     }
@@ -498,11 +498,11 @@ int lin_impl(Lat<NB, SL>, xb_handle *h, const float *scores, int T, int N, int8_
     if (post) {
         auto k = crf_lin_viterbi_kernel<NB, SL, LIN, true>;
         const size_t smp = sm + (L::S >= 1024 ? 2 * sizeof(float) * L::S : 0);        // + two staged posterior rows (see PSTAGE)
-        if (int rc = set_smem(h, k, smp)) return rc;
+        if (int rc = xb_smem_attr(h, k, smp)) return rc;
         k<<<N, NTT, smp, s>>>(scores, alpha, beta, bmax, T, N, labels, seq, qs, lens, post, abc);
     } else {
         auto k = crf_lin_viterbi_kernel<NB, SL, LIN, false>;
-        if (int rc = set_smem(h, k, sm)) return rc;
+        if (int rc = xb_smem_attr(h, k, sm)) return rc;
         k<<<N, NTT, sm, s>>>(scores, alpha, beta, bmax, T, N, labels, seq, qs, lens, nullptr, abc);
     }
     XB_LAUNCH_CHECK(h);

@@ -44,11 +44,6 @@ template <typename F> int lattice_dispatch(xb_handle *h, F &&f) {
     });
 }
 
-template <typename K> int set_smem(xb_handle *h, K kernel, size_t bytes) {
-    if (bytes > 48 * 1024) XB_CUDA(h, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    return XB_OK;
-}
-
 __device__ __forceinline__ void cp_async4(float *dst, const float *src) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"((uint32_t)__cvta_generic_to_shared(dst)), "l"(src));
 }

@@ -196,14 +196,8 @@ typedef CUresult (*encode_tiled_fn)(CUtensorMap *, CUtensorMapDataType, cuuint32
 
 }  // namespace
 
-// 2-D K-major tensor map: rows x K 16-bit elements, row pitch ld elements, box 64 x 128, 128B swizzle.
-int xb_make_tmap_2d(xb_handle *h, CUtensorMap *out, const void *base, uint64_t rows, uint64_t K, uint64_t ld) {
-    return xb_make_tmap_2d_box(h, out, base, rows, K, ld, BK, BM, 1);
-}
-
-// general form: box_inner x box_rows elements; swizzle128 = 1 -> CU_TENSOR_MAP_SWIZZLE_128B (box_inner must be 64)
-int xb_make_tmap_2d_box(xb_handle *h, CUtensorMap *out, const void *base, uint64_t rows, uint64_t K, uint64_t ld,
-                        uint32_t box_inner, uint32_t box_rows, int swizzle128) {
+int xb_make_tmap_nd(xb_handle *h, CUtensorMap *out, const void *base, int rank, int elem_bytes, const uint64_t *dims,
+                    const uint64_t *strides_bytes, const uint32_t *box, CUtensorMapSwizzle swizzle) {
     if (!h->encode_tiled) {
         void *fn = nullptr;
         cudaDriverEntryPointQueryResult qres;
@@ -212,69 +206,30 @@ int xb_make_tmap_2d_box(xb_handle *h, CUtensorMap *out, const void *base, uint64
             return xb_fail(h, XB_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available");
         h->encode_tiled = fn;
     }
-    cuuint64_t dims[2] = {K, rows};
-    cuuint64_t strides[1] = {ld * 2};
-    cuuint32_t box[2] = {box_inner, box_rows};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = reinterpret_cast<encode_tiled_fn>(h->encode_tiled)(
-        out, CU_TENSOR_MAP_DATA_TYPE_FLOAT16 /* 16-bit payload; the element type only matters for OOB fill */, 2, const_cast<void *>(base), dims,
-        strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE,
-        CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return xb_fail(h, XB_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
-    return XB_OK;
-}
-
-// rank-n form (n <= 5): dims / box in elements (innermost first), strides in BYTES for dimensions 1 .. n-1, 128B swizzle
-// (the innermost box extent must span 128 bytes); elem_bytes 2 (16-bit payload) or 4 (fp32)
-int xb_make_tmap_nd(xb_handle *h, CUtensorMap *out, const void *base, int rank, int elem_bytes, const uint64_t *dims,
-                    const uint64_t *strides_bytes, const uint32_t *box) {
-    if (!h->encode_tiled) {
-        CUtensorMap tmp;
-        if (int rc = xb_make_tmap_2d(h, &tmp, base, 128, 64, 64)) return rc;        // resolves the entry point
-    }
     if (rank < 2 || rank > 5 || (elem_bytes != 2 && elem_bytes != 4)) return xb_fail(h, XB_ERR_ARG, "tensor map rank %d / element size %d", rank, elem_bytes);
     cuuint64_t d[5], st[4];
     cuuint32_t bx[5], es[5];
     for (int i = 0; i < rank; i++) { d[i] = dims[i]; bx[i] = box[i]; es[i] = 1; }
     for (int i = 0; i + 1 < rank; i++) st[i] = strides_bytes[i];
     CUresult r = reinterpret_cast<encode_tiled_fn>(h->encode_tiled)(
-        out, elem_bytes == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, (cuuint32_t)rank,
-        const_cast<void *>(base), d, st, bx, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+        out, elem_bytes == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 /* 16-bit payload; the element type only matters for OOB fill */
+                             : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, (cuuint32_t)rank,
+        const_cast<void *>(base), d, st, bx, es, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle,
         CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return xb_fail(h, XB_ERR_CUDA, "cuTensorMapEncodeTiled (rank %d) failed with CUresult %d", rank, (int)r);
     return XB_OK;
 }
 
-// 3-D view of a (rows, 768) 16-bit activation matrix for the persistent LSTM: dims {64 k, rows, 12 k-blocks},
-// strides {1536 B, 128 B}, box {64, box_rows, box_kblocks}, 128B swizzle: one TMA lands box_kblocks K-major
-// [box_rows x 128 B] tiles.
-int xb_make_tmap_hview(xb_handle *h, CUtensorMap *out, const void *base, uint64_t rows, uint32_t box_rows,
-                       uint32_t box_kblocks) {
-    if (!h->encode_tiled) {
-        CUtensorMap tmp;
-        if (int rc = xb_make_tmap_2d(h, &tmp, base, rows, XB_FEATURES, XB_FEATURES)) return rc;   // resolves the entry point
-    }
-    cuuint64_t dims[3] = {64, rows, XB_FEATURES / 64};
-    cuuint64_t strides[2] = {XB_FEATURES * 2, 128};
-    cuuint32_t box[3] = {64, box_rows, box_kblocks};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = reinterpret_cast<encode_tiled_fn>(h->encode_tiled)(
-        out, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void *>(base), dims,
-        strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return xb_fail(h, XB_ERR_CUDA, "cuTensorMapEncodeTiled (3-D h view) failed with CUresult %d", (int)r);
-    return XB_OK;
+int xb_make_tmap_2d(xb_handle *h, CUtensorMap *out, const void *base, uint64_t rows, uint64_t K, uint64_t ld) {
+    const uint64_t dims[2] = {K, rows}, strides[1] = {ld * 2};
+    const uint32_t box[2] = {BK, BM};
+    return xb_make_tmap_nd(h, out, base, 2, 2, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
 template <bool BF16, int EPI>
 static int launch_one(xb_handle *h, const CUtensorMap &tmA, const CUtensorMap &tmB, const GemmParams &p, cudaStream_t s) {
     auto k = gemm_tc_kernel<BF16, EPI>;
-    static bool configured[64] = {};   // per instantiation and device (function attributes live in the context)
-    if (!configured[h->device & 63]) {
-        XB_CUDA(h, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-        configured[h->device & 63] = true;
-    }
+    if (int rc = xb_smem_attr(h, k, SMEM_BYTES)) return rc;
     dim3 grid((p.N + BN - 1) / BN, (p.M + BM - 1) / BM, (EPI == EPI_F32 && p.split_k > 1) ? p.split_k : 1);
     k<<<grid, 256, SMEM_BYTES, s>>>(tmA, tmB, p);
     XB_LAUNCH_CHECK(h);

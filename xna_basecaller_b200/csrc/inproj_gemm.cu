@@ -394,19 +394,21 @@ inproj_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ C
 
 template <int EPI>
 static int ip_launch(xb_handle *h, const void *w, int w_rows, IPParams p, cudaStream_t s) {
+    // (rows, 768) 16-bit as {64 k, rows, 12 k-blocks}: one TMA lands box_kblocks K-major [box_rows x 128 B] tiles
+    auto hview = [h](CUtensorMap *out, const void *base, uint64_t rows, uint32_t box_rows, uint32_t box_kblocks) {
+        const uint64_t dims[3] = {64, rows, XB_FEATURES / 64}, st[2] = {XB_FEATURES * 2, 128};
+        const uint32_t box[3] = {64, box_rows, box_kblocks};
+        return xb_make_tmap_nd(h, out, base, 3, 2, dims, st, box, CU_TENSOR_MAP_SWIZZLE_128B);
+    };
     CUtensorMap tmW, tmX;
-    if (int rc = xb_make_tmap_hview(h, &tmW, w, w_rows, BNI, KPS)) return rc;
-    if (int rc = xb_make_tmap_hview(h, &tmX, p.x, (uint64_t)p.M, BM, 2)) return rc;
+    if (int rc = hview(&tmW, w, w_rows, BNI, KPS)) return rc;
+    if (int rc = hview(&tmX, p.x, (uint64_t)p.M, BM, 2)) return rc;
     p.NT = w_rows / BNI;
     const int ntiles = (p.M + BM - 1) / BM;
     const int grid = ntiles < h->num_sms ? ntiles : h->num_sms;
     constexpr int SMEM_BYTES = IPCfg<EPI>::SMEM_BYTES;
     auto kernel = inproj_kernel<EPI>;
-    static bool configured[64] = {};      // per device: function attributes live in the device's context
-    if (!configured[h->device & 63]) {
-        XB_CUDA(h, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-        configured[h->device & 63] = true;
-    }
+    if (int rc = xb_smem_attr(h, kernel, SMEM_BYTES)) return rc;
     kernel<<<grid, IPCfg<EPI>::THREADS, SMEM_BYTES, s>>>(tmW, tmX, p);
     XB_LAUNCH_CHECK(h);
     return XB_OK;

@@ -245,29 +245,29 @@ lstm_bptt_step_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
 int xb_bptt_make_maps(xb_handle *h, BpttMaps *m, const void *dz, const void *w_hhT, const void *saved, int T, int N) {
     const uint64_t F = XB_FEATURES, G = XB_GATES;
     if (int rc = xb_make_tmap_2d(h, &m->dz_rows, dz, (uint64_t)T * N, G, G)) return rc;
-    if (int rc = xb_make_tmap_2d_box(h, &m->w_hhT, w_hhT, F, G, G, BK, BU, 1)) return rc;
+    {
+        const uint64_t dims[2] = {G, F}, st[1] = {G * 2};
+        const uint32_t box[2] = {BK, BU};
+        if (int rc = xb_make_tmap_nd(h, &m->w_hhT, w_hhT, 2, 2, dims, st, box, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
+    }
     {
         const uint64_t dims[4] = {F, (uint64_t)N, 5, (uint64_t)T};
         const uint64_t st[3] = {5 * F * 2, F * 2, (uint64_t)N * 5 * F * 2};
         const uint32_t box5[4] = {64, BM, 5, 1}, box1[4] = {64, BM, 1, 1};
-        if (int rc = xb_make_tmap_nd(h, &m->saved, saved, 4, 2, dims, st, box5)) return rc;
-        if (int rc = xb_make_tmap_nd(h, &m->saved_c, saved, 4, 2, dims, st, box1)) return rc;
+        if (int rc = xb_make_tmap_nd(h, &m->saved, saved, 4, 2, dims, st, box5, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
+        if (int rc = xb_make_tmap_nd(h, &m->saved_c, saved, 4, 2, dims, st, box1, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
     }
     {
         const uint64_t dims[4] = {F, (uint64_t)N, 4, (uint64_t)T};
         const uint64_t st[3] = {G * 2, F * 2, (uint64_t)N * G * 2};
         const uint32_t box[4] = {64, BM, 4, 1};
-        if (int rc = xb_make_tmap_nd(h, &m->dz_out, dz, 4, 2, dims, st, box)) return rc;
+        if (int rc = xb_make_tmap_nd(h, &m->dz_out, dz, 4, 2, dims, st, box, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
     }
     return XB_OK;
 }
 
 int xb_bptt_step_launch(xb_handle *h, const BpttMaps &m, const BpttStep &p, bool dependent, cudaStream_t s) {
-    static bool configured[64] = {};
-    if (!configured[h->device & 63]) {
-        XB_CUDA(h, cudaFuncSetAttribute(lstm_bptt_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-        configured[h->device & 63] = true;
-    }
+    if (int rc = xb_smem_attr(h, lstm_bptt_step_kernel, SMEM_BYTES)) return rc;
     StepParams sp;
     sp.N = p.N; sp.t_cur = p.t_cur; sp.t_prev = p.t_prev;
     sp.first = p.t_next < 0;

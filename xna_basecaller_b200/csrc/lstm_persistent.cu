@@ -48,6 +48,7 @@ constexpr int KPB = KCH / HP;              // K blocks per box
 constexpr int D_COL = 384;                 // accumulators start after the 384 columns of W_hh
 constexpr int CTR_STRIDE = 32;             // ints between counters (one 128-byte line each)
 constexpr int MAX_CTRS = 64;
+static_assert(MAX_CTRS * CTR_STRIDE == XB_LSTM_COUNTERS, "the handle allocates XB_LSTM_COUNTERS ints of counters");
 constexpr int PREFETCH_Y = 4;              // the y rows of step s + PREFETCH_Y are prefetched into L2 at step s
 
 // Geometry: SUB sub-batches of NS chunks per CTA, EW epilogue warps per sub-batch, two G buffers per sub-batch.
@@ -364,18 +365,22 @@ lstm_persistent_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_con
 template <bool SAVE>
 int launch(xb_handle *h, int layer, void *y_tnc, int T, int N, int reverse, cudaStream_t s, void *save) {
     CUtensorMap tmY, tmG;
-    if (int rc = xb_make_tmap_hview(h, &tmY, y_tnc, (uint64_t)T * N, NS, KPB)) return rc;
-    if (int rc = xb_make_tmap_2d_box(h, &tmG, h->gates, (uint64_t)T * N, XB_GATES, XB_GATES, 128, NS, 0)) return rc;
+    {       // y (T*N, 768) as {64 k, rows, 12 k-blocks}: one TMA lands KPB K-major [NS x 128 B] tiles
+        const uint64_t dims[3] = {64, (uint64_t)T * N, XB_FEATURES / 64}, st[2] = {XB_FEATURES * 2, 128};
+        const uint32_t box[3] = {64, NS, KPB};
+        if (int rc = xb_make_tmap_nd(h, &tmY, y_tnc, 3, 2, dims, st, box, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
+    }
+    {       // gates (T*N, 3072), 128 x NS boxes, not swizzled
+        const uint64_t dims[2] = {XB_GATES, (uint64_t)T * N}, st[1] = {XB_GATES * 2};
+        const uint32_t box[2] = {128, NS};
+        if (int rc = xb_make_tmap_nd(h, &tmG, h->gates, 2, 2, dims, st, box, CU_TENSOR_MAP_SWIZZLE_NONE)) return rc;
+    }
     const int max_groups = h->num_sms / TILES;                 // 6 on a 148-SM B200
     if (max_groups < 1)
         return xb_fail(h, XB_ERR_UNSUPPORTED, "the persistent LSTM needs %d co-resident CTAs, the device has %d SMs", TILES, h->num_sms);
     const int block_cap = max_groups * NB;
     auto fn = lstm_persistent_kernel<SAVE>;
-    static bool configured[64] = {};      // per device: function attributes live in the device's context
-    if (!configured[h->device & 63]) {
-        XB_CUDA(h, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-        configured[h->device & 63] = true;
-    }
+    if (int rc = xb_smem_attr(h, fn, SMEM_BYTES)) return rc;
     for (int batch0 = 0; batch0 < N; batch0 += block_cap) {
         PLParams p;
         p.T = T; p.N = N; p.reverse = reverse;
@@ -386,7 +391,7 @@ int launch(xb_handle *h, int layer, void *y_tnc, int T, int N, int reverse, cuda
         p.y = reinterpret_cast<uint16_t *>(y_tnc);
         p.counters = h->lstm_counters;
         p.save = reinterpret_cast<uint16_t *>(save);
-        XB_CUDA(h, cudaMemsetAsync(h->lstm_counters, 0, MAX_CTRS * CTR_STRIDE * sizeof(int), s));
+        XB_CUDA(h, cudaMemsetAsync(h->lstm_counters, 0, XB_LSTM_COUNTERS * sizeof(int), s));
         void *args[] = {(void *)&tmY, (void *)&tmG, (void *)&p};
         XB_CUDA(h, cudaLaunchCooperativeKernel((const void *)fn, dim3(p.G * TILES), dim3(THREADS), args, SMEM_BYTES, s));
         h->launches++;
@@ -400,11 +405,6 @@ int launch(xb_handle *h, int layer, void *y_tnc, int T, int N, int reverse, cuda
 // columns of every 128-wide tile ordered [unit][i,f,g,o] (weight repack mode 3 in xb_api.cu).
 // save != nullptr: the training forward, which also stores (T, N, 5, 768) fp16 = i, f, g, o, c for the backward pass
 int xb_lstm_recurrence_persistent(xb_handle *h, int layer, void *y_tnc, int T, int N, int reverse, cudaStream_t s, void *save) {
-    if (!h->lstm_counters) {
-        void *q = nullptr;
-        XB_CUDA(h, cudaMalloc(&q, MAX_CTRS * CTR_STRIDE * sizeof(int)));
-        h->lstm_counters = reinterpret_cast<int *>(q);
-    }
     if (save) return launch<true>(h, layer, y_tnc, T, N, reverse, s, save);
     return launch<false>(h, layer, y_tnc, T, N, reverse, s, nullptr);
 }

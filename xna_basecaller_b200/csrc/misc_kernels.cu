@@ -273,27 +273,29 @@ __global__ void ctc_simple_bwd_kernel(const float *__restrict__ scores, int T, i
 
 }  // namespace
 
-int xb_stitch_impl(xb_handle *h, const int8_t *rows, int T, const int32_t *chunk_first, const int32_t *chunk_count,
-                   const int32_t *read_len, int n_reads, int chunksize, int overlap, int stride, int reverse, int8_t *out,
-                   int out_stride, int32_t *out_len, cudaStream_t s) {
+extern "C" {
+
+int xb_stitch(xb_handle *h, const int8_t *rows, int T, const int32_t *chunk_first, const int32_t *chunk_count,
+              const int32_t *read_len, int n_reads, int chunksize, int overlap, int stride, int reverse, int8_t *out,
+              int out_stride, int32_t *out_len, void *stream) {
+    if (!h) return xb_fail(nullptr, XB_ERR_ARG, "NULL handle");
+    XB_REQUIRE(h, rows && chunk_first && chunk_count && read_len && out && out_len, "NULL buffer");
+    XB_CUDA(h, cudaSetDevice(h->device));
     XB_REQUIRE(h, n_reads > 0 && chunksize > overlap && stride > 0, "bad stitch arguments");
     const int warps = 4;
-    stitch_kernel<<<(n_reads + warps - 1) / warps, warps * 32, 0, s>>>(rows, T, chunk_first, chunk_count, read_len, n_reads,
-                                                                       chunksize, overlap, stride, reverse, out, out_stride, out_len);
+    stitch_kernel<<<(n_reads + warps - 1) / warps, warps * 32, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+        rows, T, chunk_first, chunk_count, read_len, n_reads, chunksize, overlap, stride, reverse, out, out_stride, out_len);
     XB_LAUNCH_CHECK(h);
     return XB_OK;
 }
 
-int xb_onehot_edges(xb_handle *h, const int32_t *edges_nt, int T, int N, int S, float *post, cudaStream_t s) {
-    onehot_edges_kernel<<<dim3(T, N), 256, 0, s>>>(edges_nt, T, N, S, post);
-    XB_LAUNCH_CHECK(h);
-    return XB_OK;
-}
-
-int xb_gather_chunks_impl(xb_handle *h, const void *signal, int sig_dtype, const int64_t *read_offset,
-                          const int32_t *read_len, const int32_t *chunk_read, const int32_t *chunk_start, int n_chunks,
-                          int L, float *out, cudaStream_t s) {
+int xb_gather_chunks(xb_handle *h, const void *signal, int sig_dtype, const int64_t *read_offset, const int32_t *read_len,
+                     const int32_t *chunk_read, const int32_t *chunk_start, int n_chunks, int L, float *out, void *stream) {
+    if (!h) return xb_fail(nullptr, XB_ERR_ARG, "NULL handle");
+    XB_REQUIRE(h, signal && read_offset && read_len && chunk_read && chunk_start && out, "NULL buffer");
+    XB_CUDA(h, cudaSetDevice(h->device));
     XB_REQUIRE(h, n_chunks > 0 && L > 0, "bad gather arguments");
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     dim3 grid((L + 1023) / 1024, n_chunks);
     if (sig_dtype == XB_SIG_F32)
         gather_chunks_kernel<float><<<grid, 256, 0, s>>>(reinterpret_cast<const float *>(signal), read_offset, read_len,
@@ -303,6 +305,14 @@ int xb_gather_chunks_impl(xb_handle *h, const void *signal, int sig_dtype, const
                                                            chunk_read, chunk_start, L, out);
     else
         return xb_fail(h, XB_ERR_ARG, "gather supports fp32 and int16 signal");
+    XB_LAUNCH_CHECK(h);
+    return XB_OK;
+}
+
+}  // extern "C"
+
+int xb_onehot_edges(xb_handle *h, const int32_t *edges_nt, int T, int N, int S, float *post, cudaStream_t s) {
+    onehot_edges_kernel<<<dim3(T, N), 256, 0, s>>>(edges_nt, T, N, S, post);
     XB_LAUNCH_CHECK(h);
     return XB_OK;
 }
@@ -337,8 +347,7 @@ int xb_ctc_loss_bwd_impl(xb_handle *h, const float *scores, int T, int N, const 
         if (int rc = xb_decode_alpha(h, scores, T, N, nullptr, h->logz, 0, s)) return rc;
     }
     size_t smem = sizeof(float) * (3 * NT + 1 + 2 * S);
-    if (smem > 48 * 1024)
-        XB_CUDA(h, cudaFuncSetAttribute(ctc_simple_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (int rc = xb_smem_attr(h, ctc_simple_bwd_kernel, smem)) return rc;
     ctc_simple_bwd_kernel<<<N, NT, smem, s>>>(scores, T, N, S, targets, Lmax, lengths, h->logz, normalise, h->n_base,
                                              h->state_len, grad_loss, alpha_ws, grad);
     XB_LAUNCH_CHECK(h);

@@ -234,11 +234,15 @@ preprocess_kernel(const int16_t *__restrict__ raw_all, const int64_t *__restrict
 
 }  // namespace
 
-int xb_preprocess_impl(xb_handle *h, const int16_t *raw, const int64_t *read_offset, const int32_t *read_len,
-                       const double *scaling, const int32_t *offset, int n_reads, float *out, int32_t *out_len,
-                       float *stats, cudaStream_t s) {
+extern "C" int xb_preprocess_reads(xb_handle *h, const int16_t *raw, const int64_t *read_offset, const int32_t *read_len,
+                                   const double *scaling, const int32_t *offset, int n_reads, float *out, int32_t *out_len,
+                                   float *stats, void *stream) {
+    if (!h) return xb_fail(nullptr, XB_ERR_ARG, "NULL handle");
+    XB_REQUIRE(h, raw && read_offset && read_len && scaling && offset && out && out_len && stats, "NULL buffer");
+    XB_CUDA(h, cudaSetDevice(h->device));
     XB_REQUIRE(h, n_reads > 0, "bad pre-processing arguments");
-    preprocess_kernel<<<n_reads, PP_THREADS, 0, s>>>(raw, read_offset, read_len, scaling, offset, out, out_len, stats);
+    preprocess_kernel<<<n_reads, PP_THREADS, 0, reinterpret_cast<cudaStream_t>(stream)>>>(raw, read_offset, read_len, scaling,
+                                                                                         offset, out, out_len, stats);
     XB_LAUNCH_CHECK(h);
     return XB_OK;
 }

@@ -41,14 +41,6 @@
 #include "xb_dropout.cuh"
 #include "xb_gemm.cuh"
 
-int xb_conv12_im2col(xb_handle *h, const void *signal, int sig_dtype, int N, int L, cudaStream_t s, const xb_dropout *drop);
-int xb_conv_stem_fwd_dropout(xb_handle *h, const void *signal, int sig_dtype, int N, int L, void *out_tnc,
-                             const xb_dropout *drop, void *stream);
-int xb_lstm_recurrence_persistent(xb_handle *h, int layer, void *y_tnc, int T, int N, int reverse, cudaStream_t s, void *save);
-int xb_lstm_wgrad_launch(xb_handle *h, const void *dzT, const void *xT, const void *yT, int T, int N, bool reverse, float *g_wih,
-                         float *g_whh, cudaStream_t s);
-int xb_inproj_launch(xb_handle *h, const void *x, const void *w_ih, const float *bias, void *gates, int M, cudaStream_t s);
-
 struct xb_train_ws {
     int cap_N = 0, cap_T = 0;      // capacity
     int N = 0, T = 0;              // shape of the last forward
@@ -249,13 +241,6 @@ conv1_bwd_kernel(const SIG *__restrict__ signal, int L, const float *__restrict_
     else if (tid < 24) atomicAdd(db1 + tid - 20, acc[tid]);
 }
 
-int alloc(xb_handle *h, void **p, size_t bytes) {
-    if (*p) return XB_OK;
-    cudaError_t e = cudaMalloc(p, bytes);
-    if (e != cudaSuccess) return xb_fail(h, XB_ERR_NOMEM, "training workspace: cudaMalloc of %zu bytes failed: %s", bytes, cudaGetErrorString(e));
-    return XB_OK;
-}
-
 // The three forms of the training step's transpositions (R, C) 16-bit -> (C, R) bf16:
 //   TR_BF16_COLSUM  a bf16 gradient, plus the column sums of its first nsum columns (a bias gradient)
 //   TR_F16          an fp16 activation
@@ -397,7 +382,7 @@ int gemm_bf16(xb_handle *h, int epi, const void *A, int M, int lda, const void *
 // xb_train_free frees it.  dpre / dpreT are not in it (aliases of DZ / DZT).
 struct ws_buffer { void **p; size_t bytes; };
 static std::vector<ws_buffer> ws_buffers(const xb_handle *h, xb_train_ws *w) {
-    const size_t TN = (size_t)w->cap_T * w->cap_N, F = XB_FEATURES, HP = h->head_rows_padded ? h->head_rows_padded : 3072;
+    const size_t TN = (size_t)w->cap_T * w->cap_N, F = XB_FEATURES, HP = h->head_rows_padded;
     const size_t NL = (size_t)w->cap_N * w->cap_T * XB_STRIDE;
     std::vector<ws_buffer> b;
     for (void *&p : w->x) b.push_back({&p, TN * F * 2});
@@ -430,7 +415,7 @@ static int train_ws(xb_handle *h, int N, int T, bool with_xd) {
     xb_train_ws *w = h->train;
     for (const ws_buffer &b : ws_buffers(h, w))
         if (b.p != &w->xd || with_xd)
-            if (int rc = alloc(h, b.p, b.bytes)) return rc;
+            if (int rc = xb_alloc(h, b.p, b.bytes)) return rc;
     w->dpre = w->DZ;            // conv3's (TN,768) gradients reuse the LSTM buffers (the LSTM layers are done by then)
     w->dpreT = w->DZT;
     return XB_OK;

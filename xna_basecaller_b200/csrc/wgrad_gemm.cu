@@ -129,14 +129,12 @@ int xb_lstm_wgrad_launch(xb_handle *h, const void *dzT, const void *xT, const vo
                          float *g_whh, cudaStream_t s) {
     const uint64_t TN = (uint64_t)T * N;
     CUtensorMap tmA, tmX, tmY;
-    if (int rc = xb_make_tmap_2d_box(h, &tmA, dzT, XB_GATES, TN, TN, BK, BM, 1)) return rc;
-    if (int rc = xb_make_tmap_2d_box(h, &tmX, xT, XB_FEATURES, TN, TN, BK, BN, 1)) return rc;
-    if (int rc = xb_make_tmap_2d_box(h, &tmY, yT, XB_FEATURES, TN, TN, BK, BN, 1)) return rc;
-    static bool configured[64] = {};
-    if (!configured[h->device & 63]) {
-        XB_CUDA(h, cudaFuncSetAttribute(lstm_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-        configured[h->device & 63] = true;
-    }
+    const uint64_t dims_dz[2] = {TN, XB_GATES}, dims_h[2] = {TN, XB_FEATURES}, st[1] = {TN * 2};
+    const uint32_t box_dz[2] = {BK, BM}, box_h[2] = {BK, BN};
+    if (int rc = xb_make_tmap_nd(h, &tmA, dzT, 2, 2, dims_dz, st, box_dz, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
+    if (int rc = xb_make_tmap_nd(h, &tmX, xT, 2, 2, dims_h, st, box_h, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
+    if (int rc = xb_make_tmap_nd(h, &tmY, yT, 2, 2, dims_h, st, box_h, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
+    if (int rc = xb_smem_attr(h, lstm_wgrad_kernel, SMEM_BYTES)) return rc;
     WgradParams p;
     p.K = (int)TN;
     // forward layers: steps t = 1 .. T-1 pair dz_t with h_{t-1}:  DZ^T column k + N  x  Y^T column k

@@ -21,46 +21,9 @@ int xb_fail(xb_handle *h, int code, const char *fmt, ...) {
     return code;
 }
 
-struct xb_dropout;
-int xb_conv12_im2col(xb_handle *h, const void *signal, int sig_dtype, int N, int L, cudaStream_t s,
-                     const xb_dropout *drop = nullptr);
-int xb_lstm_recurrence_persistent(xb_handle *h, int layer, void *y_tnc, int T, int N, int reverse, cudaStream_t s, void *save = nullptr);
-int xb_inproj_launch(xb_handle *h, const void *x, const void *w_ih, const float *bias, void *gates, int M, cudaStream_t s);
-int xb_head_astationary_launch(xb_handle *h, const void *x, const void *w, int w_rows, const float *bias, int head_rows,
-                               float *scores, int ldo, int M, int exp_out, cudaStream_t s);
-int xb_preprocess_impl(xb_handle *h, const int16_t *raw, const int64_t *read_offset, const int32_t *read_len,
-                       const double *scaling, const int32_t *offset, int n_reads, float *out, int32_t *out_len,
-                       float *stats, cudaStream_t s);
-int xb_ctc_loss_bwd_impl(xb_handle *h, const float *scores, int T, int N, const int32_t *targets, int Lmax,
-                         const int32_t *lengths, int normalise, const float *grad_loss, float *alpha_ws, float *grad,
-                         cudaStream_t s);
-int xb_ctc_loss_impl(xb_handle *h, const float *scores, int T, int N, const int32_t *targets, int Lmax,
-                     const int32_t *lengths, int normalise, float *loss, cudaStream_t s);
-int xb_stitch_impl(xb_handle *h, const int8_t *rows, int T, const int32_t *chunk_first, const int32_t *chunk_count,
-                   const int32_t *read_len, int n_reads, int chunksize, int overlap, int stride, int reverse, int8_t *out,
-                   int out_stride, int32_t *out_len, cudaStream_t s);
-
-void xb_train_free(xb_handle *h);
-int xb_beam_search_impl(xb_handle *h, const float *scores, const float *beta, int T, int N, int beam_width, float beam_cut,
-                        int8_t *seq, int8_t *qstring, int8_t *moves, int32_t *lens, cudaStream_t s);
-int xb_onehot_edges(xb_handle *h, const int32_t *edges_nt, int T, int N, int S, float *post, cudaStream_t s);
-int xb_gather_chunks_impl(xb_handle *h, const void *signal, int sig_dtype, const int64_t *read_offset,
-                          const int32_t *read_len, const int32_t *chunk_read, const int32_t *chunk_start, int n_chunks,
-                          int L, float *out, cudaStream_t s);
-
 namespace {
 
 int ipow(int b, int e) { int r = 1; while (e-- > 0) r *= b; return r; }
-
-template <typename T> int dev_alloc(xb_handle *h, T **p, size_t count) {
-    void *q = nullptr;
-    cudaError_t e = cudaMalloc(&q, count * sizeof(T));
-    if (e != cudaSuccess)
-        return xb_fail(h, XB_ERR_NOMEM, "cudaMalloc of %zu bytes failed: %s", count * sizeof(T), cudaGetErrorString(e));
-    *p = reinterpret_cast<T *>(q);
-    return XB_OK;
-}
-int dev_alloc_bytes(xb_handle *h, void **p, size_t bytes) { return dev_alloc<uint8_t>(h, reinterpret_cast<uint8_t **>(p), bytes); }
 
 // ---- weight repacking ------------------------------------------------------------------------------
 // dst (rows_dst, cols_dst) 16-bit <- src fp32; mode 0: plain rows (zero padding past rows_src / cols_src);
@@ -135,6 +98,48 @@ int check_tn(xb_handle *h, int T, int N) {
     return XB_OK;
 }
 
+// Every device buffer the handle owns, with its size and the group it is allocated with:
+//   BUF_DECODE   decode state, xb_create
+//   BUF_ENCODER  encoder workspace and slot 0 of the host entry points, xb_create unless XB_FLAG_NO_ENCODER
+//   BUF_WEIGHTS  weights, the first xb_load_*_weights
+//   BUF_TRAIN    the transposed weights of the training backward, the first xb_load_*_weights under XB_FLAG_TRAIN
+//   BUF_SLOT1    slot 1 of the host entry points, the first xb_compute_scores_submit into either slot
+// alloc_group allocates the buffers of a group that are still NULL; xb_destroy frees every buffer in the list.
+enum BufGroup { BUF_DECODE, BUF_ENCODER, BUF_WEIGHTS, BUF_TRAIN, BUF_SLOT1 };
+struct handle_buffer { void **p; size_t bytes; BufGroup group; };
+
+template <typename T> void **ptr_of(T *&p) { return reinterpret_cast<void **>(&p); }
+
+std::vector<handle_buffer> handle_buffers(xb_handle *h) {
+    const size_t TN = (size_t)h->max_T * h->max_N, N = h->max_N, F = XB_FEATURES, G = XB_GATES, HP = h->head_rows_padded;
+    const size_t VP = (size_t)((h->C + 31) / 32) * 32 + 4, S = (size_t)h->C * h->NZ;
+    const BufGroup D = BUF_DECODE, E = BUF_ENCODER, W = BUF_WEIGHTS, TR = BUF_TRAIN;
+    std::vector<handle_buffer> b = {
+        {ptr_of(h->alpha), (TN + N) * VP * 4, D}, {ptr_of(h->bmax), (TN + N) * VP * 4, D},
+        {ptr_of(h->beta), (TN + N) * VP * 4, D}, {ptr_of(h->logz), N * 4, D},
+        {&h->c2, TN * XB_CONV3_K * 2, E}, {&h->act0, TN * F * 2, E}, {&h->act1, TN * F * 2, E}, {&h->gates, TN * G * 2, E},
+        {ptr_of(h->scores), TN * S * 4, E}, {ptr_of(h->lstm_counters), XB_LSTM_COUNTERS * 4, E},
+        {ptr_of(h->conv1_w), 20 * 4, W}, {ptr_of(h->conv1_b), 4 * 4, W}, {ptr_of(h->conv2_w), 320 * 4, W},
+        {ptr_of(h->conv2_b), 16 * 4, W}, {&h->conv3_w, F * XB_CONV3_K * 2, W}, {ptr_of(h->conv3_b), F * 4, W},
+        {&h->head_w, HP * F * 2, W}, {ptr_of(h->head_b), HP * 4, W},
+        {&h->conv3_wT, XB_CONV3_K * F * 2, TR}, {&h->head_wT, F * HP * 2, TR}};
+    for (xb_lstm_weights &l : h->lstm)
+        b.insert(b.end(), {{&l.w_ih, G * F * 2, W}, {&l.w_hh, G * F * 2, W}, {ptr_of(l.bias), G * 4, W},
+                           {&l.w_ihT, F * G * 2, TR}, {&l.w_hhT, F * G * 2, TR}});
+    for (int i = 0; i < 2; i++) {
+        const BufGroup g = i ? BUF_SLOT1 : E;
+        b.insert(b.end(), {{&h->signal_dev[i], TN * XB_STRIDE * 4, g}, {ptr_of(h->seq_dev[i]), TN, g}, {ptr_of(h->lens_dev[i]), N * 4, g}});
+    }
+    return b;
+}
+
+int alloc_group(xb_handle *h, BufGroup group) {
+    for (const handle_buffer &b : handle_buffers(h))
+        if (b.group == group)
+            if (int rc = xb_alloc(h, b.p, b.bytes)) return rc;
+    return XB_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -199,26 +204,11 @@ int xb_create(xb_handle **out, int device, int max_N, int max_T, int n_base, int
     h->bf16 = (flags & XB_FLAG_BF16) != 0;
     h->num_sms = prop.multiProcessorCount;
     strncpy(h->alphabet, alphabet, sizeof h->alphabet - 1);
+    h->head_rows = ipow(n_base, state_len + 1);
+    h->head_rows_padded = ((h->head_rows + 127) / 128) * 128;
 
-    const size_t TN = (size_t)max_T * max_N, S = (size_t)h->C * h->NZ;
-    int rc = XB_OK;
-#define TRY(x) if (rc == XB_OK) rc = (x)
-    const size_t VP = (size_t)((h->C + 31) / 32) * 32 + 4;
-    TRY(dev_alloc(h, &h->alpha, (TN + max_N) * VP));
-    TRY(dev_alloc(h, &h->bmax, (TN + max_N) * VP));
-    TRY(dev_alloc(h, &h->beta, (TN + max_N) * VP));
-    TRY(dev_alloc(h, &h->logz, (size_t)max_N));
-    TRY(dev_alloc(h, &h->seq_dev, TN));
-    TRY(dev_alloc(h, &h->lens_dev, (size_t)max_N));
-    if (!(flags & XB_FLAG_NO_ENCODER)) {
-        TRY(dev_alloc_bytes(h, &h->c2, TN * XB_CONV3_K * 2));
-        TRY(dev_alloc_bytes(h, &h->act0, TN * XB_FEATURES * 2));
-        TRY(dev_alloc_bytes(h, &h->act1, TN * XB_FEATURES * 2));
-        TRY(dev_alloc_bytes(h, &h->gates, TN * XB_GATES * 2));
-        TRY(dev_alloc(h, &h->scores, TN * S));
-        TRY(dev_alloc_bytes(h, &h->signal_dev, TN * XB_STRIDE * sizeof(float)));
-    }
-#undef TRY
+    int rc = alloc_group(h, BUF_DECODE);
+    if (rc == XB_OK && !(flags & XB_FLAG_NO_ENCODER)) rc = alloc_group(h, BUF_ENCODER);
     if (rc != XB_OK) {
         xb_global_err = h->err;
         xb_destroy(h);
@@ -231,13 +221,8 @@ int xb_create(xb_handle **out, int device, int max_N, int max_T, int n_base, int
 int xb_destroy(xb_handle *h) {
     if (!h) return XB_OK;
     cudaSetDevice(h->device);
-    void *ptrs[] = {h->conv1_w, h->conv1_b, h->conv2_w, h->conv2_b, h->conv3_w, h->conv3_b, h->head_w, h->head_b, h->c2,
-                    h->act0, h->act1, h->gates, h->scores, h->signal_dev, h->seq_dev, h->lens_dev,
-                    h->alpha, h->bmax, h->beta, h->logz, h->lstm_counters};
-    for (void *p : ptrs)
-        if (p) cudaFree(p);
-    for (void *p : {(void *)h->signal_dev2, (void *)h->seq_dev2, (void *)h->lens_dev2})
-        if (p) cudaFree(p);
+    for (const handle_buffer &b : handle_buffers(h))
+        if (*b.p) cudaFree(*b.p);
     if (h->h2d_stream) cudaStreamDestroy(h->h2d_stream);
     if (h->d2h_stream) cudaStreamDestroy(h->d2h_stream);
     for (int i = 0; i < 2; i++)
@@ -245,39 +230,9 @@ int xb_destroy(xb_handle *h) {
             if (e) cudaEventDestroy(e);
     for (auto &sp : h->spans) { cudaEventDestroy(sp.a); cudaEventDestroy(sp.b); }
     for (auto e : h->event_pool) cudaEventDestroy(e);
-    for (auto &l : h->lstm) {
-        for (void *p : {l.w_ih, l.w_hh, (void *)l.bias, l.w_ihT, l.w_hhT})
-            if (p) cudaFree(p);
-    }
-    if (h->head_wT) cudaFree(h->head_wT);
-    if (h->conv3_wT) cudaFree(h->conv3_wT);
     xb_train_free(h);
     delete h;
     return XB_OK;
-}
-
-static int alloc_weights(xb_handle *h) {
-    if (h->conv1_w) return XB_OK;
-    const int F = XB_FEATURES;
-    h->head_rows = ipow(h->n_base, h->state_len + 1);
-    h->head_rows_padded = ((h->head_rows + 127) / 128) * 128;
-    int rc = XB_OK;
-#define TRY(x) if (rc == XB_OK) rc = (x)
-    TRY(dev_alloc(h, &h->conv1_w, 20));
-    TRY(dev_alloc(h, &h->conv1_b, 4));
-    TRY(dev_alloc(h, &h->conv2_w, 320));
-    TRY(dev_alloc(h, &h->conv2_b, 16));
-    TRY(dev_alloc_bytes(h, &h->conv3_w, (size_t)F * XB_CONV3_K * 2));
-    TRY(dev_alloc(h, &h->conv3_b, (size_t)F));
-    for (auto &l : h->lstm) {
-        TRY(dev_alloc_bytes(h, &l.w_ih, (size_t)XB_GATES * F * 2));
-        TRY(dev_alloc_bytes(h, &l.w_hh, (size_t)XB_GATES * F * 2));
-        TRY(dev_alloc(h, &l.bias, (size_t)XB_GATES));
-    }
-    TRY(dev_alloc_bytes(h, &h->head_w, (size_t)h->head_rows_padded * F * 2));
-    TRY(dev_alloc(h, &h->head_b, (size_t)h->head_rows_padded));
-#undef TRY
-    return rc;
 }
 
 #define XB_WEIGHTS_PROLOGUE()                                                                          \
@@ -285,7 +240,9 @@ static int alloc_weights(xb_handle *h) {
     XB_REQUIRE(h, !(h->flags & XB_FLAG_NO_ENCODER), "handle was created with XB_FLAG_NO_ENCODER");     \
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);                                           \
     XB_CUDA(h, cudaSetDevice(h->device));                                                              \
-    if (int rc_ = alloc_weights(h)) return rc_
+    if (int rc_ = alloc_group(h, BUF_WEIGHTS)) return rc_;                                             \
+    if (h->flags & XB_FLAG_TRAIN)                                                                      \
+        if (int rc_ = alloc_group(h, BUF_TRAIN)) return rc_
 
 int xb_load_conv_weights(xb_handle *h, const float *w1, const float *b1, const float *w2, const float *b2,
                          const float *w3, const float *b3, void *stream) {
@@ -298,7 +255,6 @@ int xb_load_conv_weights(xb_handle *h, const float *w1, const float *b1, const f
     XB_CUDA(h, cudaMemcpyAsync(h->conv2_b, b2, 16 * 4, cudaMemcpyDeviceToDevice, s));
     if (int rc = repack(h, w3, h->conv3_w, F, XB_CONV3_K, F, XB_C2_CH * XB_WINLEN, 2, s)) return rc;
     if (h->flags & XB_FLAG_TRAIN) {
-        if (!h->conv3_wT) { if (int rc = dev_alloc_bytes(h, &h->conv3_wT, (size_t)XB_CONV3_K * F * 2)) return rc; }
         if (int rc = repack(h, w3, h->conv3_wT, XB_CONV3_K, F, F, XB_C2_CH * XB_WINLEN, 6, s)) return rc;
     }
     XB_CUDA(h, cudaMemcpyAsync(h->conv3_b, b3, F * 4, cudaMemcpyDeviceToDevice, s));
@@ -316,8 +272,6 @@ int xb_load_lstm_weights(xb_handle *h, int layer, const float *w_ih, const float
     if (int rc = repack(h, w_hh, h->lstm[layer].w_hh, XB_GATES, F, XB_GATES, F, 4, s)) return rc;
     if (h->flags & XB_FLAG_TRAIN) {
         xb_lstm_weights &lw = h->lstm[layer];
-        if (!lw.w_ihT) { if (int rc = dev_alloc_bytes(h, &lw.w_ihT, (size_t)XB_GATES * F * 2)) return rc; }
-        if (!lw.w_hhT) { if (int rc = dev_alloc_bytes(h, &lw.w_hhT, (size_t)XB_GATES * F * 2)) return rc; }
         if (int rc = repack(h, w_ih, lw.w_ihT, F, XB_GATES, XB_GATES, F, 5, s)) return rc;
         if (int rc = repack(h, w_hh, lw.w_hhT, F, XB_GATES, XB_GATES, F, 5, s)) return rc;
     }
@@ -334,7 +288,6 @@ int xb_load_head_weights(xb_handle *h, const float *w, const float *b, float sca
     const int F = XB_FEATURES;
     if (int rc = repack(h, w, h->head_w, h->head_rows_padded, F, h->head_rows, F, 0, s)) return rc;
     if (h->flags & XB_FLAG_TRAIN) {
-        if (!h->head_wT) { if (int rc = dev_alloc_bytes(h, &h->head_wT, (size_t)h->head_rows_padded * F * 2)) return rc; }
         if (int rc = repack(h, w, h->head_wT, F, h->head_rows_padded, h->head_rows, F, 5, s)) return rc;
     }
     XB_CUDA(h, cudaMemsetAsync(h->head_b, 0, (size_t)h->head_rows_padded * 4, s));
@@ -451,8 +404,7 @@ int xb_encoder_fwd(xb_handle *h, const void *signal, int sig_dtype, int N, int L
 }
 
 // Fused encoder + decode of chunks that are already on the device: the head hands exp(scores) to the decode (h->scores
-// never holds log-domain scores on this route), labels / packed rows come back.  The *_host entry points and the read-set
-// pipeline run through here.
+// never holds log-domain scores on this route), labels / packed rows come back.  The read-set pipeline runs through here.
 int xb_basecall_chunks(xb_handle *h, const void *signal, int sig_dtype, int N, int L, int8_t *seq, int8_t *qstring,
                        int32_t *lens, void *stream) {
     if (!h) return xb_fail(nullptr, XB_ERR_ARG, "NULL handle");
@@ -568,69 +520,24 @@ int xb_ctc_crf_loss_bwd(xb_handle *h, const float *scores, int T, int N, const i
     return xb_ctc_loss_bwd_impl(h, scores, T, N, targets, Lmax, lengths, normalise, grad_loss, alpha_ws, grad_scores, s);
 }
 
-int xb_stitch(xb_handle *h, const int8_t *rows, int T, const int32_t *chunk_first, const int32_t *chunk_count,
-              const int32_t *read_len, int n_reads, int chunksize, int overlap, int stride, int reverse, int8_t *out,
-              int out_stride, int32_t *out_len, void *stream) {
-    if (!h) return xb_fail(nullptr, XB_ERR_ARG, "NULL handle");
-    XB_REQUIRE(h, rows && chunk_first && chunk_count && read_len && out && out_len, "NULL buffer");
-    XB_CUDA(h, cudaSetDevice(h->device));
-    return xb_stitch_impl(h, rows, T, chunk_first, chunk_count, read_len, n_reads, chunksize, overlap, stride, reverse, out,
-                          out_stride, out_len, reinterpret_cast<cudaStream_t>(stream));
-}
-
-int xb_gather_chunks(xb_handle *h, const void *signal, int sig_dtype, const int64_t *read_offset, const int32_t *read_len,
-                     const int32_t *chunk_read, const int32_t *chunk_start, int n_chunks, int L, float *out, void *stream) {
-    if (!h) return xb_fail(nullptr, XB_ERR_ARG, "NULL handle");
-    XB_REQUIRE(h, signal && read_offset && read_len && chunk_read && chunk_start && out, "NULL buffer");
-    XB_CUDA(h, cudaSetDevice(h->device));
-    return xb_gather_chunks_impl(h, signal, sig_dtype, read_offset, read_len, chunk_read, chunk_start, n_chunks, L, out,
-                                 reinterpret_cast<cudaStream_t>(stream));
-}
-
-int xb_preprocess_reads(xb_handle *h, const int16_t *raw, const int64_t *read_offset, const int32_t *read_len,
-                        const double *scaling, const int32_t *offset, int n_reads, float *out, int32_t *out_len,
-                        float *stats, void *stream) {
-    if (!h) return xb_fail(nullptr, XB_ERR_ARG, "NULL handle");
-    XB_REQUIRE(h, raw && read_offset && read_len && scaling && offset && out && out_len && stats, "NULL buffer");
-    XB_CUDA(h, cudaSetDevice(h->device));
-    return xb_preprocess_impl(h, raw, read_offset, read_len, scaling, offset, n_reads, out, out_len, stats,
-                              reinterpret_cast<cudaStream_t>(stream));
-}
-
+// xb_compute_scores_submit into slot 0 followed by xb_compute_scores_wait
 int xb_compute_scores_host(xb_handle *h, const float *signal_host, int N, int L, int8_t *seq_host, int32_t *lens_host,
                            void *stream) {
-    if (!h) return xb_fail(nullptr, XB_ERR_ARG, "NULL handle");
-    XB_REQUIRE(h, signal_host && seq_host && lens_host, "NULL buffer");
-    XB_REQUIRE(h, L > 0 && L % XB_STRIDE == 0, "chunk length %d must be a positive multiple of the stride %d", L, XB_STRIDE);
-    const int T = L / XB_STRIDE;
-    if (int rc = check_tn(h, T, N)) return rc;
-    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    XB_CUDA(h, cudaMemcpyAsync(h->signal_dev, signal_host, (size_t)N * L * sizeof(float), cudaMemcpyHostToDevice, s));
-    if (int rc = xb_basecall_chunks(h, h->signal_dev, XB_SIG_F32, N, L, h->seq_dev, nullptr, h->lens_dev, stream)) return rc;
-    XB_CUDA(h, cudaMemcpyAsync(seq_host, h->seq_dev, (size_t)N * T, cudaMemcpyDeviceToHost, s));
-    XB_CUDA(h, cudaMemcpyAsync(lens_host, h->lens_dev, (size_t)N * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-    XB_CUDA(h, cudaStreamSynchronize(s));
-    return XB_OK;
+    if (int rc = xb_compute_scores_submit(h, 0, signal_host, N, L, seq_host, lens_host, stream)) return rc;
+    return xb_compute_scores_wait(h, 0);
 }
 
-// Pipelined form of xb_compute_scores_host: two slots; submit() enqueues H2D (own copy stream), encoder + decode (the
-// caller's stream) and D2H (second copy stream) of one batch and returns, wait() blocks until the slot's results are in
-// the host buffers.  With batch i+1 submitted before batch i is awaited, the copies of one batch hide under the kernels
-// of the other.  A slot must be awaited before it is submitted again; host buffers must stay valid until then.
-static int pipeline_init(xb_handle *h) {
-    if (h->h2d_stream) return XB_OK;
-    const size_t TN = (size_t)h->max_T * h->max_N;
-    XB_CUDA(h, cudaMalloc(&h->signal_dev2, TN * XB_STRIDE * sizeof(float)));
-    XB_CUDA(h, cudaMalloc(reinterpret_cast<void **>(&h->seq_dev2), TN));
-    XB_CUDA(h, cudaMalloc(reinterpret_cast<void **>(&h->lens_dev2), (size_t)h->max_N * sizeof(int32_t)));
-    XB_CUDA(h, cudaStreamCreateWithFlags(&h->h2d_stream, cudaStreamNonBlocking));
-    XB_CUDA(h, cudaStreamCreateWithFlags(&h->d2h_stream, cudaStreamNonBlocking));
-    for (int i = 0; i < 2; i++) {
-        XB_CUDA(h, cudaEventCreateWithFlags(&h->ev_h2d[i], cudaEventDisableTiming));
-        XB_CUDA(h, cudaEventCreateWithFlags(&h->ev_enc[i], cudaEventDisableTiming));
-        XB_CUDA(h, cudaEventCreateWithFlags(&h->ev_dec[i], cudaEventDisableTiming));
-        XB_CUDA(h, cudaEventCreateWithFlags(&h->ev_done[i], cudaEventDisableTiming));
-    }
+// Host-buffer basecalling in two slots: submit() enqueues H2D (own copy stream), encoder + decode (the caller's stream)
+// and D2H (second copy stream) of one batch and returns, wait() blocks until the slot's results are in the host buffers.
+// With batch i+1 submitted before batch i is awaited, the copies of one batch hide under the kernels of the other.  A
+// slot must be awaited before it is submitted again; host buffers must stay valid until then.
+static int pipeline_init(xb_handle *h) {       // each piece once: a call after a failure creates what is missing
+    if (int rc = alloc_group(h, BUF_SLOT1)) return rc;
+    for (cudaStream_t *st : {&h->h2d_stream, &h->d2h_stream})
+        if (!*st) XB_CUDA(h, cudaStreamCreateWithFlags(st, cudaStreamNonBlocking));
+    for (int i = 0; i < 2; i++)
+        for (cudaEvent_t *e : {&h->ev_h2d[i], &h->ev_enc[i], &h->ev_dec[i], &h->ev_done[i]})
+            if (!*e) XB_CUDA(h, cudaEventCreateWithFlags(e, cudaEventDisableTiming));
     return XB_OK;
 }
 
@@ -642,12 +549,13 @@ int xb_compute_scores_submit(xb_handle *h, int slot, const float *signal_host, i
     XB_REQUIRE(h, L > 0 && L % XB_STRIDE == 0, "chunk length %d must be a positive multiple of the stride %d", L, XB_STRIDE);
     const int T = L / XB_STRIDE;
     if (int rc = check_tn(h, T, N)) return rc;
-    if (!h->signal_dev) return xb_fail(h, XB_ERR_STATE, "handle was created without the encoder");
+    if (!h->signal_dev[0]) return xb_fail(h, XB_ERR_STATE, "handle was created without the encoder");
+    XB_REQUIRE(h, h->expand_blanks, "the fused route needs expand_blanks (Viterbi decode over C*NZ scores)");
     if (int rc = pipeline_init(h)) return rc;
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    void *sig = slot ? h->signal_dev2 : h->signal_dev;
-    int8_t *seq = slot ? h->seq_dev2 : h->seq_dev;
-    int32_t *lens = slot ? h->lens_dev2 : h->lens_dev;
+    void *sig = h->signal_dev[slot];
+    int8_t *seq = h->seq_dev[slot];
+    int32_t *lens = h->lens_dev[slot];
     if (h->slot_used[slot]) {       // the slot's previous batch: its signal has been consumed, its results have left
         XB_CUDA(h, cudaStreamWaitEvent(h->h2d_stream, h->ev_enc[slot], 0));
         XB_CUDA(h, cudaStreamWaitEvent(s, h->ev_done[slot], 0));

@@ -8,6 +8,7 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <string>
+#include <unordered_map>
 #include <vector>
 
 #include "../../include/xna_basecaller.h"
@@ -19,6 +20,7 @@
 #define XB_C2_CH 16              // channels after the second convolution
 #define XB_C2_HALO 9             // winlen // 2
 #define XB_CONV3_K 320           // 19*16 = 304 padded to a multiple of 64 (zero weights)
+#define XB_LSTM_COUNTERS 2048    // ints of the persistent LSTM kernel's step counters (lstm_persistent.cu MAX_CTRS x CTR_STRIDE)
 
 struct xb_lstm_weights {
     void *w_ih = nullptr;        // (3072, 768) 16-bit, rows gate-interleaved (see xb_api.cu)
@@ -65,13 +67,12 @@ struct xb_handle {
     void *act0 = nullptr, *act1 = nullptr;   // (max_T, max_N, 768) 16-bit ping-pong
     void *gates = nullptr;       // (max_T, max_N, 3072) 16-bit hoisted input projection
     float *scores = nullptr;     // (max_T, max_N, C*NZ) fp32 (used by the host entry points)
-    void *signal_dev = nullptr;  // (max_N, max_T*5) fp32 staging for the host entry points
-    int8_t *seq_dev = nullptr;   // (max_N, max_T)
-    int32_t *lens_dev = nullptr; // (max_N)
-    // second slot + copy streams of the pipelined host entry points (xb_compute_scores_submit / _wait), created on first use
-    void *signal_dev2 = nullptr;
-    int8_t *seq_dev2 = nullptr;
-    int32_t *lens_dev2 = nullptr;
+    int *lstm_counters = nullptr; // XB_LSTM_COUNTERS per-group step counters of the persistent LSTM kernel
+    // the two slots of the host entry points (xb_compute_scores_submit / _wait): slot 0 is allocated with the encoder
+    // workspace, slot 1, the copy streams and the events on first use
+    void *signal_dev[2] = {};    // (max_N, max_T*5) fp32 staging
+    int8_t *seq_dev[2] = {};     // (max_N, max_T)
+    int32_t *lens_dev[2] = {};   // (max_N)
     cudaStream_t h2d_stream = nullptr, d2h_stream = nullptr;
     cudaEvent_t ev_h2d[2] = {nullptr, nullptr}, ev_enc[2] = {nullptr, nullptr}, ev_dec[2] = {nullptr, nullptr},
                 ev_done[2] = {nullptr, nullptr};
@@ -84,7 +85,6 @@ struct xb_handle {
     float *bmax = nullptr;       // linear decode: bm_hat; log-domain scans: Max-semiring beta
     float *beta = nullptr;       // linear decode: b_hat;  beam search: Log-semiring beta
     float *logz = nullptr;       // (max_N)
-    int *lstm_counters = nullptr; // per-group step counters of the persistent LSTM kernel
 
     // training (XB_FLAG_TRAIN; workspace allocated by the first xb_encoder_fwd_train, see train_bwd.cu)
     void *head_wT = nullptr;     // (768, head_rows_padded) bf16 = W_head^T
@@ -93,6 +93,8 @@ struct xb_handle {
 
     // driver entry point for TMA descriptors (resolved at run time: no link-time libcuda dependency)
     void *encode_tiled = nullptr;
+    // largest dynamic shared-memory size set per kernel on this handle (xb_smem_attr)
+    std::unordered_map<const void *, size_t> smem_attr;
 };
 
 extern thread_local std::string xb_global_err;
@@ -136,6 +138,30 @@ int xb_fail(xb_handle *h, int code, const char *fmt, ...);
         if (!(cond)) return xb_fail((h), XB_ERR_ARG, __VA_ARGS__);                               \
     } while (0)
 
+// *p = cudaMalloc(bytes) unless *p is already set: allocating a set of buffers through this again after a failure
+// completes the set
+inline int xb_alloc(xb_handle *h, void **p, size_t bytes) {
+    if (*p) return XB_OK;
+    cudaError_t e = cudaMalloc(p, bytes);
+    if (e != cudaSuccess) return xb_fail(h, XB_ERR_NOMEM, "cudaMalloc of %zu bytes failed: %s", bytes, cudaGetErrorString(e));
+    return XB_OK;
+}
+
+// Allows `kernel` `bytes` of dynamic shared memory.  Above the default 48 KB the limit is a function attribute of the
+// device's context; the handle records the largest size it has set per kernel, so the attribute is set once per size
+// step instead of per launch, and never lowered below what another handle on the same device has set.
+template <typename K> int xb_smem_attr(xb_handle *h, K kernel, size_t bytes) {
+    if (bytes <= 48 * 1024) return XB_OK;
+    size_t &set = h->smem_attr[reinterpret_cast<const void *>(kernel)];
+    if (bytes <= set) return XB_OK;
+    cudaFuncAttributes fa;
+    XB_CUDA(h, cudaFuncGetAttributes(&fa, kernel));
+    if ((size_t)fa.maxDynamicSharedSizeBytes > bytes) bytes = fa.maxDynamicSharedSizeBytes;
+    XB_CUDA(h, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    set = bytes;
+    return XB_OK;
+}
+
 // ---- 16-bit type helpers (fp16 default, bf16 with XB_FLAG_BF16) ---------------------------------
 template <bool BF16> struct xb16;
 template <> struct xb16<false> {
@@ -165,7 +191,37 @@ template <> struct xb16<true> {
     }
 };
 
-// ---- entry points implemented in the other translation units ------------------------------------
+// ---- functions one translation unit defines and others call ------------------------------------------
+struct xb_dropout;
+// xb_api.cu
+int xb_conv_stem_fwd_dropout(xb_handle *h, const void *signal, int sig_dtype, int N, int L, void *out_tnc,
+                             const xb_dropout *drop, void *stream);
+// conv_stem.cu
+int xb_conv12_im2col(xb_handle *h, const void *signal, int sig_dtype, int N, int L, cudaStream_t s,
+                     const xb_dropout *drop = nullptr);
+// lstm_persistent.cu
+int xb_lstm_recurrence_persistent(xb_handle *h, int layer, void *y_tnc, int T, int N, int reverse, cudaStream_t s,
+                                  void *save = nullptr);
+// inproj_gemm.cu
+int xb_inproj_launch(xb_handle *h, const void *x, const void *w_ih, const float *bias, void *gates, int M, cudaStream_t s);
+int xb_head_astationary_launch(xb_handle *h, const void *x, const void *w, int w_rows, const float *bias, int head_rows,
+                               float *scores, int ldo, int M, int exp_out, cudaStream_t s);
+// wgrad_gemm.cu
+int xb_lstm_wgrad_launch(xb_handle *h, const void *dzT, const void *xT, const void *yT, int T, int N, bool reverse, float *g_wih,
+                         float *g_whh, cudaStream_t s);
+// train_bwd.cu
+void xb_train_free(xb_handle *h);
+// misc_kernels.cu
+int xb_onehot_edges(xb_handle *h, const int32_t *edges_nt, int T, int N, int S, float *post, cudaStream_t s);
+int xb_ctc_loss_impl(xb_handle *h, const float *scores, int T, int N, const int32_t *targets, int Lmax,
+                     const int32_t *lengths, int normalise, float *loss, cudaStream_t s);
+int xb_ctc_loss_bwd_impl(xb_handle *h, const float *scores, int T, int N, const int32_t *targets, int Lmax,
+                         const int32_t *lengths, int normalise, const float *grad_loss, float *alpha_ws, float *grad,
+                         cudaStream_t s);
+// beam_search.cu
+int xb_beam_search_impl(xb_handle *h, const float *scores, const float *beta, int T, int N, int beam_width, float beam_cut,
+                        int8_t *seq, int8_t *qstring, int8_t *moves, int32_t *lens, cudaStream_t s);
+// crf_decode.cu, crf_decode_lin.cu
 int xb_decode_alpha(xb_handle *h, const float *scores, int T, int N, float *alpha, float *logz, int use_max, cudaStream_t s);
 int xb_decode_backward(xb_handle *h, const float *scores, int T, int N, float *bmax, float *beta, int mode, cudaStream_t s);
 int xb_decode_lin(xb_handle *h, const float *scores, int lin_input, int T, int N, int8_t *labels, int8_t *seq, int8_t *qs,

@@ -15,13 +15,13 @@ struct GemmParams {
     const void *dy = nullptr;      // (T, NB, 768) bf16: gradient w.r.t. the stem output
 };
 
-int xb_make_tmap_2d(xb_handle *h, CUtensorMap *out, const void *base, uint64_t rows, uint64_t K, uint64_t ld);
-int xb_make_tmap_2d_box(xb_handle *h, CUtensorMap *out, const void *base, uint64_t rows, uint64_t K, uint64_t ld,
-                        uint32_t box_inner, uint32_t box_rows, int swizzle128);
-int xb_make_tmap_hview(xb_handle *h, CUtensorMap *out, const void *base, uint64_t rows, uint32_t box_rows,
-                       uint32_t box_kblocks);
+// TMA descriptor of a rank-n tensor (2 <= n <= 5): dims / box in elements (innermost first), strides in BYTES for
+// dimensions 1 .. n-1; elem_bytes 2 (16-bit payload) or 4 (fp32).  With CU_TENSOR_MAP_SWIZZLE_128B the innermost box
+// extent must span 128 bytes.
 int xb_make_tmap_nd(xb_handle *h, CUtensorMap *out, const void *base, int rank, int elem_bytes, const uint64_t *dims,
-                    const uint64_t *strides_bytes, const uint32_t *box);
+                    const uint64_t *strides_bytes, const uint32_t *box, CUtensorMapSwizzle swizzle);
+// the GEMM operand: rows x K 16-bit elements, row pitch ld elements, box 64 x 128, 128B swizzle
+int xb_make_tmap_2d(xb_handle *h, CUtensorMap *out, const void *base, uint64_t rows, uint64_t K, uint64_t ld);
 
 // lstm_bptt.cu: one step of back-propagation through time of an LSTM layer (programmatic dependent launches)
 struct BpttMaps {
